@@ -19,6 +19,11 @@ Printed JSON (rank 0, one line):
 
 --impl reference times the CPU implementation alone (the reference itself is Python/Chainer and
 cannot travel to the GPU box, so this is the oracle port -- kind "port").
+
+--dump-outputs DIR (rank 0) writes what the headline path returned in its last timed step: DIR/loss.npy (the float32
+scalar loss) and DIR/grad_rows.npy (float32 (DUMP_FRAMES, V): the gradient rows of the frames dump_frames() picks with
+a fixed seed out of the (T,B,V) gradient, which at 717 MB is too large to keep whole).  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import importlib
@@ -40,6 +45,7 @@ METRIC = "CTC fwd+bwd utterance-frames/sec at B=64,T=800,V=3500"
 UNIT = "frames/s"
 FALLBACK_HBM_GBS = 6650.0
 REF_SAMPLE_UTTS = 4        # utterances of the workload the reference's NumPy path processes per timed step (~1.5 s)
+DUMP_FRAMES = 2048         # gradient rows --dump-outputs keeps: 2048 * V * 4 bytes = 28.7 MB
 
 
 def config_dict(world):
@@ -150,6 +156,25 @@ def algorithmic_bytes(V, in_len, B, T):
     return k1, k3
 
 
+def dump_frames(T, B):
+    """Flat frame indices t * B + b (ascending) of the gradient rows --dump-outputs writes: a fixed seeded sample."""
+    return np.sort(np.random.RandomState(0).choice(T * B, min(DUMP_FRAMES, T * B), replace=False))
+
+
+def sample_outputs(loss, grad):
+    """Device copies of a step's outputs that --dump-outputs keeps: the loss and the dump_frames() rows of the gradient."""
+    import torch
+    T, B, V = grad.shape
+    rows = torch.from_numpy(dump_frames(T, B)).to(grad.device)
+    return {"loss": loss.detach().clone(), "grad_rows": grad.detach().reshape(T * B, V).index_select(0, rows)}
+
+
+def write_outputs(dirname, outputs):
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(dirname, name + ".npy"), t.cpu().numpy().astype(np.float32))
+
+
 def port_baseline(prob, threads, budget_s=6.0):
     """Oracle C port (banded restatement of the reference algorithm, float64, OpenMP), forward+backward over the WHOLE
     64-utterance workload, repeated for ~budget_s seconds."""
@@ -173,7 +198,7 @@ class ReferenceSample(object):
     every bigram id -1 = plain CTC, SURVEY.md 8c) on the first REF_SAMPLE_UTTS utterances of the workload.  One step =
     GramCTC.forward + GramCTC.backward, exactly what a training step of the reference runs.  Its cost is linear in the
     number of utterances (every op is per utterance, SURVEY.md 8e), so frames/s of the sample is frames/s of the
-    workload.  Available wherever the reference's files are: /root/reference, or oracle/_ref on the GPU box."""
+    workload.  Available wherever the reference's files are (oracle/ref_stub.py: REFERENCE_ROOT)."""
 
     def __init__(self, prob, n=REF_SAMPLE_UTTS):
         from oracle import ref_stub
@@ -292,7 +317,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="do not also time the step as a CUDA graph replay")
     ap.add_argument("--no-kernel-loop", action="store_true",
                     help="skip the kernel-only loop of the dominant kernel (for ncu launch lists: steps only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and a fixed sample of the gradient rows of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     # Exactly ONE line goes to stdout: the JSON.  Libraries write banners there (NCCL prints its version on the first
@@ -423,6 +454,7 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     elapsed_ms, fwd_ms, bwd_ms = [float(v) for v in t.tolist()]
     loss_value = float(loss.item())
+    eager_outputs = sample_outputs(loss, x.grad) if args.dump_outputs else None
 
     # ---- the dominant kernel alone (gradient_ring_kernel): K launches of b200ctc_backward through the C ABI on the
     #      workspace of one forward, bracketed by CUDA events on the launching stream ----
@@ -465,7 +497,7 @@ def main():
 
     # ---- the same step captured once in a CUDA graph and replayed (single GPU): identical kernels on identical
     #      buffers, minus the host launch path and the launch/dependency gaps between the kernels ----
-    graph_ms = None
+    graph_ms, graph_outputs = None, None
     # Several GPUs: the graph holds the rank-local part of the step (capturing the NCCL all-reduce hung on this image);
     # the all-reduce of the graph's loss output is issued eagerly behind the replays (reduce_loss), as in the eager step.
     # B200CTC_BENCH_GRAPH_MULTI=0 switches the multi-GPU replay off.
@@ -510,6 +542,7 @@ def main():
                     dist.all_reduce(gt, op=dist.ReduceOp.MAX)      # slowest rank; any rank's mismatch disables it
                 if float(gt[1].item()) == 0.0:
                     graph_ms = float(gt[0].item())
+                    graph_outputs = sample_outputs(gl, x.grad) if args.dump_outputs else None
             except Exception as exc:                               # the eager number stands
                 sys.stderr.write("bench.py: CUDA graph replay skipped (%s)\n" % exc)
 
@@ -546,6 +579,8 @@ def main():
     step_bytes = k1_bytes + k3_bytes
     eager_ms_per_step = elapsed_ms / args.steps
     ms_per_step = min(eager_ms_per_step, graph_ms) if graph_ms else eager_ms_per_step
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, graph_outputs if graph_ms and graph_ms < eager_ms_per_step else eager_outputs)
     value = world * B * T / (ms_per_step * 1e-3)
     k3_time_ms = k3_ms if k3_ms else bwd_ms
     achieved = k3_bytes / (k3_time_ms * 1e-3) / 1e9

@@ -30,13 +30,16 @@ import numpy as np
 _STAGED = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 REFERENCE_ROOT = os.environ.get("B200CTC_REFERENCE_ROOT") or (
     "/root/reference" if os.path.isfile("/root/reference/asr/loss/gram_ctc.py") else _STAGED)
-STAGED_FILES = ("asr/loss/gram_ctc.py", "asr/error.py", "asr/vocab.py", "asr/utils.py", "asr/nn/layernorm.py")
+STAGED_FILES = ("asr/loss/gram_ctc.py", "asr/error.py", "asr/vocab.py", "asr/utils.py", "asr/nn/layernorm.py",
+                "asr/data/processing.py")
 
 
-def stage(src_root="/root/reference"):
-    """Copy the reference files of the path, unmodified, into oracle/_ref/ (build container only)."""
+def stage(src_root=None):
+    """Copy the reference files of the path, unmodified, from src_root (default: the checkout REFERENCE_ROOT names)
+    into oracle/_ref/."""
     import shutil
-    if not os.path.isfile(os.path.join(src_root, "asr", "loss", "gram_ctc.py")):
+    src_root = src_root or REFERENCE_ROOT
+    if os.path.abspath(src_root) == _STAGED or not os.path.isfile(os.path.join(src_root, "asr", "loss", "gram_ctc.py")):
         return False
     for rel in STAGED_FILES:
         dst = os.path.join(_STAGED, rel)

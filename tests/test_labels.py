@@ -31,6 +31,13 @@ def test_labels_match_reference_golden(path):
     assert np.array_equal(xl.numpy(), g["ref_x_length"])
     # one host block behind all four views (one copy moves everything to the device)
     assert t.untyped_storage().data_ptr() == big.untyped_storage().data_ptr() == tl.untyped_storage().data_ptr()
+    # the transcriptions as strings through tokenizer=: the golden tokens are the reference tokeniser's output for them
+    # (tests/golden/generate_golden_labels.py), so a lookup of that output stands in for the reference's tokeniser
+    reference_tokens = {"".join(s): s for s in sentences}
+    t, big, xl, tl = mine().labels_to_minibatch(["".join(s) for s in sentences], g["x_length"], int(g["Lmax"]), ids, 0,
+                                                tokenizer=lambda s: list(reference_tokens[s]))
+    assert np.array_equal(t.numpy(), g["ref_t"]) and np.array_equal(big.numpy(), g["ref_bigram"])
+    assert np.array_equal(tl.numpy(), g["ref_t_length"]) and np.array_equal(xl.numpy(), g["ref_x_length"])
 
 
 def test_golden_set_is_present():

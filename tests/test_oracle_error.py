@@ -51,6 +51,12 @@ def test_oracle_matches_reference_live():
     assert err.compute_character_error_rate([1, 2], []) == oerr.character_error_rate([1, 2], []) == 1.0
 
 
+def test_character_error_rate_of_empty_sequences_is_the_references():
+    # the reference's compute_character_error_rate returns these (asr/error.py:8-9 and :24; checked against it live above)
+    assert oerr.character_error_rate([], [1, 2, 3]) == 3
+    assert oerr.character_error_rate([1, 2], []) == 1.0
+
+
 def test_collapse_is_the_prev_token_state_machine():
     # asr/error.py:38-47: a blank resets prev_token, repeats are dropped, a repeat after a blank counts again
     assert oerr.collapse([0, 3, 3, 0, 3, 4, 4, 4, 0, 0, 5], 0) == [3, 3, 4, 5]
