@@ -12,6 +12,9 @@ normalised tensor, its transpose and their gradients are never materialised (csr
     loss = layernorm_ctc(z, ln.gamma, ln.beta, t_batch, ID_BLANK, x_length_batch, t_length_batch)
     # instead of:  y_batch = model(x_batch)  [..., LayerNormalization, swapaxes/reshape/split_axis]
     #              loss = F.connectionist_temporal_classification(y_batch, t_batch, ID_BLANK, x_length_batch, t_length_batch)
+
+    loss = layernorm_gram_ctc(z, ln.gamma, ln.beta, t_batch, bigram_batch, ID_BLANK, x_length_batch, t_length_batch,
+                              joint_ctc=args.joint_training)     # Gram-CTC, optionally + CTC (joint training)
 """
 import numpy as np
 import torch
@@ -106,7 +109,7 @@ def _layernorm_loss(kind, z, gamma, beta, labels, bigrams, blank_symbol, input_l
     labels = _as_int32(labels, dev, "labels")
     if labels.dim() != 2 or labels.shape[0] != B:
         raise ValueError("labels must have shape (B, Lmax)")
-    if kind == _lib.KIND_GRAM:
+    if kind != _lib.KIND_CTC:
         bigrams = _as_int32(bigrams, dev, "label_bigram")
         if bigrams.shape != labels.shape:
             raise ValueError("label_bigram must have the shape of label_unigram")
@@ -136,7 +139,13 @@ def layernorm_ctc(z, gamma, beta, t, blank_symbol, input_length=None, label_leng
 
 
 def layernorm_gram_ctc(z, gamma, beta, label_unigram, label_bigram, blank_symbol, input_length=None, length_unigram=None,
-                       reduce="mean", **kw):
-    """The same in front of ``gram_ctc`` (asr/loss/gram_ctc.py:300)."""
-    return _layernorm_loss(_lib.KIND_GRAM, z, gamma, beta, label_unigram, label_bigram, blank_symbol, input_length,
+                       reduce="mean", joint_ctc=False, **kw):
+    """The same in front of ``gram_ctc`` (asr/loss/gram_ctc.py:300).
+
+    ``joint_ctc=True`` is the joint-training objective of run/gram_ctc/cnn/train.py:196-198 (``args.joint_training``):
+    ``gram_ctc(...) + connectionist_temporal_classification(..., label_unigram, ...)`` on the same normalised activations,
+    as ``gram_ctc(..., joint_ctc=True)`` computes it.  Per-utterance losses are the sums of the two losses, the reduced
+    loss is ``scale * sum_b (gram_b + ctc_b)``, and dz / dgamma / dbeta are the gradients of the sum."""
+    kind = _lib.KIND_JOINT if joint_ctc else _lib.KIND_GRAM
+    return _layernorm_loss(kind, z, gamma, beta, label_unigram, label_bigram, blank_symbol, input_length,
                            length_unigram, reduce, **kw)

@@ -111,8 +111,9 @@ int forward_impl(const LnInput *ln, int kind, const float *acts, int64_t stride_
         if ((!ln->z && (size_t)B * T > 0) || !ln->gamma || !ln->beta) return fail(B200CTC_INVALID_ARGUMENT, "z, gamma or beta is NULL%s");
         if (argmax_out) return fail(B200CTC_UNSUPPORTED, "the fused LayerNormalization path has no greedy output%s");
         if (!ln_supported(kind, B, T, V, Lmax, ln->zs_v, ln->zs_b, ln->z))
-            return fail(B200CTC_UNSUPPORTED, "fused LayerNormalization needs kind CTC or Gram-CTC, V <= 4080, <= 480 emission columns, "
-                                             "and 16-byte aligned rows of z (pitch %% 4 == 0)%s");
+            return fail(B200CTC_UNSUPPORTED, "fused LayerNormalization needs V <= 4080, <= 480 emission columns, a label length whose "
+                                             "backward tile fits shared memory at this V, and 16-byte aligned rows of z "
+                                             "(pitch %% 4 == 0)%s");
     }
     if (!labels && Lmax > 0) return fail(B200CTC_INVALID_ARGUMENT, "labels is NULL%s");
     if (kind != B200CTC_KIND_CTC && !bigrams && Lmax > 0) return fail(B200CTC_INVALID_ARGUMENT, "bigrams is NULL for Gram-CTC%s");
@@ -276,7 +277,6 @@ int b200ctc_ln_workspace_bytes(int kind, int B, int T, int V, int Lmax, size_t *
     if (!bytes_out) return fail(B200CTC_INVALID_ARGUMENT, "bytes_out is NULL%s");
     int rc = validate(kind, B, T, V, Lmax, 0, false);
     if (rc) return rc;
-    if (kind == B200CTC_KIND_JOINT) return fail(B200CTC_UNSUPPORTED, "the joint objective has no fused LayerNormalization path%s");
     *bytes_out = make_ln_layout(kind, B, T, V, Lmax).total;
     return B200CTC_OK;
 }
@@ -307,7 +307,8 @@ int b200ctc_ln_backward(int kind, const float *z, int64_t zstride_b, int64_t zst
     if (!z || !gamma || !beta || !grad_loss || !dz || !workspace) return fail(B200CTC_INVALID_ARGUMENT, "NULL pointer%s");
     if (!ln_supported(kind, B, T, V, Lmax, zstride_v, zstride_b, z) || (dzstride_v & 3) != 0 || (dzstride_b & 3) != 0 ||
         (reinterpret_cast<uintptr_t>(dz) & 15) != 0)
-        return fail(B200CTC_UNSUPPORTED, "fused LayerNormalization needs kind CTC or Gram-CTC, V <= 4080 and 16-byte aligned rows of z and dz%s");
+        return fail(B200CTC_UNSUPPORTED, "fused LayerNormalization needs V <= 4080, a label length whose backward tile fits shared "
+                                         "memory at this V, and 16-byte aligned rows of z and dz%s");
     const LnLayout ll = make_ln_layout(kind, B, T, V, Lmax);
     if (workspace_bytes < ll.total) return fail(B200CTC_WORKSPACE_TOO_SMALL, "workspace too small%s");
     GradParams g;

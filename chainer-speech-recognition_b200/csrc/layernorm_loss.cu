@@ -25,9 +25,14 @@
 //            (it is still there) and stores dz = rstd * (dn - mean_v(dn) - n * mean_v(dn*n)).
 // 12 bytes per element again -- for the loss AND the normalisation AND both transposes.
 //
+// Joint Gram-CTC + CTC objective (run/gram_ctc/cnn/train.py:196-198): the forward pass is Gram-CTC's plus the second,
+// plain-CTC lattice on the same emission rows (api.cu); the backward kernel adds the plain-CTC posteriors to the Gram-CTC
+// ones node by node in phase (a) and doubles the softmax term (two losses).
+//
 // Limits of this version: V <= 4080 (a tile must stay resident in shared memory in the backward kernel: 17 boxes),
-// rows of z 16-byte aligned (T_pitch % 4 == 0 -- a TMA requirement), at most 480 emission columns.  Outside them the
-// entry points return B200CTC_UNSUPPORTED and the caller uses the unfused path.
+// rows of z 16-byte aligned (T_pitch % 4 == 0 -- a TMA requirement), at most 480 emission columns, and a backward ring
+// of at least K + 2 boxes next to the lattice's per-tile tables (plan_ln_backward: long labels at a large V do not fit).
+// Outside them the entry points return B200CTC_UNSUPPORTED and the caller uses the unfused path.
 #include <cuda.h>
 #include <stdio.h>
 #include <mutex>
@@ -47,6 +52,7 @@ constexpr int kLnBoxRows = 16 * kLnWarps;                  // 240 rows: one step
 constexpr uint32_t kLnBoxBytes = kLnBoxRows * kLnTT * 4;   // 7.5 KB
 constexpr int kLnMetaRing = 64;                            // >= ring slots: a padded tile takes one slot and one record
 constexpr int kLnMaxCols = 32 * kLnWarps;                  // emission columns one tile pass can gather: one per compute thread
+constexpr int kLnJointPre = 4;                             // joint backward: plain-CTC alpha/beta items a thread requests ahead
 
 #ifdef B200CTC_EXPERIMENT
 // phase timers (tools/ln_phases.py): per CTA and warp, cycles per phase of the tile loop
@@ -688,7 +694,8 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
 // ---------------------------------------------------------------------------------------------
 // Rows that do not exist get gamma = beta = 0 in the shared-memory table: their dn is 0 (nothing enters the per-frame
 // sums) and what they add to this thread's dgamma/dbeta slots is never stored.  Frames that do not exist (padding) get
-// rstd = 0 and scale = 0, which makes every quantity of theirs exactly zero.  No predicates in the sweeps.
+// rstd = 0 and a log2 normaliser of -inf (softmax 0), which makes every quantity of theirs exactly zero.  No predicates in
+// the sweeps.
 // dz leaves as it came in: sweep 2 writes each box's image over the z it was computed from, and lane 1 of the producer
 // warp hands the boxes to the TMA engine as tile stores (an SM storing 32-byte pieces itself spends 16 L1 wavefronts
 // per instruction: the LSU, not HBM, bounded the first version of this kernel).
@@ -748,9 +755,11 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
     const int per = d.kind == 0 ? 2 : 3;
     const float inv_v = 1.f / (float)d.V;
     const int nwt = Vt / 32 + 1;                          // words of the bitmap / prefix tables in shared memory
-    float dgam[KMAX], dbet[KMAX];
+    // dgamma (h = 0) or dbeta (h = 1) of this thread's rows: the two threads of a row add up their halves of every tile
+    // with one shuffle and keep one sum each (one register per box instead of two: sweep 1 is the register peak)
+    float dgb[KMAX];
 #pragma unroll
-    for (int k = 0; k < KMAX; ++k) { dgam[k] = 0.f; dbet[k] = 0.f; }
+    for (int k = 0; k < KMAX; ++k) dgb[k] = 0.f;
 
     SlotIter it = {0u, 0u};
     unsigned seq = 0, n_ab = 0;
@@ -776,43 +785,81 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
             for (int i = tid; i < m.Nb; i += 32 * kLnWarps) csr[wl.Nmax + 1 + i] = __ldg(unode + i);
             for (int i = tid; i < wl.nwords; i += 32 * kLnWarps) { bm_sm[i] = __ldg(bm_g + i); bm_sm[nwt + i] = (unsigned)__ldg(pc_g + i); }
         }
+        // Joint objective: each blank / unigram node of the Gram-CTC lattice shares its symbol occurrence with one node of
+        // the plain-CTC lattice (3i <-> 2i, 3i+1 <-> 2i+1; bigram nodes have no partner, gradient.cu joint_partner).
+        // Adding the partner's posterior to e[j] leaves the per-id merge, the blank sums and sweep 2 as they are.  The
+        // partner's alpha/beta come from global memory straight into registers, requested here so that their round trip
+        // hides behind the wait for the Gram-CTC rows: no shared memory is taken from the ring.  The plain-CTC lattice's P
+        // comes the same way (not in the tile record: a larger record would take shared memory from the ring too).
+        const int nfv = min(kLnTT, m.Tb - m.t0);
+        const int Nbp = (m.Nb + 31) & ~31;
+        const int nitems = nfv * Nbp;
+        const float2 *a2g = reinterpret_cast<const float2 *>(p.ws + wl.off_av2) + ((size_t)m.b * d.T + m.t0) * wl.Np2;
+        const float2 *b2g = reinterpret_cast<const float2 *>(p.ws + wl.off_bv2) + ((size_t)m.b * d.T + m.t0) * wl.Np2 + 1;
+        auto ctc_partner_ab = [&](int i) {                // (alpha.m, alpha.e, beta.m, beta.e); probability 0 if none
+            float4 v = make_float4(0.f, SENT, 0.f, SENT);
+            const int f = i / Nbp, j = i - f * Nbp;
+            if (wl.joint && j < m.Nb && j % 3 != 2) {
+                const int jc = 2 * (j / 3) + j % 3;
+                const float2 a = __ldg(a2g + (size_t)f * wl.Np2 + jc), bb = __ldg(b2g + (size_t)f * wl.Np2 + jc);
+                v = make_float4(a.x, a.y, bb.x, bb.y);
+            }
+            return v;
+        };
+        float Ph2 = 0.f, Pl2 = 0.f;
+        if (wl.joint) {
+            const UttInfo *u2 = reinterpret_cast<const UttInfo *>(p.ws + wl.off_utt2) + m.b;
+            Ph2 = __ldg(&u2->Ph);
+            Pl2 = __ldg(&u2->Pl);
+        }
+        float4 ab2[kLnJointPre];
+#pragma unroll
+        for (int q = 0; q < kLnJointPre; ++q) {
+            const int i = tid + q * 32 * kLnWarps;
+            ab2[q] = (wl.joint && i < nitems) ? ctc_partner_ab(i) : make_float4(0.f, SENT, 0.f, SENT);
+        }
         mbar_spin(&abbar[0], n_ab & 1u, 15);
         ++n_ab;
         LN_T(2);
         // per-frame constants of this thread's four frames (staged by the producer)
-        float rs[4], mur[4], nl[4], scj[4];
+        float rs[4], mur[4], nl[4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const bool valid = m.t0 + 4 * h + j < m.Tb;
             const float rr = valid ? fc[kLnTT + 4 * h + j] : 0.f;
             rs[j] = rr; mur[j] = valid ? -fc[4 * h + j] * rr : 0.f;
-            nl[j] = valid ? -fc[2 * kLnTT + 4 * h + j] : 0.f;
-            scj[j] = valid ? m.sc : 0.f;
+            nl[j] = valid ? -fc[2 * kLnTT + 4 * h + j] : -INFINITY;
         }
+        const float scs = wl.joint ? 2.f * m.sc : m.sc;                     // joint: two losses, two softmax terms
         {
             // alpha * beta / P of every node of every valid frame
             const float2 *a_sm = reinterpret_cast<const float2 *>(smem + sm.off_ab);
             const float2 *b_sm = a_sm + (size_t)kLnTT * wl.Np;
-            const int nfv = min(kLnTT, m.Tb - m.t0);
-            const int Nbp = (m.Nb + 31) & ~31;
             // a warp's 32 items are 32 consecutive nodes of ONE frame (Nbp and the stride are multiples of 32): the blank
             // nodes among them are summed by shuffle and left as one partial per 32-node chunk, summed in order below
-            for (int i = tid; i < nfv * Nbp; i += 32 * kLnWarps) {
+            auto node_item = [&](int i, const float4 &c2) {
                 const int f = i / Nbp, j = i - f * Nbp;
                 float e = 0.f;
                 if (j < m.Nb) {
                     e = node_posterior(a_sm[f * wl.Np + j], b_sm[f * wl.Np + j + wl.boff], m.Ph, m.Pl);
+                    if (wl.joint && j % 3 != 2) e += node_posterior(make_float2(c2.x, c2.y), make_float2(c2.z, c2.w), Ph2, Pl2);
                     ebuf[f * Nst + j] = e;
                 }
                 const float bp = warp_sum((j < m.Nb && j % per == 0) ? e : 0.f);
                 if (lane == 0) bpart[f * kLnBlankChunks + (j >> 5)] = bp;
+            };
+#pragma unroll
+            for (int q = 0; q < kLnJointPre; ++q) {
+                const int i = tid + q * 32 * kLnWarps;
+                if (i < nitems) node_item(i, ab2[q]);
             }
+            // long lattices (joint: more than kLnJointPre items per thread): the rest loads as it goes
+            for (int i = tid + kLnJointPre * 32 * kLnWarps; i < nitems; i += 32 * kLnWarps) node_item(i, ctc_partner_ab(i));
         }
         bar_compute();
         if (tid == 0) mbar_arrive(&abbar[1]);                                 // alpha/beta and the frame constants can be refilled
         {
             // merged per emitted id, in node order (deterministic); the blank collects every per-th node
-            const int nfv = min(kLnTT, m.Tb - m.t0);
             for (int i = tid; i < kLnTT * m.Ub; i += 32 * kLnWarps) {
                 const int f = i / m.Ub, u = i - f * m.Ub;
                 float ps = 0.f;
@@ -857,15 +904,16 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
                     }
                     const float n0 = fmaf(zq.x, rs[0], mur[0]), n1 = fmaf(zq.y, rs[1], mur[1]);
                     const float n2 = fmaf(zq.z, rs[2], mur[2]), n3 = fmaf(zq.w, rs[3], mur[3]);
-                    const float g0 = fmaf(ex2_approx(fmaf(fmaf(n0, g_, b_), LOG2E_HI, nl[0])), scj[0], -p0);
-                    const float g1 = fmaf(ex2_approx(fmaf(fmaf(n1, g_, b_), LOG2E_HI, nl[1])), scj[1], -p1);
-                    const float g2 = fmaf(ex2_approx(fmaf(fmaf(n2, g_, b_), LOG2E_HI, nl[2])), scj[2], -p2);
-                    const float g3 = fmaf(ex2_approx(fmaf(fmaf(n3, g_, b_), LOG2E_HI, nl[3])), scj[3], -p3);
+                    const float g0 = fmaf(ex2_approx(fmaf(fmaf(n0, g_, b_), LOG2E_HI, nl[0])), scs, -p0);
+                    const float g1 = fmaf(ex2_approx(fmaf(fmaf(n1, g_, b_), LOG2E_HI, nl[1])), scs, -p1);
+                    const float g2 = fmaf(ex2_approx(fmaf(fmaf(n2, g_, b_), LOG2E_HI, nl[2])), scs, -p2);
+                    const float g3 = fmaf(ex2_approx(fmaf(fmaf(n3, g_, b_), LOG2E_HI, nl[3])), scs, -p3);
                     const float d0 = g0 * g_, d1 = g1 * g_, d2 = g2 * g_, d3 = g3 * g_;
                     s1[0] += d0; s1[1] += d1; s1[2] += d2; s1[3] += d3;
                     s2[0] = fmaf(d0, n0, s2[0]); s2[1] = fmaf(d1, n1, s2[1]); s2[2] = fmaf(d2, n2, s2[2]); s2[3] = fmaf(d3, n3, s2[3]);
-                    dbet[k] += (g0 + g1) + (g2 + g3);                          // bias backward: sum over (b, t)
-                    dgam[k] = fmaf(g0, n0, fmaf(g1, n1, fmaf(g2, n2, fmaf(g3, n3, dgam[k]))));      // scale backward
+                    const float tb = (g0 + g1) + (g2 + g3);                    // bias backward: sum over (b, t)
+                    const float tg = fmaf(g0, n0, fmaf(g1, n1, fmaf(g2, n2, g3 * n3)));      // scale backward
+                    dgb[k] += (h ? tb : tg) + __shfl_xor_sync(0xffffffffu, h ? tg : tb, 1);
                     dn[k] = make_float4(d0, d1, d2, d3);
                 }
             }
@@ -917,16 +965,12 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
         LN_T(7);
     }
     LN_T_FLUSH(w);
-    // ---- this CTA's share of dgamma / dbeta: the two halves of a row pair up, then one partial row per CTA ----
+    // ---- this CTA's share of dgamma / dbeta: one partial row per CTA ----
     const int Vp = K * kLnBoxRows;
-    float *part = reinterpret_cast<float *>(p.ws + p.off_part) + (size_t)blockIdx.x * 2 * Vp;
+    float *part = reinterpret_cast<float *>(p.ws + p.off_part) + (size_t)blockIdx.x * 2 * Vp + (size_t)h * Vp;
 #pragma unroll
-    for (int k = 0; k < KMAX; ++k) {
-        const float g = dgam[k] + __shfl_xor_sync(0xffffffffu, dgam[k], 1);
-        const float b = dbet[k] + __shfl_xor_sync(0xffffffffu, dbet[k], 1);
-        const int v = kLnBoxRows * k + vrow;
-        if (k < K && h == 0) { part[v] = g; part[Vp + v] = b; }
-    }
+    for (int k = 0; k < KMAX; ++k)
+        if (k < K) part[kLnBoxRows * k + vrow] = dgb[k];
 }
 
 // dgamma[v] = sum over CTAs of their partial rows, in CTA order (deterministic)
@@ -943,6 +987,20 @@ __global__ void ln_reduce_params_kernel(const float *part, int nparts, int Vp, i
 }
 
 static int ln_kmax(int K) { return K <= 5 ? 5 : (K <= 9 ? 9 : (K <= 15 ? 15 : 17)); }
+
+// The backward kernel's shared-memory plan -- the one place that decides whether a shape's backward pass can run:
+// launch_ln_backward launches with it and ln_supported refuses (at the forward call, before any work is enqueued) every
+// shape whose ring would hold fewer than K + 2 boxes.  Everything but the ring is fixed by (V, Lmax, kind): two alpha/beta
+// rows per frame of a tile, the merged posteriors, the node posteriors with their blank partials, the symbol tables, the
+// gamma/beta table, the id bitmap and one box of zeros; the ring gets what is left.  The joint objective's plain-CTC
+// lattice takes nothing here (phase (a) of ln_gradient_kernel reads it into registers): its plan is Gram-CTC's.
+LnSmem plan_ln_backward(const WsLayout &w) {
+    const int K = (w.V + kLnBoxRows - 1) / kLnBoxRows;
+    const int Vt = ln_kmax(K) * kLnBoxRows;
+    return plan_ln_smem(K, (size_t)2 * kLnTT * w.Np * 8, (size_t)kLnTT * ((w.Umax + 3) & ~3),
+                        (size_t)kLnTT * w.Np + (size_t)kLnTT * kLnBlankChunks, (size_t)2 * w.Nmax + 2, (size_t)2 * Vt,
+                        (size_t)2 * (Vt / 32 + 1), kLnBoxBytes);
+}
 
 // ---- host side ----
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
@@ -1013,10 +1071,11 @@ LnLayout make_ln_layout(int kind, int B, int T, int V, int Lmax) {
 }
 
 int ln_supported(int kind, int B, int T, int V, int Lmax, int64_t zs_v, int64_t zs_b, const void *z) {
-    (void)B; (void)T;
-    if (kind != 0 && kind != 1) return 0;                           // the joint objective is not fused yet
+    if (kind < 0 || kind > 2) return 0;
     if (V > 17 * kLnBoxRows) return 0;
     if (1 + (kind == 0 ? Lmax : 2 * Lmax) > kLnMaxCols) return 0;
+    const int K = (V + kLnBoxRows - 1) / kLnBoxRows;
+    if (plan_ln_backward(make_layout(kind, B, T, V, Lmax)).R < K + 2) return 0;
     if ((zs_v & 3) != 0 || (zs_b & 3) != 0 || (reinterpret_cast<uintptr_t>(z) & 15) != 0) return 0;
     return encode_tiled_fn() != nullptr;
 }
@@ -1073,11 +1132,7 @@ cudaError_t launch_ln_backward(const GradParams &g, const LnLayout &ll, const vo
     p.grad_loss = g.grad_loss; p.per_utterance = g.per_utterance; p.scale = g.scale;
     p.dz = dz; p.dzs_b = dzs_b; p.dzs_v = dzs_v; p.dgamma = dgamma; p.dbeta = dbeta;
     const int Vp = p.K * kLnBoxRows;
-    const int Vt = ln_kmax(p.K) * kLnBoxRows;
-    const LnSmem sm = plan_ln_smem(p.K, (size_t)2 * kLnTT * ll.w.Np * 8, (size_t)kLnTT * ((ll.w.Umax + 3) & ~3),
-                                   (size_t)kLnTT * ll.w.Np + (size_t)kLnTT * kLnBlankChunks, (size_t)2 * ll.w.Nmax + 2, (size_t)2 * Vt,
-                                   (size_t)2 * (Vt / 32 + 1),
-                                   kLnBoxBytes);
+    const LnSmem sm = plan_ln_backward(ll.w);
     if (sm.R < p.K + 2) { note_failure_site("shared-memory plan"); return cudaErrorInvalidConfiguration; }
     p.R = sm.R;
     p.group = ln_group();

@@ -42,7 +42,7 @@
 extern "C" {
 #endif
 
-#define B200CTC_VERSION 200
+#define B200CTC_VERSION 201
 
 enum {
     B200CTC_OK = 0,
@@ -127,8 +127,13 @@ int b200ctc_backward(int kind,
  *   dgamma, dbeta  float32 (V) or NULL: sums over all frames of the batch, in a fixed order (deterministic)
  * with LayerNormalization's backward (asr/nn/layernorm.py:48-60) and both transposes folded in: z is read once in
  * forward, once in backward, dz is written once.  loss outputs, grad_loss / per_utterance / scale as in
- * b200ctc_forward / b200ctc_backward.  Returns B200CTC_UNSUPPORTED (use the unfused entry points) for the joint
- * objective, V > 4080, more than 480 emission columns (1 + Lmax for CTC, 1 + 2*Lmax for Gram-CTC) or unaligned rows.
+ * b200ctc_forward / b200ctc_backward.  kind may be B200CTC_KIND_JOINT: the loss outputs are then the sums of the
+ * Gram-CTC and the plain-CTC loss, and dz / dgamma / dbeta are the gradients of that sum.
+ * Returns B200CTC_UNSUPPORTED (use the unfused entry points) for V > 4080, more than 480 emission columns (1 + Lmax for
+ * CTC, 1 + 2*Lmax for Gram-CTC and joint), unaligned rows, or an Lmax too long for the backward kernel's tile to fit in
+ * shared memory at this V (at V = 4080: Lmax > 97 for CTC, Lmax > 63 for Gram-CTC and joint).  b200ctc_ln_forward
+ * already refuses a shape whose backward pass could not run, so a caller can take the unfused path before any work is
+ * enqueued.
  */
 int b200ctc_ln_workspace_bytes(int kind, int B, int T, int V, int Lmax, size_t *bytes_out);
 int b200ctc_ln_forward(int kind,
