@@ -13,16 +13,12 @@ import tempfile
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "_lib")
-# B200CTC_EXPERIMENT=1 selects the experiment build (-DB200CTC_EXPERIMENT: timeline hooks and tuning knobs for tools/);
-# it is a separate file, so the product library never carries them
-EXPERIMENT = os.environ.get("B200CTC_EXPERIMENT") == "1"
-_NAME = "libb200ctc_exp" if EXPERIMENT else "libb200ctc"
-SO_PATH = os.path.join(LIBDIR, _NAME + ".so")
-STAMP = os.path.join(LIBDIR, _NAME + ".stamp")
+SO_PATH = os.path.join(LIBDIR, "libb200ctc.so")
+STAMP = os.path.join(LIBDIR, "libb200ctc.stamp")
 SOURCES = ["api.cu", "host_cache.cu", "softmax_gather.cu", "lattice.cu", "gradient.cu", "greedy_error.cu", "layernorm_loss.cu"]
 HEADERS = ["common.cuh", "kernels.h", "row_ring.cuh", "prep.cuh", os.path.join("..", "..", "include", "b200ctc.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
-              "-Xcompiler", "-fPIC", "-shared", "-cudart", "shared"] + (["-DB200CTC_EXPERIMENT"] if EXPERIMENT else [])
+              "-Xcompiler", "-fPIC", "-shared", "-cudart", "shared"]
 
 
 def find_nvcc():
@@ -68,7 +64,7 @@ def build(force=False, verbose=False):
             env = dict(os.environ)
             env.pop("CC", None)      # the image exports a broken CC wrapper; let nvcc find the PATH g++
             env.pop("CXX", None)
-            fd, tmp = tempfile.mkstemp(prefix=_NAME + ".", suffix=".so.tmp", dir=LIBDIR)
+            fd, tmp = tempfile.mkstemp(prefix="libb200ctc.", suffix=".so.tmp", dir=LIBDIR)
             os.close(fd)
             try:
                 cmd = [nvcc] + NVCC_FLAGS + ["-o", tmp] + [os.path.join(CSRC, s) for s in SOURCES]

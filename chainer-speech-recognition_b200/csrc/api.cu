@@ -134,7 +134,7 @@ int forward_impl(const LnInput *ln, int kind, const float *acts, int64_t stride_
     d.acts = acts; d.stride_t = stride_t; d.stride_b = stride_b;
     d.labels = labels; d.bigrams = kind != B200CTC_KIND_CTC ? bigrams : nullptr;
     d.input_lengths = input_lengths; d.label_lengths = label_lengths;
-    d.progress = 0;
+    d.concurrent = 0;
     unsigned char *ws = static_cast<unsigned char *>(workspace);
     const int nprog = B * w.nblk;
     zero_header_kernel<<<(nprog + 255) / 256 > 0 ? (nprog + 255) / 256 : 1, 256, 0, stream>>>(
@@ -144,7 +144,7 @@ int forward_impl(const LnInput *ln, int kind, const float *acts, int64_t stride_
     LatticeParams lp;
     lp.d = d; lp.w = w; lp.ws = ws;
     lp.loss_per_utt = loss_per_utt; lp.loss_reduced = loss_reduced; lp.loss_scale = loss_scale;
-    lp.W = 0; lp.S = 0; lp.second = 0; lp.dbg_nostore = 0;
+    lp.W = 0; lp.S = 0; lp.second = 0;
     int st = 0;
     // joint Gram-CTC + CTC: the plain-CTC lattice is a second launch behind the Gram-CTC one (same stream), on the
     // same emission rows; it adds its loss to loss_per_utt and reduces the batch
@@ -173,10 +173,7 @@ int forward_impl(const LnInput *ln, int kind, const float *acts, int64_t stride_
         st = 0;
     }
     if (side) {
-        d.progress = 3;
-#ifdef B200CTC_EXPERIMENT
-        if (knobs().dbg_progress >= 0) d.progress = knobs().dbg_progress;
-#endif
+        d.concurrent = 1;
         lp.d = d;
         if ((rc = check_cuda(cudaEventRecord(side->fork, stream), "fork event"))) return rc;
         if (ln) {
@@ -186,15 +183,12 @@ int forward_impl(const LnInput *ln, int kind, const float *acts, int64_t stride_
         if ((rc = check_cuda(cudaStreamWaitEvent(side->stream, side->fork, 0), "fork wait"))) return rc;
         if ((rc = check_cuda(launch_lattice(lp, side->stream, &st, true), "lattice kernel"))) return rc;
         if (w.joint && !st) {
-            lp2.d.progress = d.progress;
+            lp2.d.concurrent = d.concurrent;
             if ((rc = check_cuda(launch_lattice(lp2, side->stream, &st, false), "CTC lattice kernel"))) return rc;
         }
         if ((rc = check_cuda(cudaEventRecord(side->join, side->stream), "join event"))) return rc;
         if ((rc = check_cuda(cudaStreamWaitEvent(stream, side->join, 0), "join wait"))) return rc;
     } else {
-#ifdef B200CTC_EXPERIMENT
-        if (knobs().dbg_progress >= 0) d.progress = knobs().dbg_progress & 64;      // streaming-rate experiment (softmax_gather.cu)
-#endif
         if (ln) {
             if ((rc = check_cuda(launch_ln_forward(d, ll, ws, ln->z, ln->zs_b, ln->zs_v, ln->gamma, ln->beta, 0, stream),
                                  "layernorm softmax/gather kernel"))) return rc;
@@ -208,28 +202,7 @@ int forward_impl(const LnInput *ln, int kind, const float *acts, int64_t stride_
 
 }  // namespace
 
-#ifdef B200CTC_EXPERIMENT
-namespace b200ctc {
-void lattice_set_debug(long long *p);
-void lattice_set_timeline(long long *p);
-void softmax_set_timeline(long long *p);
-void softmax_set_roles(long long *p);
-void ln_set_debug(long long *p);
-void gradient_set_timeline(long long *p);
-}
-#endif
-
 extern "C" {
-
-#ifdef B200CTC_EXPERIMENT
-/* profiling hooks of the experiment build (tools/step_timeline.py, tools/lattice_timeline.py); not part of the ABI */
-void b200ctc_debug_lattice(long long *p) { b200ctc::lattice_set_debug(p); }
-void b200ctc_debug_k1_roles(long long *p) { b200ctc::softmax_set_roles(p); }
-void b200ctc_debug_ln(long long *p) { b200ctc::ln_set_debug(p); }
-void b200ctc_debug_timeline(long long *p) {
-    b200ctc::softmax_set_timeline(p); b200ctc::lattice_set_timeline(p); b200ctc::gradient_set_timeline(p);
-}
-#endif
 
 int b200ctc_version(void) { return B200CTC_VERSION; }
 
@@ -267,7 +240,7 @@ int b200ctc_backward(int kind, const float *acts, int64_t stride_t, int64_t stri
     g.d.kind = kind == B200CTC_KIND_CTC ? 0 : 1; g.d.B = B; g.d.T = T; g.d.V = V; g.d.Lmax = Lmax; g.d.blank = blank;
     g.d.acts = acts; g.d.stride_t = stride_t; g.d.stride_b = stride_b;
     g.d.labels = labels; g.d.bigrams = bigrams; g.d.input_lengths = nullptr; g.d.label_lengths = nullptr;
-    g.d.progress = 0;
+    g.d.concurrent = 0;
     g.grad_loss = grad_loss; g.per_utterance = per_utterance; g.scale = scale;
     g.grad_out = grad_out; g.gstride_t = gstride_t; g.gstride_b = gstride_b;
     return check_cuda(launch_gradient(g, w, workspace, static_cast<cudaStream_t>(stream_)), "gradient kernel");
@@ -315,7 +288,7 @@ int b200ctc_ln_backward(int kind, const float *z, int64_t zstride_b, int64_t zst
     g.d.kind = kind == B200CTC_KIND_CTC ? 0 : 1; g.d.B = B; g.d.T = T; g.d.V = V; g.d.Lmax = Lmax; g.d.blank = blank;
     g.d.acts = nullptr; g.d.stride_t = 0; g.d.stride_b = 0;
     g.d.labels = labels; g.d.bigrams = bigrams; g.d.input_lengths = nullptr; g.d.label_lengths = nullptr;
-    g.d.progress = 0;
+    g.d.concurrent = 0;
     g.grad_loss = grad_loss; g.per_utterance = per_utterance; g.scale = scale;
     g.grad_out = nullptr; g.gstride_t = 0; g.gstride_b = 0;
     return check_cuda(launch_ln_backward(g, ll, workspace, z, zstride_b, zstride_v, gamma, beta, dz, dzstride_b, dzstride_v, dgamma,

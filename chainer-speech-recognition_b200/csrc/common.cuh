@@ -153,25 +153,11 @@ __device__ __forceinline__ float node_posterior(float2 a, float2 b, float Ph, fl
     return (a.x * b.x) * ex2_approx((a.y + b.y) - Ph) * Pinv;
 }
 
-// ---- timeline hook (tools/step_timeline.py): first CTA start / last CTA end of a kernel, in globaltimer ns ----
-__device__ __forceinline__ long long global_ns() {
-    long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-__device__ __forceinline__ void timeline_mark(long long *tl, int kernel_slot, bool end) {
-    if (tl && threadIdx.x == 0) {
-        if (end) atomicMax(tl + 2 * kernel_slot + 1, global_ns());
-        else atomicMin(tl + 2 * kernel_slot, global_ns());
-    }
-}
-
 // ---- frame progress between the softmax/gather kernel and a concurrently running lattice kernel ----
 // Producer: called by ONE lane after a __syncwarp() that follows the warp's stores of the frame's emission row.
-__device__ __forceinline__ void signal_frame_done(unsigned char *ws, const WsLayout &w, int b, int t, bool relaxed = false) {
+__device__ __forceinline__ void signal_frame_done(unsigned char *ws, const WsLayout &w, int b, int t) {
     unsigned *p = reinterpret_cast<unsigned *>(ws + w.off_prog) + (size_t)b * w.nblk + t / kProgBlock;
-    if (relaxed) asm volatile("red.relaxed.gpu.global.add.u32 [%0], 1;" ::"l"(p) : "memory");
-    else asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(p) : "memory");
+    asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(p) : "memory");
 }
 // Consumer (whole warp): how many of the blocks blk0, blk0 + step, blk0 + 2*step, ... (up to 32, inside [0, nblk))
 // are complete, counted from the front.  Block k of an utterance with Tb frames is complete when its counter has
@@ -276,11 +262,6 @@ __device__ __forceinline__ void bulk_g2s_hint(void *dst_smem, const void *src_gm
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
                      smem_u32(dst_smem)),
                  "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
-                 : "memory");
-}
-__device__ __forceinline__ void bulk_s2g_hint(void *dst_gmem, const void *src_smem, uint32_t bytes, uint64_t policy) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(dst_gmem),
-                 "r"(smem_u32(src_smem)), "r"(bytes), "l"(policy)
                  : "memory");
 }
 // shared -> global bulk copy (bulk-group completion)

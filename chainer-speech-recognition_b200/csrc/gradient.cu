@@ -11,20 +11,11 @@
 // One warp per frame, frames handed out by a ticket counter; 128-bit streaming loads/stores.  Which
 // columns carry a posterior is looked up in a per-utterance V-bit bitmap (1 word per 32 columns, L1
 // resident), so the correction happens in registers and every gradient element is written once.
-#include <stdlib.h>
 #include "common.cuh"
 #include "kernels.h"
 #include "row_ring.cuh"
 
 namespace b200ctc {
-
-#ifdef B200CTC_EXPERIMENT
-__device__ long long *g_tl_k3 = nullptr;      // timeline hook, see common.cuh
-void gradient_set_timeline(long long *p) { cudaMemcpyToSymbol(g_tl_k3, &p, sizeof(p)); }
-#define B200CTC_TL_K3(end) timeline_mark(g_tl_k3, 3, end)
-#else
-#define B200CTC_TL_K3(end) ((void)0)
-#endif
 
 namespace {
 
@@ -216,20 +207,17 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) gradient_kernel(GradParams 
 // ---------------------------------------------------------------------------------------------
 // Store a row image that sits in shared memory at the same 16-byte phase as its destination: the aligned body as
 // one bulk copy, the <= 3 floats in front of and behind it with ordinary stores.  Called by one lane.
-__device__ __forceinline__ void store_row_image(float *dst, const float *src_sm, int V, uint64_t policy, bool hint) {
+__device__ __forceinline__ void store_row_image(float *dst, const float *src_sm, int V) {
     const int head = min(V, (4 - row_misalignment(dst)) & 3);
     const int body = (V - head) & ~3;
     for (int i = 0; i < head; ++i) dst[i] = src_sm[i];
     for (int i = head + body; i < V; ++i) dst[i] = src_sm[i];
-    if (body > 0) {
-        if (hint) bulk_s2g_hint(dst + head, src_sm + head, (uint32_t)body * 4u, policy);
-        else bulk_s2g(dst + head, src_sm + head, (uint32_t)body * 4u);
-    }
+    if (body > 0) bulk_s2g(dst + head, src_sm + head, (uint32_t)body * 4u);
     bulk_commit();
 }
 
 __global__ void __launch_bounds__(kRingThreads, 1) gradient_ring_kernel(GradParams gp, WsLayout w, unsigned char *ws,
-                                                                       int b_major, RingLayout rl, int l2_hints) {
+                                                                       int b_major, RingLayout rl) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Ring ring = ring_setup(smem_raw, rl);
     const ProblemDesc &d = gp.d;
@@ -241,11 +229,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) gradient_ring_kernel(GradPara
     const uint32_t span_max = (uint32_t)ring_row_bytes(d.V);             // where the alpha row starts in a slot
     const uint32_t ab_bytes = (uint32_t)w.Np * 8u;
     const uint32_t ab2_bytes = w.joint ? (uint32_t)w.Np2 * 8u : 0u;      // joint: + the plain-CTC lattice's alpha/beta rows
-    const uint64_t l2pol = l2_policy_evict_first();
-    const bool l2hint = (l2_hints & 1) != 0;        // row loads
-    const bool l2hint_st = (l2_hints & 4) != 0;     // row stores
     // extra region: [V + 4 floats of zeros][utterance records]
-    B200CTC_TL_K3(false);
     float *zero_row = reinterpret_cast<float *>(smem_raw + rl.off_extra);
     // the utterance records, once per CTA: a consumer's row then starts without a round trip to L2
     UttInfo *utt_sm = reinterpret_cast<UttInfo *>(zero_row + ((d.V + 4 + 3) & ~3));
@@ -274,7 +258,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) gradient_ring_kernel(GradPara
                 else { t = (int)(f / d.B); b = (int)(f % d.B); }
                 if (t >= (utt_cached ? utt_sm[b].Tb : utt[b].Tb)) {                  // :296 -- zeros, straight from smem
                     float *dst = gp.grad_out + (int64_t)t * gp.gstride_t + (int64_t)b * gp.gstride_b;
-                    store_row_image(dst, zero_row + row_misalignment(dst), d.V, l2pol, l2hint_st);
+                    store_row_image(dst, zero_row + row_misalignment(dst), d.V);
                 } else {
                     need = true;
                 }
@@ -293,8 +277,8 @@ __global__ void __launch_bounds__(kRingThreads, 1) gradient_ring_kernel(GradPara
                     ring.meta[s].b = b; ring.meta[s].t = t; ring.meta[s].kind = 0; ring.meta[s].off = off;
                     ring_publish(ring, s, myq);
                     mbar_arrive_expect_tx(&ring.full[s], span + 2 * ab_bytes + 2 * ab2_bytes);
-                    if (l2hint) bulk_g2s_hint(ring.slot(s), src - off, span, &ring.full[s], l2pol);
-                    else bulk_g2s(ring.slot(s), src - off, span, &ring.full[s]);
+                    // no L2 hint: evict-first on these loads measured 2 us slower here (unlike kernel 1)
+                    bulk_g2s(ring.slot(s), src - off, span, &ring.full[s]);
                     bulk_g2s(ring.slot(s) + span_max, av_all + ((size_t)b * d.T + t) * w.Np, ab_bytes, &ring.full[s]);
                     bulk_g2s(ring.slot(s) + span_max + ab_bytes, bv_all + ((size_t)b * d.T + t) * w.Np, ab_bytes, &ring.full[s]);
                     if (w.joint) {
@@ -324,7 +308,6 @@ __global__ void __launch_bounds__(kRingThreads, 1) gradient_ring_kernel(GradPara
         }
         ring_stop(ring, q, lane);
         bulk_wait_all<0>();
-        B200CTC_TL_K3(true);
         // re-arm the queue for a possible second backward over the same workspace
         if (lane == 0) {
             __threadfence();
@@ -441,7 +424,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) gradient_ring_kernel(GradPara
             fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) {
-                store_row_image(dst, row, d.V, l2pol, l2hint_st);
+                store_row_image(dst, row, d.V);
                 bulk_wait_read<0>();             // the TMA engine has read the slot: hand it back to the producer
                 mbar_arrive(&ring.empty[s]);
             }
@@ -467,13 +450,13 @@ cudaError_t launch_gradient(const GradParams &g, const WsLayout &w, const void *
     const size_t extra = sizeof(float) * (size_t)((g.d.V + 4 + 3) & ~3) + (g.d.B <= kUttCache ? sizeof(UttInfo) * (size_t)g.d.B : 0);
     const RingLayout rl = make_ring(ring_row_bytes(g.d.V) + sizeof(float) * (4 * (size_t)w.Np + (w.joint ? 4 * (size_t)w.Np2 : 0)), extra);
     if (ring_usable(g.d.acts, g.d.stride_t, g.d.stride_b, g.d.V, rl) &&
-        ring_usable(g.grad_out, g.gstride_t, g.gstride_b, g.d.V, rl) && !knobs().no_tma_k3) {
+        ring_usable(g.grad_out, g.gstride_t, g.gstride_b, g.d.V, rl)) {
         long long ctas = (frames + kTicketBatch - 1) / kTicketBatch;
         if (ctas > sm_count()) ctas = sm_count();
         if (ctas < 1) ctas = 1;
         cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void *>(gradient_ring_kernel), rl.total);
         if (e != cudaSuccess) return e;
-        gradient_ring_kernel<<<(int)ctas, kRingThreads, rl.total, stream>>>(g, w, wsb, b_major, rl, knobs().l2_hints);
+        gradient_ring_kernel<<<(int)ctas, kRingThreads, rl.total, stream>>>(g, w, wsb, b_major, rl);
         return cudaGetLastError();
     }
     const int per_warp = w.Np + ((w.Umax + 3) & ~3) + (w.joint ? w.Np2 : 0);

@@ -4,9 +4,7 @@
 // has to stay well below that.  Everything that does not change between calls is looked up once:
 //   * the SM count of each device (cudaDeviceGetAttribute is a driver round trip),
 //   * the opt-in dynamic shared memory size and carve-out preference of each kernel (cudaFuncSetAttribute is only
-//     called again when a launch needs MORE than what was granted before),
-//   * the environment switches (read at first use, never again).
-#include <stdlib.h>
+//     called again when a launch needs MORE than what was granted before).
 #include <mutex>
 
 #include "kernels.h"
@@ -64,28 +62,6 @@ cudaError_t ensure_dynamic_smem(const void *func, size_t bytes) {
     }
     if (slot && bytes > slot->granted) slot->granted = bytes > 48 * 1024 ? bytes : 48 * 1024;
     return cudaSuccess;
-}
-
-const Knobs &knobs() {
-    static Knobs k;
-    static std::once_flag once;
-    std::call_once(once, [] {
-        k.no_tma = getenv("B200CTC_NO_TMA") != nullptr;
-        if (const char *e = getenv("B200CTC_LN_GROUP")) k.ln_group = atoi(e) > 0 ? atoi(e) : 0;      // tile order of the fused-LN kernels
-#ifdef B200CTC_EXPERIMENT
-        k.no_tma_k1 = getenv("B200CTC_NO_TMA_K1") != nullptr;
-        k.no_tma_k3 = getenv("B200CTC_NO_TMA_K3") != nullptr;
-        k.gram_k3 = getenv("B200CTC_GRAM_K3") != nullptr;
-        k.lat_nostore = getenv("B200CTC_LAT_NOSTORE") != nullptr;
-        if (const char *e = getenv("B200CTC_LAT_STAGES")) k.lat_stages = atoi(e) < 2 ? 2 : atoi(e);
-        if (const char *e = getenv("B200CTC_RING_KB")) k.ring_kb = atoi(e);
-        if (const char *e = getenv("B200CTC_DBG_PROGRESS")) k.dbg_progress = atoi(e);
-        if (const char *e = getenv("B200CTC_LAT_K")) k.lat_k = atoi(e);
-        if (const char *e = getenv("B200CTC_LAT_CH")) k.lat_ch = atoi(e);
-        if (const char *e = getenv("B200CTC_L2_HINTS")) k.l2_hints = atoi(e);
-#endif
-    });
-    return k;
 }
 
 }  // namespace b200ctc

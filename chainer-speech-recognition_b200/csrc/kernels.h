@@ -11,9 +11,8 @@ struct ProblemDesc {
     const float *acts;
     int64_t stride_t, stride_b;
     const int32_t *labels, *bigrams, *input_lengths, *label_lengths;
-    int progress;   // bit 0: the lattice kernel runs concurrently with the softmax/gather kernel -- the latter signals
-                    //        every finished frame (progress counters) and the former waits on them;
-                    // bit 1: tickets walk the frames from both ends (what the concurrent lattice wants)
+    int concurrent; // the lattice kernel runs next to the softmax/gather kernel: the latter signals every finished
+                    // frame (progress counters), the former waits on them, and tickets walk the frames from both ends
 };
 
 // kernel 1: fused log-softmax statistics + label gather (+ optional greedy argmax)
@@ -35,16 +34,6 @@ int current_device();
 int sm_count();                                                        // per device
 // opt-in dynamic shared memory + maximum carve-out for `func`; cudaFuncSetAttribute only when more is needed than before
 cudaError_t ensure_dynamic_smem(const void *func, size_t bytes);
-// environment switches, read once per process.  B200CTC_NO_TMA forces the plain-LDG row kernels (tests of the fallback);
-// the rest are experiment knobs that only exist in -DB200CTC_EXPERIMENT builds (tools/), never in the product library
-struct Knobs {
-    bool no_tma = false;
-    bool no_tma_k1 = false, no_tma_k3 = false, gram_k3 = false, lat_nostore = false;
-    int lat_stages = 0, ring_kb = 0, dbg_progress = -1, lat_k = 0, lat_ch = 0, ln_group = 0;
-    int l2_hints = 2;          // bit 0: gradient kernel, bit 1: softmax/gather kernel mark their row streams evict-first in L2
-                               // (measured: the forward pass gains 4 us, the gradient kernel loses 2 -- only the first is on)
-};
-const Knobs &knobs();
 
 // kernel 2: alpha/beta lattice recursion (+ symbol-table CTAs, + batch loss reduction by the last CTA)
 struct LatticeParams {
@@ -56,7 +45,6 @@ struct LatticeParams {
     float loss_scale;
     int W;                   // warps per direction
     int S;                   // pipeline stages
-    int dbg_nostore;         // timing experiment: skip the alpha/beta row stores
     int second;              // 1: this is the plain-CTC lattice of a joint call -- no symbol-table CTAs, its own
                              //    completion counter, and its loss is ADDED to loss_per_utt (the Gram-CTC launch,
                              //    earlier in the stream, has written its own there) before the batch is reduced

@@ -45,22 +45,11 @@
 //
 // The same launch carries B extra CTAs that build the gradient kernel's symbol tables (prep.cuh) while
 // the recursion runs, and the last alpha CTA to finish reduces the batch loss in a fixed order.
-#include <stdlib.h>
 #include "common.cuh"
 #include "kernels.h"
 #include "prep.cuh"
 
 namespace b200ctc {
-
-#ifdef B200CTC_EXPERIMENT
-__device__ long long *g_tl_k2 = nullptr;      // timeline hook, see common.cuh
-void lattice_set_timeline(long long *p) { cudaMemcpyToSymbol(g_tl_k2, &p, sizeof(p)); }
-__device__ long long *g_lat_dbg = nullptr;   // profiling hook (tools/lattice_timeline.py): per-warp cycle breakdown
-__device__ __forceinline__ long long gtime() { long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-#define B200CTC_TL_K2(slot, end) timeline_mark(g_tl_k2, slot, end)
-#else
-#define B200CTC_TL_K2(slot, end) ((void)0)
-#endif
 
 namespace {
 
@@ -387,22 +376,12 @@ __device__ __forceinline__ void run_direction(LaneState<K, GRAM> &st, const DirP
     int stage = 0;
     uint32_t wrap = 0;
     bool early = false;                                       // the wait for the coming chunk already succeeded
-#ifdef B200CTC_EXPERIMENT
-    long long acc_wait = 0, acc_work = 0, acc_tail = 0;
-    const bool prof = (g_lat_dbg != nullptr) && lane == 0 && blockIdx.x < 64;
-#else
-    constexpr bool prof = false;
-    long long acc_wait = 0, acc_work = 0, acc_tail = 0;
-#endif
     for (int ch = 0; ch < nchunks; ++ch) {
         const int cnt = min(CH, n - ch * CH);
-        long long tq0 = 0, tq1 = 0, tq2 = 0;
-        if (prof) tq0 = clock64();
         if (!early) {
             if (ch == 0) mbar_wait_backoff(&wait_bar[stage], wrap & 1u);
             else mbar_wait(&wait_bar[stage], wrap & 1u);
         }
-        if (prof) { tq1 = clock64(); acc_wait += tq1 - tq0; }
 
         const uint32_t lp_s = after_wait(pp.lp + (uint32_t)stage * stage_bytes);
         const uint32_t bin = after_wait(has_prev ? pp.bnd + (uint32_t)((w - 1) * S + stage) * bnd_chunk_bytes : pp.bnd_none);
@@ -430,21 +409,10 @@ __device__ __forceinline__ void run_direction(LaneState<K, GRAM> &st, const DirP
         // pull the mantissas back into [1,2): they moved by at most 2^-CH .. 3^CH since the last time
 #pragma unroll
         for (int r = 0; r < K; ++r) renorm_pair(st.m[r], st.e[r]);
-        if (prof) { tq2 = clock64(); acc_work += tq2 - tq1; }
         __syncwarp();
         if (lane == 0) mbar_arrive(&done_bar[stage]);
         stage = nstage; wrap = nwrap;
-        if (prof) acc_tail += clock64() - tq2;
     }
-#ifdef B200CTC_EXPERIMENT
-    if (prof) {
-        long long *o = g_lat_dbg + ((size_t)blockIdx.x * 32 + w) * 8;
-        o[0] = acc_wait; o[1] = 0; o[2] = 0; o[3] = acc_work; o[4] = acc_tail; o[5] = nchunks;
-        o[6] = gtime();
-    }
-#else
-    (void)acc_wait; (void)acc_work; (void)acc_tail;
-#endif
 }
 
 template <int K, bool GRAM>
@@ -538,7 +506,6 @@ __global__ void __launch_bounds__(32 * (MAXW + 1)) lattice_kernel(LatticeParams 
     }
     const int b = blockIdx.x >> 1;
     const int dir = blockIdx.x & 1;                        // 0: alpha, 1: beta
-    B200CTC_TL_K2(1 + dir, false);
     const int W = p.W, S = p.S;
     // warps [0,W): recursion, warp W: I/O.  Read through a shuffle so that the compiler knows the value is
     // warp-uniform: every branch below is then a uniform branch, and the recursion's shuffles need no divergence
@@ -583,21 +550,17 @@ __global__ void __launch_bounds__(32 * (MAXW + 1)) lattice_kernel(LatticeParams 
         c.out_g = dir == 0 ? av : bv;
         c.Wlp = p.w.W; c.Np = p.w.Np; c.Nb = Nb; c.W = W; c.S = S; c.boff = p.w.boff;
         if (io) {
-            if (dir == 0) io_direction<false, CH>(pp, c, 0, Tb, lane, p.ws, p.w, b, (d.progress & 1) != 0, &hdr->stalled);
-            else          io_direction<true, CH>(pp, c, Tb - 1, Tb, lane, p.ws, p.w, b, (d.progress & 1) != 0, &hdr->stalled);
+            if (dir == 0) io_direction<false, CH>(pp, c, 0, Tb, lane, p.ws, p.w, b, d.concurrent != 0, &hdr->stalled);
+            else          io_direction<true, CH>(pp, c, Tb - 1, Tb, lane, p.ws, p.w, b, d.concurrent != 0, &hdr->stalled);
         } else {
             LaneState<K, GRAM> st;
             init_lane<K, GRAM>(st, d, b, Lb, Nb, dir == 1, 32 * w + lane);
-#ifdef B200CTC_EXPERIMENT
-            if (p.dbg_nostore) st.valid = 0u;            // timing experiment only (B200CTC_LAT_NOSTORE): results are garbage
-#endif
             if (dir == 0) run_direction<K, GRAM, false, CH>(st, pp, c, 0, Tb, w, lane);         // alpha: frames 0 .. Tb-1
             else          run_direction<K, GRAM, true, CH>(st, pp, c, Tb - 1, Tb, w, lane);     // beta:  frames Tb-1 .. 0
         }
     }
     if (dir == 1) {                                        // the beta CTA is done
         __syncthreads();
-        B200CTC_TL_K2(2, true);
         return;
     }
     __threadfence_block();
@@ -656,30 +619,37 @@ __global__ void __launch_bounds__(32 * (MAXW + 1)) lattice_kernel(LatticeParams 
         if (*reinterpret_cast<volatile unsigned *>(&hdr->stalled) != 0u) acc = (double)__int_as_float(0x7fc00000);
         if (lane == 0) *p.loss_reduced = (float)(acc * (double)p.loss_scale);
     }
-    B200CTC_TL_K2(1, true);
 }
 
-template <int K, bool GRAM, int MAXW, int CH>
-cudaError_t launch_w(const LatticeParams &p, size_t smem, cudaStream_t stream) {
-    auto kern = lattice_kernel<K, GRAM, MAXW, CH>;
-    // the SM's L1/shared split is chosen per kernel: ask for the maximum so that a lattice CTA and a ring CTA of the
-    // softmax/gather kernel (which asks for the same) can share an SM
-    cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void *>(kern), smem);
-    if (e != cudaSuccess) return e;
-    kern<<<(p.second ? 2 : 3) * p.d.B, 32 * (p.W + 1), smem, stream>>>(p);
-    return cudaGetLastError();
-}
+using LatticeKernel = void (*)(LatticeParams);
 
-// instantiated combinations: few warps -> 16-frame chunks; many warps -> shorter chunks (see kMaxStages)
+// the instantiation with MAXW compute warps and the chunk length CH out of CHS, or nullptr
+template <int K, bool GRAM, int MAXW, int... CHS>
+LatticeKernel with_chunk(int CH) {
+    LatticeKernel kern = nullptr;
+    ((kern = CH == CHS ? lattice_kernel<K, GRAM, MAXW, CHS> : kern), ...);
+    return kern;
+}
 template <int K, bool GRAM>
-cudaError_t launch_one(const LatticeParams &p, int CH, size_t smem, cudaStream_t stream) {
-    if (p.W <= 3)
-        return CH == 16 ? launch_w<K, GRAM, 3, 16>(p, smem, stream)
-                        : (CH == 8 ? launch_w<K, GRAM, 3, 8>(p, smem, stream) : launch_w<K, GRAM, 3, 4>(p, smem, stream));
-    if (p.W <= 7)
-        return CH == 16 ? launch_w<K, GRAM, 7, 16>(p, smem, stream)
-                        : (CH == 8 ? launch_w<K, GRAM, 7, 8>(p, smem, stream) : launch_w<K, GRAM, 7, 4>(p, smem, stream));
-    return CH >= 8 ? launch_w<K, GRAM, kMaxWarpsPerDir, 8>(p, smem, stream) : launch_w<K, GRAM, kMaxWarpsPerDir, 4>(p, smem, stream);
+LatticeKernel any_tier(int W, int CH) {
+    if (W <= 3) return with_chunk<K, GRAM, 3, 16>(CH);
+    if (W <= 7) return with_chunk<K, GRAM, 7, 16, 8, 4>(CH);
+    return with_chunk<K, GRAM, kMaxWarpsPerDir, 8, 4>(CH);
+}
+// The instantiated kernels: exactly the (K, W, CH) that launch_lattice's plan can reach.  Up to 3 warps the chunk is
+// always 16 frames (CHmin); a chunk starts at 8 frames beyond 7 warps or 3 nodes per lane; CTC K = 4 means more than
+// 512 nodes, so W >= 5; Gram-CTC K = 6 means more than 1536 nodes, so W >= 9.  nullptr: no kernel for the plan.
+LatticeKernel lattice_kernel_for(int kind, int K, int W, int CH) {
+    if (kind == 0) {
+        if (K == 2) return any_tier<2, false>(W, CH);
+        if (K == 4 && W > 3)
+            return W <= 7 ? with_chunk<4, false, 7, 8, 4>(CH) : with_chunk<4, false, kMaxWarpsPerDir, 8, 4>(CH);
+        return nullptr;
+    }
+    if (K == 1) return any_tier<1, true>(W, CH);
+    if (K == 3) return any_tier<3, true>(W, CH);
+    if (K == 6 && W > 7) return with_chunk<6, true, kMaxWarpsPerDir, 8, 4>(CH);
+    return nullptr;
 }
 
 constexpr size_t kLatticeSmemBudget = 224 * 1024;
@@ -694,10 +664,6 @@ WsLayout ctc_view_of_joint(const WsLayout &w) {
     return v;
 }
 
-#ifdef B200CTC_EXPERIMENT
-void lattice_set_debug(long long *p) { cudaMemcpyToSymbol(g_lat_dbg, &p, sizeof(p)); }
-#endif
-
 int lattice_max_nodes(int kind) { return kind == 0 ? 32 * 4 * kMaxWarpsPerDir - 3 : 32 * 6 * kMaxWarpsPerDir; }      // - 3: phantom nodes of the 4-node mapping
 
 cudaError_t launch_lattice(LatticeParams p, cudaStream_t stream, int *status, bool concurrent, size_t *smem_out,
@@ -711,13 +677,6 @@ cudaError_t launch_lattice(LatticeParams p, cudaStream_t stream, int *status, bo
     int K;
     if (kind == 0) K = (Nmax <= 32 * 2 * 8) ? 2 : 4;
     else K = (Nmax <= 32 * kGenericMaxWarps) ? 1 : ((Nmax <= 32 * 3 * kMaxWarpsPerDir) ? 3 : 6);
-#ifdef B200CTC_EXPERIMENT
-    if (kind == 1 && knobs().gram_k3 && K == 1) K = 3;
-    if (knobs().lat_k > 0 && (Nmax + 32 * knobs().lat_k - 1) / (32 * knobs().lat_k) <= kMaxWarpsPerDir) {
-        if (kind == 0 && (knobs().lat_k == 2 || knobs().lat_k == 4 || knobs().lat_k == 8)) K = knobs().lat_k;
-        if (kind == 1 && (knobs().lat_k == 3 || knobs().lat_k == 6 || (knobs().lat_k == 1 && Nmax <= 32 * kGenericMaxWarps))) K = knobs().lat_k;
-    }
-#endif
     const int W = (Nmax + (kind == 0 && K == 4 ? 3 : 0) + 32 * K - 1) / (32 * K);      // + the reversed direction's phantom nodes
     if (W > kMaxWarpsPerDir) { *status = 2; return cudaSuccess; }
     const int PAD = kind == 0 ? 2 : 7;
@@ -735,10 +694,6 @@ cudaError_t launch_lattice(LatticeParams p, cudaStream_t stream, int *status, bo
     const size_t budget = concurrent ? (size_t)64 * 1024 : kLatticeSmemBudget;
     while (CH > CHmin && plan_smem(p.w.W, W, want, PAD, CH).total > budget) CH >>= 1;
     int S = want;
-#ifdef B200CTC_EXPERIMENT
-    if (knobs().lat_stages >= 2) S = knobs().lat_stages;
-    if (knobs().lat_ch == 16 || knobs().lat_ch == 8 || knobs().lat_ch == 4) CH = (W > 7 && knobs().lat_ch == 16) ? 8 : knobs().lat_ch;
-#endif
     while (S > 2 && plan_smem(p.w.W, W, S, PAD, CH).total > kLatticeSmemBudget) --S;
     const SmemPlan sp = plan_smem(p.w.W, W, S, PAD, CH);
     if (sp.total > kLatticeSmemBudget) { *status = 2; return cudaSuccess; }
@@ -746,18 +701,17 @@ cudaError_t launch_lattice(LatticeParams p, cudaStream_t stream, int *status, bo
     const size_t prep = p.second ? 0 : prep_smem_bytes(kind, p.d.Lmax, p.w.nwords);
     if (prep > smem) smem = prep;
     if (smem > 227 * 1024) { *status = 2; return cudaSuccess; }
+    const LatticeKernel kern = lattice_kernel_for(kind, K, W, CH);
+    if (!kern) { *status = 2; return cudaSuccess; }
     p.W = W; p.S = S;
-    p.dbg_nostore = 0;
-#ifdef B200CTC_EXPERIMENT
-    p.dbg_nostore = knobs().lat_nostore ? 1 : 0;
-#endif
     if (smem_out) *smem_out = smem;
     if (!launch) return cudaSuccess;
-    if (kind == 0)
-        return K == 2 ? launch_one<2, false>(p, CH, smem, stream)
-                      : (K == 4 ? launch_one<4, false>(p, CH, smem, stream) : launch_one<8, false>(p, CH, smem, stream));
-    if (K == 1) return launch_one<1, true>(p, CH, smem, stream);
-    return K == 3 ? launch_one<3, true>(p, CH, smem, stream) : launch_one<6, true>(p, CH, smem, stream);
+    // the SM's L1/shared split is chosen per kernel: ask for the maximum so that a lattice CTA and a ring CTA of the
+    // softmax/gather kernel (which asks for the same) can share an SM
+    cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void *>(kern), smem);
+    if (e != cudaSuccess) return e;
+    kern<<<(p.second ? 2 : 3) * p.d.B, 32 * (p.W + 1), smem, stream>>>(p);
+    return cudaGetLastError();
 }
 
 }  // namespace b200ctc

@@ -54,18 +54,6 @@ constexpr int kLnMetaRing = 64;                            // >= ring slots: a p
 constexpr int kLnMaxCols = 32 * kLnWarps;                  // emission columns one tile pass can gather: one per compute thread
 constexpr int kLnJointPre = 4;                             // joint backward: plain-CTC alpha/beta items a thread requests ahead
 
-#ifdef B200CTC_EXPERIMENT
-// phase timers (tools/ln_phases.py): per CTA and warp, cycles per phase of the tile loop
-__device__ long long *g_ln_dbg = nullptr;
-#define LN_T_DECL long long *const ln_dbg = g_ln_dbg; long long ln_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}; long long ln_last = ln_dbg ? clock64() : 0
-#define LN_T(i) do { if (ln_dbg) { const long long now_ = clock64(); ln_acc[i] += now_ - ln_last; ln_last = now_; } } while (0)
-#define LN_T_FLUSH(w) do { if (ln_dbg && lane == 0) { for (int i_ = 0; i_ < 8; ++i_) ln_dbg[((size_t)blockIdx.x * 16 + (w)) * 8 + i_] = ln_acc[i_]; } } while (0)
-#else
-#define LN_T_DECL
-#define LN_T(i) ((void)0)
-#define LN_T_FLUSH(w) ((void)0)
-#endif
-
 // Everything a tile's consumers need to know about it, fetched by the producer lane (a dependent global load at the
 // start of a tile would stall all fifteen compute warps for its round trip)
 struct LnTileMeta {
@@ -142,29 +130,22 @@ __device__ __forceinline__ float4 lds128(uint32_t addr) {
     asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
     return v;
 }
-#ifdef B200CTC_EXPERIMENT
-#define LN_WATCHDOG(site, it_) do { if (++(it_) > (1ll << 25)) { printf("LN HANG site %d block %d thread %d\n", site, (int)blockIdx.x, (int)threadIdx.x); __trap(); } } while (0)
-#else
-#define LN_WATCHDOG(site, it_) ((void)(it_))
-#endif
 // For the lanes of the producer warp, which share ONE warp while running different loops: a suspending wait in one
 // lane would put the others to sleep with it, so these lanes only probe (test_wait returns at once) and nap.
-__device__ __forceinline__ void mbar_poll(uint64_t *bar, uint32_t parity, int site = 0) {
-    [[maybe_unused]] long long it_ = 0;
-    (void)it_; (void)site;
-    while (!mbar_test_wait(bar, parity)) { __nanosleep(40); LN_WATCHDOG(site, it_); }
+__device__ __forceinline__ void mbar_poll(uint64_t *bar, uint32_t parity) {
+    while (!mbar_test_wait(bar, parity)) __nanosleep(40);
 }
 __device__ __forceinline__ void bar_compute() { asm volatile("bar.sync 1, %0;" ::"n"(32 * kLnWarps) : "memory"); }
 
 // ---- tile order ----
-inline int ln_group() { return knobs().ln_group > 0 ? knobs().ln_group : kLnGroup; }
 // A tile takes 32 bytes out of every row of z, rows 4*T bytes apart: what DRAM sees depends on which tiles are in flight
 // TOGETHER.  Groups of G consecutive 8-frame blocks of one utterance get consecutive tickets, so the SMs working on them
 // touch 32*G contiguous bytes of every row at about the same time.  G = 4 (one 128-byte line) is the measured best:
-// 8 and 16 change nothing, 32 and whole rows are slower (B200CTC_LN_GROUP in the experiment build) -- longer groups
+// 8 and 16 change nothing, 32 and whole rows are slower (measured with a tuning switch that is in git history) -- longer groups
 // serve the lattice kernel in coarser lumps and balance the variable-length utterances worse.  Groups walk the time axis from
 // both ends (the alpha CTAs of the lattice kernel consume frames in ascending, the beta CTAs in descending order).
-__device__ __forceinline__ bool ln_tile_of_ticket(unsigned f, int B, int nTB, bool two_ended, int G, int &b, int &tb) {
+__device__ __forceinline__ bool ln_tile_of_ticket(unsigned f, int B, int nTB, bool two_ended, int &b, int &tb) {
+    constexpr int G = kLnGroup;
     const int sub = (int)(f % (unsigned)G);
     const unsigned q = f / (unsigned)G;
     b = (int)(q % (unsigned)B);
@@ -268,7 +249,7 @@ __device__ __forceinline__ float2 ln_emission_pair(float x, float la, float lb) 
 }
 
 struct LnParams {
-    ProblemDesc d;                  // d.acts unused; kind/B/T/V/Lmax/blank/labels/bigrams/lengths/progress as usual
+    ProblemDesc d;                  // d.acts unused; kind/B/T/V/Lmax/blank/labels/bigrams/lengths/concurrent as usual
     WsLayout w;
     unsigned char *ws;
     const float *z;                 // (B, V, T): element (b, v, t) at z[b*zs_b + v*zs_v + t]
@@ -279,7 +260,6 @@ struct LnParams {
     int K;                          // boxes per tile = ceil(V / 240)
     int nTB;                        // 8-frame blocks = ceil(T / 8)
     int R;                          // ring slots
-    int group;                      // 8-frame blocks of one utterance that get consecutive tickets (ln_tile_of_ticket)
     // backward only
     const float *grad_loss;
     int per_utterance;
@@ -304,20 +284,20 @@ __device__ __forceinline__ void ln_producer(const CUtensorMap *tmap, const CUten
     LnTileMeta *metas = reinterpret_cast<LnTileMeta *>(smem + sm.off_meta);
     WsHeader *hdr = reinterpret_cast<WsHeader *>(p.ws + p.w.off_hdr);
     const UttInfo *utt = reinterpret_cast<const UttInfo *>(p.ws + p.w.off_utt);
-    const int G = p.group;
+    constexpr int G = kLnGroup;
     const unsigned tiles = (unsigned)p.d.B * (unsigned)(((p.nTB + G - 1) / G) * G);
     const unsigned R = (unsigned)p.R;
     const int K = p.K;
     unsigned box = 0, seq = 0, n_ab = 0;             // boxes / tile records / alpha-beta loads issued by this CTA
     auto claim = [&](unsigned bx) {                  // wait until the box slot's previous occupant was released
-        if (bx >= R) mbar_poll(&empty[bx % R], ((bx / R) - 1u) & 1u, BACKWARD ? 11 : 1);
+        if (bx >= R) mbar_poll(&empty[bx % R], ((bx / R) - 1u) & 1u);
         return (int)(bx % R);
     };
     unsigned f = BACKWARD ? blockIdx.x : atomicAdd(&hdr->k1_ticket, 1u);
     while (f < tiles) {
         const unsigned fnext = BACKWARD ? f + gridDim.x : atomicAdd(&hdr->k1_ticket, 1u);     // in flight while we issue
         int b, tb;
-        const bool real = ln_tile_of_ticket(f, p.d.B, p.nTB, !BACKWARD && (p.d.progress & 2) != 0, G, b, tb);
+        const bool real = ln_tile_of_ticket(f, p.d.B, p.nTB, !BACKWARD && p.d.concurrent != 0, b, tb);
         f = fnext;
         if (!real) continue;
         const int t0 = tb * kLnTT;
@@ -351,7 +331,7 @@ __device__ __forceinline__ void ln_producer(const CUtensorMap *tmap, const CUten
             const int nfr = min(kLnTT, p.d.T - t0);
             const uint32_t bytes = (uint32_t)nfr * (uint32_t)p.w.Np * 8u;
             const uint32_t fbytes = (uint32_t)min(kLnTT, p.Tq - t0) * 4u;          // 16 or 32 bytes
-            if (n_ab > 0) mbar_poll(&abbar[1], (n_ab - 1u) & 1u, 12);
+            if (n_ab > 0) mbar_poll(&abbar[1], (n_ab - 1u) & 1u);
             ++n_ab;
             const size_t fo = (size_t)b * p.Tq + t0;                                // 16-byte aligned rows of the per-frame arrays
             const float2 *av = reinterpret_cast<const float2 *>(p.ws + p.w.off_av) + ((size_t)b * p.d.T + t0) * p.w.Np;
@@ -382,9 +362,7 @@ __device__ __forceinline__ void ln_signaller(const LnParams &p, unsigned char *s
     LnSignalFifo *ff = reinterpret_cast<LnSignalFifo *>(smem + sm.off_fifo);
     unsigned taken = 0;
     for (;;) {
-        [[maybe_unused]] long long it_ = 0;
-        (void)it_;
-        while (*reinterpret_cast<volatile unsigned *>(&ff->head) == taken) { __nanosleep(100); LN_WATCHDOG(2, it_); }
+        while (*reinterpret_cast<volatile unsigned *>(&ff->head) == taken) __nanosleep(100);
         __threadfence_block();
         const volatile int *e = reinterpret_cast<volatile int *>(&ff->entry[taken % kLnFifo]);
         const int b = e[0], blk = e[1], n = e[2];
@@ -395,9 +373,7 @@ __device__ __forceinline__ void ln_signaller(const LnParams &p, unsigned char *s
     }
 }
 __device__ __forceinline__ void ln_signal_push(LnSignalFifo *ff, unsigned &pushed, int b, int blk, int n) {
-    [[maybe_unused]] long long it_ = 0;
-    (void)it_;
-    while (pushed - *reinterpret_cast<volatile unsigned *>(&ff->tail) >= (unsigned)kLnFifo) { __nanosleep(64); LN_WATCHDOG(3, it_); }
+    while (pushed - *reinterpret_cast<volatile unsigned *>(&ff->tail) >= (unsigned)kLnFifo) __nanosleep(64);
     ff->entry[pushed % kLnFifo] = make_int4(b, blk, n, 0);
     __threadfence_block();                           // the tile's stores (ordered by the CTA barrier) and the entry, then the head
     *reinterpret_cast<volatile unsigned *>(&ff->head) = ++pushed;
@@ -417,12 +393,9 @@ __device__ __forceinline__ void ln_storer(const CUtensorMap *tmap_out, const LnP
     unsigned slot = 0;
     for (unsigned n = 0;; ++n) {
         bool stop = false;
-        [[maybe_unused]] long long it_ = 0;
-        (void)it_;
         while (!mbar_test_wait(outbar, n & 1u)) {
             if (*total == n + 1u) { stop = true; break; }
             __nanosleep(40);
-            LN_WATCHDOG(13, it_);
         }
         if (stop) break;
         const LnTileMeta m = metas[n % kLnMetaRing];
@@ -454,14 +427,8 @@ struct SlotIter {
     unsigned slot, phase;
     __device__ __forceinline__ void next(unsigned R) { if (++slot == R) { slot = 0; phase ^= 1u; } }
 };
-__device__ __forceinline__ void mbar_spin(uint64_t *bar, uint32_t parity, int site = 0) {
-    [[maybe_unused]] long long it_ = 0;
-    (void)it_; (void)site;
-#ifdef B200CTC_EXPERIMENT
-    while (!mbar_test_wait(bar, parity)) { LN_WATCHDOG(site, it_); }     // watchdog build: probe, count, report
-#else
+__device__ __forceinline__ void mbar_spin(uint64_t *bar, uint32_t parity) {
     while (!mbar_try_wait(bar, parity)) { }                              // try_wait suspends the thread in hardware while it waits
-#endif
 }
 
 
@@ -504,7 +471,7 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
     LnSignalFifo *fifo = reinterpret_cast<LnSignalFifo *>(smem + sm.off_fifo);
     if (w == kLnWarps) {
         if (lane == 0) ln_producer<false>(&tmap, nullptr, p, smem, sm);
-        else if (lane == 1 && (d.progress & 1)) ln_signaller(p, smem, sm);
+        else if (lane == 1 && d.concurrent) ln_signaller(p, smem, sm);
         return;
     }
     const int r = lane >> 1, h = lane & 1;
@@ -522,10 +489,8 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
 
     SlotIter it = {0u, 0u};
     unsigned seq = 0, pushed = 0;
-    LN_T_DECL;
     for (;;) {
-        mbar_spin(&full[it.slot], it.phase, 4);
-        LN_T(0);
+        mbar_spin(&full[it.slot], it.phase);
         const LnTileMeta m = metas[seq % kLnMetaRing];
         ++seq;
         if (m.kind < 0) break;
@@ -553,7 +518,7 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
             for (int k = 0; k < KMAX; ++k) {
                 z[k] = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (k < K) {
-                    if (k > 0) mbar_spin(&full[s.slot], s.phase, 5);
+                    if (k > 0) mbar_spin(&full[s.slot], s.phase);
                     const uint32_t box = ring + s.slot * kLnBoxBytes;
                     z[k] = lds128(box + lane_off);
                     if (sym_box == k) { zs0 = lds128(box + sym_off); zs1 = lds128(box + sym_off + 16); }
@@ -564,7 +529,6 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
             }
             it = s;
         }
-        LN_T(1);
 
         // ---- round 1: mean and centred second moment of every frame (asr/nn/layernorm.py:41-44) ----
         Moments mo[4];
@@ -589,12 +553,7 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
         int fih;
         const Moments mr = reduce_frames16(mo[0], mo[1], mo[2], mo[3], lane, merge_moments, fih);
         if (lane < 8) { const float v3[3] = {mr.n, mr.mean, mr.m2}; red_store<3>(red, 4 * h + fih, w, v3); }
-        LN_T(2);
-#ifdef B200CTC_EXPERIMENT
-        if (d.progress & 64) continue;        // streaming-rate experiment: the tile is in registers, the boxes are free again -- next
-#endif
         bar_compute();
-        LN_T(3);
         if (w < kLnTT) {
             Moments a;
             const float *src = red + (w * 16 + (lane & 15)) * 4;
@@ -612,7 +571,6 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
             }
         }
         bar_compute();
-        LN_T(4);
 
         // ---- round 2: a = gamma * (z - mean) * rstd + beta (asr/nn/nn.py:265), in place; softmax statistics ----
         MaxSum ms[4];
@@ -643,7 +601,6 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
         }
         const MaxSum sr = reduce_frames16(ms[0], ms[1], ms[2], ms[3], lane, merge_maxsum, fih);
         if (lane < 8) { const float v2[2] = {sr.m, sr.s}; red_store<2>(red, 4 * h + fih, w, v2); }
-        LN_T(5);
         bar_compute();
         if (w < kLnTT) {
             MaxSum a;
@@ -662,7 +619,6 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
             }
         }
         bar_compute();
-        LN_T(6);
 
         // ---- emission probabilities of the lattice's symbols ----
         if (tid < ncol) {
@@ -682,11 +638,9 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
             }
         }
         bar_compute();            // rows stored; also protects red/tot against the next tile
-        if (tid == 0 && (d.progress & 1)) ln_signal_push(fifo, pushed, m.b, m.t0 / kProgBlock, min(kLnTT, Tb - m.t0));
-        LN_T(7);
+        if (tid == 0 && d.concurrent) ln_signal_push(fifo, pushed, m.b, m.t0 / kProgBlock, min(kLnTT, Tb - m.t0));
     }
-    if (tid == 0 && (d.progress & 1)) ln_signal_push(fifo, pushed, -1, 0, 0);
-    LN_T_FLUSH(w);
+    if (tid == 0 && d.concurrent) ln_signal_push(fifo, pushed, -1, 0, 0);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -763,10 +717,8 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
 
     SlotIter it = {0u, 0u};
     unsigned seq = 0, n_ab = 0;
-    LN_T_DECL;
     for (;;) {
-        mbar_spin(&full[it.slot], it.phase, 14);
-        LN_T(0);
+        mbar_spin(&full[it.slot], it.phase);
         const LnTileMeta m = metas[seq % kLnMetaRing];
         ++seq;
         if (m.kind < 0) {
@@ -818,9 +770,8 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
             const int i = tid + q * 32 * kLnWarps;
             ab2[q] = (wl.joint && i < nitems) ? ctc_partner_ab(i) : make_float4(0.f, SENT, 0.f, SENT);
         }
-        mbar_spin(&abbar[0], n_ab & 1u, 15);
+        mbar_spin(&abbar[0], n_ab & 1u);
         ++n_ab;
-        LN_T(2);
         // per-frame constants of this thread's four frames (staged by the producer)
         float rs[4], mur[4], nl[4];
 #pragma unroll
@@ -878,7 +829,6 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
             }
         }
         bar_compute();
-        LN_T(3);
 
         // ---- sweep 1: g = softmax * sc - posterior;  dn = g * gamma;  per-frame sums of dn and dn * n ----
         float4 dn[KMAX];
@@ -891,7 +841,7 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
             for (int k = 0; k < KMAX; ++k) {
                 dn[k] = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (k < K) {
-                    if (k > 0) mbar_spin(&full[s.slot], s.phase, 16);
+                    if (k > 0) mbar_spin(&full[s.slot], s.phase);
                     const float4 zq = lds128(ring + s.slot * kLnBoxBytes + lane_off);
                     s.next(R);
                     const int v = kLnBoxRows * k + vrow;
@@ -919,7 +869,6 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
             }
             it = s;
         }
-        LN_T(4);
         // ---- the two per-frame sums of LayerNormalization's backward (asr/nn/layernorm.py:48-60) ----
         int fih;
         const Pair2 pr = reduce_frames16(Pair2{s1[0], s2[0]}, Pair2{s1[1], s2[1]}, Pair2{s1[2], s2[2]}, Pair2{s1[3], s2[3]}, lane,
@@ -935,7 +884,6 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
             if (lane == 0) { tot[w * 8 + 0] = a * inv_v; tot[w * 8 + 1] = b * inv_v; }
         }
         bar_compute();
-        LN_T(5);
         float c1r[4], c2r[4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) { c1r[j] = -tot[(4 * h + j) * 8 + 0] * rs[j]; c2r[j] = -tot[(4 * h + j) * 8 + 1] * rs[j]; }
@@ -959,12 +907,9 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
             }
         }
         fence_proxy_async_smem();     // the images are read by the TMA engine
-        LN_T(6);
         bar_compute();                // images complete; red / tot / post / tables are reused by the next tile
         if (tid == 0) mbar_arrive(&abbar[2]);      // store lane: this tile's boxes are ready
-        LN_T(7);
     }
-    LN_T_FLUSH(w);
     // ---- this CTA's share of dgamma / dbeta: one partial row per CTA ----
     const int Vp = K * kLnBoxRows;
     float *part = reinterpret_cast<float *>(p.ws + p.off_part) + (size_t)blockIdx.x * 2 * Vp + (size_t)h * Vp;
@@ -1052,10 +997,6 @@ cudaError_t launch_ln(Kern kern, int grid, const LnParams &p, const LnSmem &sm, 
 
 }  // namespace
 
-#ifdef B200CTC_EXPERIMENT
-void ln_set_debug(long long *p) { cudaMemcpyToSymbol(g_ln_dbg, &p, sizeof(p)); }
-#endif
-
 LnLayout make_ln_layout(int kind, int B, int T, int V, int Lmax) {
     LnLayout l;
     l.w = make_layout(kind, B, T, V, Lmax);
@@ -1102,7 +1043,6 @@ cudaError_t launch_ln_forward(const ProblemDesc &d, const LnLayout &ll, void *ws
         sm.R = 2 * p.K + 4;
     }
     p.R = sm.R;
-    p.group = ln_group();
     CUtensorMap map;
     if (!make_z_map(&map, z, d.B, d.T, d.V, zs_b, zs_v)) return cudaErrorInvalidValue;
     long long tiles = (long long)d.B * p.nTB;
@@ -1135,7 +1075,6 @@ cudaError_t launch_ln_backward(const GradParams &g, const LnLayout &ll, const vo
     const LnSmem sm = plan_ln_backward(ll.w);
     if (sm.R < p.K + 2) { note_failure_site("shared-memory plan"); return cudaErrorInvalidConfiguration; }
     p.R = sm.R;
-    p.group = ln_group();
     CUtensorMap map, map_dz;
     if (!make_z_map(&map, z, d.B, d.T, d.V, zs_b, zs_v)) { note_failure_site("tensor map of z"); return cudaErrorInvalidValue; }
     if (!make_z_map(&map_dz, dz, d.B, d.T, d.V, dzs_b, dzs_v)) { note_failure_site("tensor map of dz"); return cudaErrorInvalidValue; }

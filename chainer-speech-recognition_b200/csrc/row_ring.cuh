@@ -18,7 +18,6 @@
 // Requirement (checked by the host dispatcher, which otherwise uses the plain LDG kernels): at least kMinSlots
 // such spans fit in shared memory.
 #pragma once
-#include <stdlib.h>
 #include "common.cuh"
 #include "kernels.h"
 
@@ -57,20 +56,13 @@ struct RingLayout {
     size_t off_meta, off_full, off_empty, off_next, off_extra, total;
 };
 
-inline size_t ring_budget() {
-#ifdef B200CTC_EXPERIMENT
-    if (knobs().ring_kb > 0) return (size_t)knobs().ring_kb * 1024;
-#endif
-    return kRingSmemBudget;
-}
-
 // smem_reserve: shared memory to leave free on the SM for a CTA of another kernel that is meant to run next to
 // this one (the lattice kernel next to the softmax/gather kernel); 0 = none.
 inline RingLayout make_ring(size_t slot_payload, size_t extra_bytes, size_t smem_reserve = 0, int consumers = kRingConsumers) {
     RingLayout r;
     r.slot_bytes = align_up(slot_payload, 128);
     const size_t fixed = (size_t)kMaxSlots * (sizeof(RowMeta) + 16) + extra_bytes + 256;
-    long long budget = (long long)ring_budget();
+    long long budget = (long long)kRingSmemBudget;
     if (smem_reserve) {
         const long long room = 228 * 1024 - 2 * 1024 - (long long)smem_reserve;       // 1 KB per CTA is the driver's
         if (room < budget) budget = room;
@@ -138,7 +130,7 @@ __device__ __forceinline__ int ring_claim(const Ring &r, unsigned q) {
 
 // Consumer side (whole warp): take the next row, whichever it is.  Rows are NOT dealt out round-robin: a row that has
 // landed would then wait for "its" consumer while others idle -- at 66 % consumer utilisation that wait was as long
-// as the processing itself and kept a third of the ring's slots out of flight (tools/k1_roles.py).
+// as the processing itself and kept a third of the ring's slots out of flight (measured per warp, DESIGN.md §3).
 __device__ __forceinline__ unsigned ring_next_row(const Ring &r, int lane) {
     unsigned q = 0;
     if (lane == 0) q = atomicAdd(r.next, 1u);
@@ -187,20 +179,6 @@ __device__ __forceinline__ void ring_stop(const Ring &r, unsigned q, int lane) {
         }
     }
     __syncwarp();
-}
-
-// Producer side (whole warp): ticket handling.  Lane 0 keeps the *next* batch's ticket in flight in `pend`
-// (the atomic's latency hides behind the batch being issued); ring_take_batch broadcasts the batch that
-// is due now and immediately requests the following one.
-__device__ __forceinline__ void ring_first_ticket(unsigned *ticket, unsigned &pend, int lane, int batch) {
-    pend = 0;
-    if (lane == 0) pend = atomicAdd(ticket, (unsigned)batch);
-}
-__device__ __forceinline__ unsigned ring_take_batch(unsigned *ticket, unsigned &pend, int lane, int batch,
-                                                    unsigned frames) {
-    const unsigned base = __shfl_sync(0xffffffffu, pend, 0);
-    if (base < frames && lane == 0) pend = atomicAdd(ticket, (unsigned)batch);
-    return base;
 }
 
 #endif  // __CUDACC__

@@ -8,26 +8,11 @@
 // No (T,B,V) log-probability tensor is ever materialised.
 //
 // One warp per frame, 128-bit loads, online (max, sum) per lane, warp-shuffle reduction.
-#include <stdlib.h>
 #include "common.cuh"
 #include "kernels.h"
 #include "row_ring.cuh"
 
 namespace b200ctc {
-
-#ifdef B200CTC_EXPERIMENT
-__device__ long long *g_tl_k1 = nullptr;      // timeline hook, see common.cuh
-void softmax_set_timeline(long long *p) { cudaMemcpyToSymbol(g_tl_k1, &p, sizeof(p)); }
-#define B200CTC_TL_K1(end) timeline_mark(g_tl_k1, 0, end)
-// role breakdown (tools/k1_roles.py): per CTA and warp, cycles spent [0] waiting for a ticket / a row, [1] waiting for a
-// free slot (producer) / processing (consumer), [2] rows handled, [3] total cycles
-__device__ long long *g_k1_roles = nullptr;
-void softmax_set_roles(long long *p) { cudaMemcpyToSymbol(g_k1_roles, &p, sizeof(p)); }
-#define K1_CLK() (g_k1_roles ? clock64() : 0ll)
-#else
-#define K1_CLK() 0ll
-#define B200CTC_TL_K1(end) ((void)0)
-#endif
 
 namespace {
 
@@ -44,7 +29,7 @@ constexpr int kUnroll = 4;
 // row is one contiguous 4*V-byte read either way.
 // (Tried and dropped: walking every utterance from ITS two ends, in groups ordered by decreasing length so that the
 // rows produced last belong to the shortest utterances.  The exposed lattice tail shrank from 33 to 27 us, but this
-// kernel lost 8 us to the scattered row order -- no net gain, tools/step_timeline.py.)
+// kernel lost 8 us to the scattered row order -- no net gain, measured on per-kernel timelines.)
 __device__ __forceinline__ void frame_of_ticket(unsigned f, int B, int T, bool two_ended, int &b, int &t) {
     const int slice = (int)(f / (unsigned)B);
     b = (int)(f % (unsigned)B);
@@ -215,7 +200,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) softmax_gather_kernel(Probl
         f = __shfl_sync(0xffffffffu, f, 0);
         if (f >= frames) break;
         int b, t;
-        frame_of_ticket(f, d.B, d.T, (d.progress & 2) != 0, b, t);
+        frame_of_ticket(f, d.B, d.T, d.concurrent != 0, b, t);
         int Tb = d.input_lengths ? d.input_lengths[b] : d.T;
         Tb = max(0, min(Tb, d.T));
         const bool valid = t < Tb;
@@ -229,7 +214,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) softmax_gather_kernel(Probl
         if (!valid) continue;
         float la, lb;
         split_lse2(row_max, lse2, la, lb);
-        if (lane == 0 && pend_b >= 0 && (d.progress & 1)) signal_frame_done(ws, w, pend_b, pend_t);
+        if (lane == 0 && pend_b >= 0 && d.concurrent) signal_frame_done(ws, w, pend_b, pend_t);
         if (lane == 0) lse_out[(size_t)b * d.T + t] = la + lb;
         // gather: column 0 = blank, 1..Lmax = labels, Lmax+1.. = bigrams (gram_ctc.py:24-32, :155)
         int Lb = d.label_lengths ? d.label_lengths[b] : d.Lmax;
@@ -250,7 +235,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) softmax_gather_kernel(Probl
         __syncwarp();
         pend_b = b; pend_t = t;
     }
-    if (lane == 0 && pend_b >= 0 && (d.progress & 1)) signal_frame_done(ws, w, pend_b, pend_t);
+    if (lane == 0 && pend_b >= 0 && d.concurrent) signal_frame_done(ws, w, pend_b, pend_t);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -263,10 +248,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) softmax_gather_kernel(Probl
 // consumer warp that was 28 us of a 105 us kernel.  So the consumers only note finished rows in a small
 // shared-memory FIFO (CTA-scope ordering, cheap) and one extra warp drains all FIFOs with ONE GPU-scope fence per
 // sweep, then bumps the progress counters (the __syncthreads / thread 0 fences / atomic pattern of a grid barrier).
-#ifndef B200CTC_K1_CONSUMERS
-#define B200CTC_K1_CONSUMERS 10
-#endif
-constexpr int kK1Consumers = B200CTC_K1_CONSUMERS;
+constexpr int kK1Consumers = 10;
 constexpr int kK1Threads = 32 * (1 + kK1Consumers + 1);   // producer + consumers + signal warp
 constexpr int kGatherRegs = 4;                         // emitted ids per lane on the early-release path (<= 128 columns)
 constexpr int kFifoDepth = 4;
@@ -360,18 +342,16 @@ __device__ __forceinline__ void fast_row_finish(float ref, float sl, float &la, 
 template <bool ARGMAX>
 __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(ProblemDesc d, WsLayout w,
                                                                               unsigned char *ws,
-                                                                              int64_t *argmax_out, RingLayout rl, int l2_hints) {
+                                                                              int64_t *argmax_out, RingLayout rl) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Ring ring = ring_setup(smem_raw, rl);
     const uint64_t l2pol = l2_policy_evict_first();
-    const bool l2hint = (l2_hints & 2) != 0;
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     WsHeader *hdr = reinterpret_cast<WsHeader *>(ws + w.off_hdr);
     const unsigned frames = (unsigned)d.B * (unsigned)d.T;
-    B200CTC_TL_K1(false);
     SignalFifo *fifo = reinterpret_cast<SignalFifo *>(smem_raw + rl.off_extra);
-    const bool signalling = (d.progress & 1) != 0;
+    const bool signalling = d.concurrent != 0;
     if (threadIdx.x < kK1Consumers) { fifo->head[threadIdx.x] = 0u; fifo->tail[threadIdx.x] = 0u; }
     // clamped lengths of every utterance, once per CTA: the producer then turns a ticket into copies without a round
     // trip to L2 in between (that round trip, per batch of 8 rows, was 15 % of its time)
@@ -394,9 +374,6 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
     if (warp == 0) {
         // ===== producer (lane i owns frame i of the current batch) =====
         unsigned q = 0;
-        long long r_wait0 = 0, r_wait1 = 0, r_rows = 0;
-        const long long r_begin = K1_CLK();
-        (void)r_begin;
         // one batch of tickets -> rows into the ring; returns false when the queue is exhausted
         auto issue_batch = [&](unsigned base) -> bool {
             if (base >= frames) return false;
@@ -404,7 +381,7 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
             int b = 0, t = 0, Lb = 0;
             bool valid = false, need = false;
             if (lane < ring.batch && f < frames) {
-                frame_of_ticket(f, d.B, d.T, (d.progress & 2) != 0, b, t);
+                frame_of_ticket(f, d.B, d.T, d.concurrent != 0, b, t);
                 int Tb;
                 if (len_cached) { Tb = len_sm[b]; Lb = len_sm[d.B + b]; }
                 else {
@@ -420,8 +397,6 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
             const unsigned myq = q + (unsigned)__popc(mask & ((1u << lane) - 1u));
             // every lane issues its row as soon as ITS slot is free, in whatever order the consumers hand slots back
             bool pending = need;
-            const long long c1 = K1_CLK();
-            r_rows += __popc(mask);
             while (__any_sync(0xffffffffu, pending)) {
                 bool issued = false;
                 if (pending && ring_slot_free(ring, myq)) {
@@ -434,14 +409,13 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
                     ring.meta[s].Lb = Lb;
                     ring_publish(ring, s, myq);
                     mbar_arrive_expect_tx(&ring.full[s], span);
-                    if (l2hint) bulk_g2s_hint(ring.slot(s), src - off, span, &ring.full[s], l2pol);
-                    else bulk_g2s(ring.slot(s), src - off, span, &ring.full[s]);
+                    // evict-first in L2 (common.cuh): measured 4 us off the forward pass
+                    bulk_g2s_hint(ring.slot(s), src - off, span, &ring.full[s], l2pol);
                     pending = false;
                     issued = true;
                 }
                 if (!__any_sync(0xffffffffu, issued)) __nanosleep(40);
             }
-            r_wait1 += K1_CLK() - c1;
             q += (unsigned)__popc(mask);
             return true;
         };
@@ -452,25 +426,14 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
         unsigned pa = 0, pb = 0;
         if (lane == 0) { pa = atomicAdd(&hdr->k1_ticket, (unsigned)ring.batch); pb = atomicAdd(&hdr->k1_ticket, (unsigned)ring.batch); }
         for (;;) {
-            long long c0 = K1_CLK();
             unsigned base = __shfl_sync(0xffffffffu, pa, 0);
             if (lane == 0 && base < frames) pa = atomicAdd(&hdr->k1_ticket, (unsigned)ring.batch);
-            r_wait0 += K1_CLK() - c0;
             if (!issue_batch(base)) break;
-            c0 = K1_CLK();
             base = __shfl_sync(0xffffffffu, pb, 0);
             if (lane == 0 && base < frames) pb = atomicAdd(&hdr->k1_ticket, (unsigned)ring.batch);
-            r_wait0 += K1_CLK() - c0;
             if (!issue_batch(base)) break;
         }
         ring_stop(ring, q, lane);
-        B200CTC_TL_K1(true);
-#ifdef B200CTC_EXPERIMENT
-        if (g_k1_roles && lane == 0) {
-            long long *o = g_k1_roles + ((size_t)blockIdx.x * 16 + 0) * 4;
-            o[0] = r_wait0; o[1] = r_wait1; o[2] = r_rows; o[3] = clock64() - r_begin;
-        }
-#endif
         return;
     }
 
@@ -479,30 +442,15 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
     float2 *lp_out = reinterpret_cast<float2 *>(ws + w.off_lp);
     if (warp - 1 >= ring.nc) return;                      // short ring: fewer active consumers (row_ring.cuh)
     unsigned pushed = 0;
-    long long c_wait = 0, c_proc = 0, c_rows = 0;
-    const long long c_begin = K1_CLK();
-    (void)c_begin;
     for (;;) {
         const unsigned q = ring_next_row(ring, lane);
-        const long long c0 = K1_CLK();
         const int s = ring_acquire(ring, q);
-        const long long c1 = K1_CLK();
-        c_wait += c1 - c0;
         const RowMeta m = ring.meta[s];
         if (m.kind < 0) {                       // stop record: hand the slot back (the ring may be shorter than
             __syncwarp();                       // the number of consumers) and leave
             if (lane == 0) mbar_arrive(&ring.empty[s]);
             break;
         }
-#ifdef B200CTC_EXPERIMENT
-        if (d.progress & 64) {                  // streaming-rate experiment: rows are dropped as they land (results are garbage)
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&ring.empty[s]);
-            c_proc += K1_CLK() - c1;
-            ++c_rows;
-            continue;
-        }
-#endif
         float *slotf = reinterpret_cast<float *>(ring.slot(s));
         const float *row = slotf + m.off;                              // element v of the frame
         const float4 *row4 = reinterpret_cast<const float4 *>(slotf);  // the aligned span, float4 by float4
@@ -618,16 +566,8 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
         }
         __syncwarp();
         if (lane == 0 && !released) mbar_arrive(&ring.empty[s]);
-        c_proc += K1_CLK() - c1;
-        ++c_rows;
     }
     if (signalling && lane == 0) fifo_push(fifo, warp - 1, pushed, -1, 0);
-#ifdef B200CTC_EXPERIMENT
-    if (g_k1_roles && lane == 0) {
-        long long *o = g_k1_roles + ((size_t)blockIdx.x * 16 + warp) * 4;
-        o[0] = c_wait; o[1] = c_proc; o[2] = c_rows; o[3] = clock64() - c_begin;
-    }
-#endif
 }
 
 __global__ void __launch_bounds__(kWarpsPerCta * 32) argmax_kernel(const float *acts, int64_t stride_t,
@@ -663,7 +603,6 @@ int grid_for_frames(long long frames) {
 // row that is only 4-byte aligned) fit in shared memory; base pointer and strides are in floats, so any of them do.
 bool ring_usable(const void *base, int64_t stride_t, int64_t stride_b, int V, const RingLayout &rl) {
     (void)stride_t; (void)stride_b; (void)V;
-    if (knobs().no_tma) return false;
     return (reinterpret_cast<uintptr_t>(base) & 3) == 0 && rl.slots >= kMinSlots;
 }
 
@@ -673,7 +612,7 @@ cudaError_t launch_softmax_gather(const ProblemDesc &d, const WsLayout &w, void 
     if (frames == 0) return cudaSuccess;
     unsigned char *wsb = static_cast<unsigned char *>(ws);
     const RingLayout rl = make_ring(ring_row_bytes(d.V), kFifoBytes + (d.B <= kLenCache ? 8 * (size_t)d.B : 0), smem_reserve, kK1Consumers);
-    if (ring_usable(d.acts, d.stride_t, d.stride_b, d.V, rl) && !knobs().no_tma_k1) {
+    if (ring_usable(d.acts, d.stride_t, d.stride_b, d.V, rl)) {
         long long ctas = (frames + kTicketBatch - 1) / kTicketBatch;
         if (ctas > sm_count()) ctas = sm_count();
         if (ctas < 1) ctas = 1;
@@ -681,11 +620,11 @@ cudaError_t launch_softmax_gather(const ProblemDesc &d, const WsLayout &w, void 
         if (argmax_out) {
             e = ensure_dynamic_smem(reinterpret_cast<const void *>(softmax_gather_ring_kernel<true>), rl.total);
             if (e != cudaSuccess) return e;
-            softmax_gather_ring_kernel<true><<<(int)ctas, kK1Threads, rl.total, stream>>>(d, w, wsb, argmax_out, rl, knobs().l2_hints);
+            softmax_gather_ring_kernel<true><<<(int)ctas, kK1Threads, rl.total, stream>>>(d, w, wsb, argmax_out, rl);
         } else {
             e = ensure_dynamic_smem(reinterpret_cast<const void *>(softmax_gather_ring_kernel<false>), rl.total);
             if (e != cudaSuccess) return e;
-            softmax_gather_ring_kernel<false><<<(int)ctas, kK1Threads, rl.total, stream>>>(d, w, wsb, nullptr, rl, knobs().l2_hints);
+            softmax_gather_ring_kernel<false><<<(int)ctas, kK1Threads, rl.total, stream>>>(d, w, wsb, nullptr, rl);
         }
         return cudaGetLastError();
     }
