@@ -50,6 +50,9 @@ def _bind(lib):
     lib.b200ctc_greedy_argmax.restype = c.c_int
     lib.b200ctc_greedy_argmax.argtypes = [c.c_void_p, c.c_int64, c.c_int64, c.c_int, c.c_int, c.c_int,
                                           c.c_void_p, c.c_void_p]
+    lib.b200ctc_ln_greedy_argmax.restype = c.c_int
+    lib.b200ctc_ln_greedy_argmax.argtypes = [c.c_void_p, c.c_int64, c.c_int64, c.c_void_p, c.c_void_p, c.c_int, c.c_int,
+                                             c.c_int, c.c_void_p, c.c_void_p]
     lib.b200ctc_greedy_error.restype = c.c_int
     lib.b200ctc_greedy_error.argtypes = [c.c_void_p, c.c_void_p, c.c_int, c.c_int, c.c_void_p, c.c_int, c.c_int,
                                          c.c_void_p, c.c_int, c.c_int, c.c_int, c.c_void_p, c.c_void_p, c.c_void_p,

@@ -4,5 +4,5 @@ from .gram_ctc import gram_ctc, joint_gram_ctc, GramCTC                         
 from .ctc import connectionist_temporal_classification, ctc, ConnectionistTemporalClassification   # noqa: F401
 from ._function import greedy_argmax                                         # noqa: F401
 from .host import ctc_host, gram_ctc_host                                   # noqa: F401
-from .layernorm_loss import layernorm_ctc, layernorm_gram_ctc                         # noqa: F401
+from .layernorm_loss import layernorm_ctc, layernorm_gram_ctc, layernorm_greedy_argmax   # noqa: F401
 from .graphed import GraphedStep                                             # noqa: F401

@@ -15,6 +15,9 @@ normalised tensor, its transpose and their gradients are never materialised (csr
 
     loss = layernorm_gram_ctc(z, ln.gamma, ln.beta, t_batch, bigram_batch, ID_BLANK, x_length_batch, t_length_batch,
                               joint_ctc=args.joint_training)     # Gram-CTC, optionally + CTC (joint training)
+
+    y = layernorm_greedy_argmax(z, ln.gamma, ln.beta)              # the development loop's greedy ids, (B, T)
+    # instead of:  y = xp.argmax(model(x, split_into_variables=False).data, axis=2)
 """
 import numpy as np
 import torch
@@ -75,12 +78,8 @@ class LayerNormLossFunction(torch.autograd.Function):
         return (dz, dgamma if ctx.needs_input_grad[1] else None, dbeta if ctx.needs_input_grad[2] else None) + (None,) * 9
 
 
-def _layernorm_loss(kind, z, gamma, beta, labels, bigrams, blank_symbol, input_length, label_length, reduce,
-                    batch_global=None, group=None):
-    if reduce not in ("mean", "no"):                             # gram_ctc.py:224-227
-        raise ValueError("only 'mean' and 'no' are valid for 'reduce', but '%s' is given" % reduce)
-    if isinstance(blank_symbol, bool) or not isinstance(blank_symbol, (int, np.integer)):   # :303-304
-        raise TypeError("blank_symbol must be non-negative integer.")
+def _layernorm_inputs(z, gamma, beta):
+    """z (B, V, 1, T) or (B, V, T) -> a (B, V, T) view with time stride 1; gamma, beta -> float32 (V,) on z's device."""
     z, gamma, beta = as_device_tensor(z), as_device_tensor(gamma), as_device_tensor(beta)
     if not isinstance(z, torch.Tensor) or z.dim() not in (3, 4):
         raise TypeError("z must be the (B, V, 1, T) output of the model's last convolution")
@@ -96,7 +95,7 @@ def _layernorm_loss(kind, z, gamma, beta, labels, bigrams, blank_symbol, input_l
         z3 = z
     if z3.stride(2) != 1 and z3.shape[2] > 1:
         z3 = z3.contiguous()
-    B, V, T = z3.shape
+    V = z3.shape[1]
     dev = z3.device
     gamma = gamma.to(device=dev, dtype=torch.float32).reshape(-1).contiguous() if not (
         gamma.device == dev and gamma.dtype == torch.float32 and gamma.dim() == 1 and gamma.is_contiguous()) else gamma
@@ -104,6 +103,18 @@ def _layernorm_loss(kind, z, gamma, beta, labels, bigrams, blank_symbol, input_l
         beta.device == dev and beta.dtype == torch.float32 and beta.dim() == 1 and beta.is_contiguous()) else beta
     if gamma.numel() != V or beta.numel() != V:
         raise ValueError("gamma and beta must have one entry per vocabulary id (V = %d)" % V)
+    return z3, gamma, beta
+
+
+def _layernorm_loss(kind, z, gamma, beta, labels, bigrams, blank_symbol, input_length, label_length, reduce,
+                    batch_global=None, group=None):
+    if reduce not in ("mean", "no"):                             # gram_ctc.py:224-227
+        raise ValueError("only 'mean' and 'no' are valid for 'reduce', but '%s' is given" % reduce)
+    if isinstance(blank_symbol, bool) or not isinstance(blank_symbol, (int, np.integer)):   # :303-304
+        raise TypeError("blank_symbol must be non-negative integer.")
+    z3, gamma, beta = _layernorm_inputs(z, gamma, beta)
+    B, V, T = z3.shape
+    dev = z3.device
     blank_symbol = int(blank_symbol)
     assert 0 <= blank_symbol < V                                 # :305-306
     labels = _as_int32(labels, dev, "labels")
@@ -149,3 +160,21 @@ def layernorm_gram_ctc(z, gamma, beta, label_unigram, label_bigram, blank_symbol
     kind = _lib.KIND_JOINT if joint_ctc else _lib.KIND_GRAM
     return _layernorm_loss(kind, z, gamma, beta, label_unigram, label_bigram, blank_symbol, input_length,
                            length_unigram, reduce, **kw)
+
+
+def layernorm_greedy_argmax(z, gamma, beta):
+    """The development loop's ``xp.argmax(model(x, split_into_variables=False).data, axis=2)`` (run/ctc/cnn/train.py:232)
+    for a model built without its final LayerNormalization: the (B, T) int64 greedy ids of
+    ``gamma * normalize_layer(z) + beta`` for every frame, from one read of z.  Takes z, gamma and beta as
+    ``layernorm_ctc`` does and raises what it raises; the result goes straight into ``compute_minibatch_error``.
+    numpy.argmax rules: the first of equal maxima wins, NaN counts as maximal.  Builds no autograd edge."""
+    z3, gamma, beta = _layernorm_inputs(z, gamma, beta)
+    z3, gamma, beta = z3.detach(), gamma.detach(), beta.detach()
+    B, V, T = z3.shape
+    dev = z3.device
+    out = torch.empty((B, T), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.load().b200ctc_ln_greedy_argmax(
+            z3.data_ptr(), z3.stride(0), z3.stride(1), gamma.data_ptr(), beta.data_ptr(), B, T, V, out.data_ptr(),
+            _stream_ptr(dev)))
+    return out

@@ -305,6 +305,25 @@ int b200ctc_greedy_argmax(const float *acts, int64_t stride_t, int64_t stride_b,
                       "argmax kernel");
 }
 
+int b200ctc_ln_greedy_argmax(const float *z, int64_t zstride_b, int64_t zstride_v, const float *gamma, const float *beta,
+                             int B, int T, int V, int64_t *argmax_out, void *stream_) {
+    if (B < 0 || T < 0 || V <= 0) return fail(B200CTC_INVALID_ARGUMENT, "bad dimensions%s");
+    if ((size_t)B * T == 0) return B200CTC_OK;
+    if (!z || !gamma || !beta || !argmax_out) return fail(B200CTC_INVALID_ARGUMENT, "NULL pointer%s");
+    if ((long long)B * (long long)T >= (1ll << 31))
+        return fail(B200CTC_UNSUPPORTED, "B*T = %s%lld frames exceeds 2^31", "", (long long)B * T);
+    if (V > 4080 || (zstride_v & 3) != 0 || (zstride_b & 3) != 0 || (reinterpret_cast<uintptr_t>(z) & 15) != 0)
+        return fail(B200CTC_UNSUPPORTED, "fused LayerNormalization needs V <= 4080 and 16-byte aligned rows of z "
+                                         "(pitch %% 4 == 0)%s");
+    const cudaError_t e = launch_ln_argmax(z, zstride_b, zstride_v, gamma, beta, B, T, V, argmax_out,
+                                           static_cast<cudaStream_t>(stream_));
+    if (e == cudaErrorNotSupported) {
+        (void)cudaGetLastError();
+        return fail(B200CTC_UNSUPPORTED, "the driver cannot describe z as a TMA tensor (cuTensorMapEncodeTiled)%s");
+    }
+    return check_cuda(e, "layernorm argmax kernel");
+}
+
 int b200ctc_greedy_error(const int64_t *argmax, const int32_t *input_lengths, int B, int T, const int32_t *labels,
                          int Lmax, int blank, const int32_t *expansion, int V, int E, int uint8_wrap, int32_t *hyp_out,
                          int32_t *hyp_len, int32_t *ref_len, int32_t *distance, double *err_per_utt, double *err_mean,

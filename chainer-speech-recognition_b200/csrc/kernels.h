@@ -83,6 +83,10 @@ cudaError_t launch_ln_forward(const ProblemDesc &d, const LnLayout &ll, void *ws
 cudaError_t launch_ln_backward(const GradParams &g, const LnLayout &ll, const void *ws, const float *z, int64_t zs_b,
                                int64_t zs_v, const float *gamma, const float *beta, float *dz, int64_t dzs_b, int64_t dzs_v,
                                float *dgamma, float *dbeta, cudaStream_t stream);
+// greedy argmax of the normalised z (all T frames), one read of z and no workspace; the caller has checked V <= 4080 and
+// 16-byte aligned rows.  cudaErrorNotSupported: the driver could not describe z as a TMA tensor
+cudaError_t launch_ln_argmax(const float *z, int64_t zs_b, int64_t zs_v, const float *gamma, const float *beta, int B, int T, int V,
+                             int64_t *argmax_out, cudaStream_t stream);
 
 // evaluation path: greedy collapse + gram expansion + edit distance + error rate (greedy_error.cu)
 cudaError_t launch_greedy_error(const int64_t *argmax, const int32_t *input_lengths, int B, int T, const int32_t *labels,

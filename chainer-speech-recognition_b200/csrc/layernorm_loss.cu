@@ -24,6 +24,9 @@
 //            accumulate per thread over all tiles (a thread's rows never change); sweep 2 re-reads z from the ring
 //            (it is still there) and stores dz = rstd * (dn - mean_v(dn) - n * mean_v(dn*n)).
 // 12 bytes per element again -- for the loss AND the normalisation AND both transposes.
+//   argmax   (ln_argmax_kernel): the development loop's greedy ids (run/ctc/cnn/train.py:224-234) from one read of z.
+//            Round 1 as in forward, then the best (value, row) of every frame, merged numpy.argmax-style; every frame
+//            of the padded batch is decoded (asr/error.py:40).  No workspace, one launch.
 //
 // Joint Gram-CTC + CTC objective (run/gram_ctc/cnn/train.py:196-198): the forward pass is Gram-CTC's plus the second,
 // plain-CTC lattice on the same emission rows (api.cu); the backward kernel adds the plain-CTC posteriors to the Gram-CTC
@@ -32,7 +35,8 @@
 // Limits of this version: V <= 4080 (a tile must stay resident in shared memory in the backward kernel: 17 boxes),
 // rows of z 16-byte aligned (T_pitch % 4 == 0 -- a TMA requirement), at most 480 emission columns, and a backward ring
 // of at least K + 2 boxes next to the lattice's per-tile tables (plan_ln_backward: long labels at a large V do not fit).
-// Outside them the entry points return B200CTC_UNSUPPORTED and the caller uses the unfused path.
+// Outside them the entry points return B200CTC_UNSUPPORTED and the caller uses the unfused path.  The argmax has only
+// the first two limits.
 #include <cuda.h>
 #include <stdio.h>
 #include <mutex>
@@ -270,14 +274,19 @@ struct LnParams {
 };
 
 // ---- producer lane: tickets -> tile records -> TMA box loads, as far ahead as the ring allows ----
-// BACKWARD: tile i of the kernel goes to CTA i % gridDim.x (a fixed assignment makes the dgamma/dbeta sums
-// deterministic); forward: tiles are drawn from the global ticket counter (variable-length utterances balance
+// kLnBackward: tile i of the kernel goes to CTA i % gridDim.x (a fixed assignment makes the dgamma/dbeta sums
+// deterministic); kLnForward: tiles are drawn from the global ticket counter (variable-length utterances balance
 // themselves, and the order serves the lattice kernel running next to it).
 // Tiles whose frames are all padding never reach the compute warps: the forward pass skips them, the backward pass
 // stores their zeros (gram_ctc.py:296; LayerNormalization's backward of zero is zero) straight from a box of zeros.
-template <bool BACKWARD>
+// kLnArgmax: every frame is decoded (all T of them, asr/error.py:40), so every tile is work of the same size: the fixed
+// assignment of the backward pass, with no counter to reset and nothing but z to load.
+enum LnPass { kLnForward, kLnBackward, kLnArgmax };
+template <int PASS>
 __device__ __forceinline__ void ln_producer(const CUtensorMap *tmap, const CUtensorMap *tmap_out, const LnParams &p,
                                             unsigned char *smem, const LnSmem &sm) {
+    constexpr bool BACKWARD = PASS == kLnBackward;
+    constexpr bool FIXED = PASS != kLnForward;
     uint64_t *full = reinterpret_cast<uint64_t *>(smem + sm.off_full);
     uint64_t *empty = reinterpret_cast<uint64_t *>(smem + sm.off_empty);
     uint64_t *abbar = reinterpret_cast<uint64_t *>(smem + sm.off_abbar);          // [0] full, [1] empty
@@ -293,11 +302,11 @@ __device__ __forceinline__ void ln_producer(const CUtensorMap *tmap, const CUten
         if (bx >= R) mbar_poll(&empty[bx % R], ((bx / R) - 1u) & 1u);
         return (int)(bx % R);
     };
-    unsigned f = BACKWARD ? blockIdx.x : atomicAdd(&hdr->k1_ticket, 1u);
+    unsigned f = FIXED ? blockIdx.x : atomicAdd(&hdr->k1_ticket, 1u);
     while (f < tiles) {
-        const unsigned fnext = BACKWARD ? f + gridDim.x : atomicAdd(&hdr->k1_ticket, 1u);     // in flight while we issue
+        const unsigned fnext = FIXED ? f + gridDim.x : atomicAdd(&hdr->k1_ticket, 1u);     // in flight while we issue
         int b, tb;
-        const bool real = ln_tile_of_ticket(f, p.d.B, p.nTB, !BACKWARD && p.d.concurrent != 0, b, tb);
+        const bool real = ln_tile_of_ticket(f, p.d.B, p.nTB, !FIXED && p.d.concurrent != 0, b, tb);
         f = fnext;
         if (!real) continue;
         const int t0 = tb * kLnTT;
@@ -308,6 +317,8 @@ __device__ __forceinline__ void ln_producer(const CUtensorMap *tmap, const CUten
             const UttInfo ui = utt[b];
             mm.Tb = ui.Tb; mm.Lb = ui.Lb; mm.Nb = ui.Nb; mm.Ub = ui.Ub; mm.ublank = ui.ublank; mm.Ph = ui.Ph; mm.Pl = ui.Pl;
             mm.sc = (p.per_utterance ? __ldg(p.grad_loss + b) : __ldg(p.grad_loss)) * p.scale;      // gram_ctc.py:291-294
+        } else if (PASS == kLnArgmax) {
+            mm.Tb = p.d.T; mm.Lb = 0;
         } else {
             int Tb = p.d.input_lengths ? __ldg(p.d.input_lengths + b) : p.d.T;
             int Lb = p.d.label_lengths ? __ldg(p.d.label_lengths + b) : p.d.Lmax;
@@ -431,6 +442,49 @@ __device__ __forceinline__ void mbar_spin(uint64_t *bar, uint32_t parity) {
     while (!mbar_try_wait(bar, parity)) { }                              // try_wait suspends the thread in hardware while it waits
 }
 
+// ---- round 1 of the tile kernels: mean and centred second moment of every frame (asr/nn/layernorm.py:41-44) ----
+// z: this thread's rows 240k + 16w + lane/2 of frames 4h .. 4h+3, zeros where a row does not exist (fn of them do; fmissing
+// = KMAX - fn).  Per thread, then over the 16 lanes of a half, then over the warps through `red`: after one meeting of
+// the compute warps, lane 0 of warp f < 8 hands frame f's (count, mean, centred second moment) over all V rows to
+// `finish`.  Returns the frame this lane's half-warp result belongs to (4h + the returned value).
+template <int KMAX, typename F>
+__device__ __forceinline__ int ln_frame_moments(const float4 (&z)[KMAX], float fn, float inv_n, float fmissing, int lane, int h,
+                                                int w, float *red, F finish) {
+    Moments mo[4];
+    {
+        float sx = 0.f, sy = 0.f, sz = 0.f, sw = 0.f;
+#pragma unroll
+        for (int k = 0; k < KMAX; ++k) { sx += z[k].x; sy += z[k].y; sz += z[k].z; sw += z[k].w; }      // missing rows are zeros
+        const float mx_ = sx * inv_n, my_ = sy * inv_n, mz_ = sz * inv_n, mw_ = sw * inv_n;
+        float qx = 0.f, qy = 0.f, qz = 0.f, qw = 0.f;
+#pragma unroll
+        for (int k = 0; k < KMAX; ++k) {
+            const float dx = z[k].x - mx_, dy = z[k].y - my_, dz = z[k].z - mz_, dw = z[k].w - mw_;
+            qx = fmaf(dx, dx, qx); qy = fmaf(dy, dy, qy); qz = fmaf(dz, dz, qz); qw = fmaf(dw, dw, qw);
+        }
+        // a missing row read as 0 and contributed mean^2: take that back
+        mo[0].mean = mx_; mo[0].m2 = fmaf(-fmissing * mx_, mx_, qx);
+        mo[1].mean = my_; mo[1].m2 = fmaf(-fmissing * my_, my_, qy);
+        mo[2].mean = mz_; mo[2].m2 = fmaf(-fmissing * mz_, mz_, qz);
+        mo[3].mean = mw_; mo[3].m2 = fmaf(-fmissing * mw_, mw_, qw);
+        mo[0].n = mo[1].n = mo[2].n = mo[3].n = fn;
+    }
+    int fih;
+    const Moments mr = reduce_frames16(mo[0], mo[1], mo[2], mo[3], lane, merge_moments, fih);
+    if (lane < 8) { const float v3[3] = {mr.n, mr.mean, mr.m2}; red_store<3>(red, 4 * h + fih, w, v3); }
+    bar_compute();
+    if (w < kLnTT) {
+        Moments a;
+        const float *src = red + (w * 16 + (lane & 15)) * 4;
+        a.n = src[0]; a.mean = src[1]; a.m2 = src[2];
+        if ((lane & 15) >= kLnWarps) { a.n = 0.f; a.mean = 0.f; a.m2 = 0.f; }
+#pragma unroll
+        for (int o = 1; o < 16; o <<= 1) a = merge_moments(a, Moments::shfl_xor(a, o));
+        if (lane == 0) finish(a);
+    }
+    return fih;
+}
+
 
 // ---------------------------------------------------------------------------------------------
 // forward
@@ -470,7 +524,7 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
     const int lane = threadIdx.x & 31;
     LnSignalFifo *fifo = reinterpret_cast<LnSignalFifo *>(smem + sm.off_fifo);
     if (w == kLnWarps) {
-        if (lane == 0) ln_producer<false>(&tmap, nullptr, p, smem, sm);
+        if (lane == 0) ln_producer<kLnForward>(&tmap, nullptr, p, smem, sm);
         else if (lane == 1 && d.concurrent) ln_signaller(p, smem, sm);
         return;
     }
@@ -531,45 +585,14 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
         }
 
         // ---- round 1: mean and centred second moment of every frame (asr/nn/layernorm.py:41-44) ----
-        Moments mo[4];
-        {
-            float sx = 0.f, sy = 0.f, sz = 0.f, sw = 0.f;
-#pragma unroll
-            for (int k = 0; k < KMAX; ++k) { sx += z[k].x; sy += z[k].y; sz += z[k].z; sw += z[k].w; }      // missing rows are zeros
-            const float mx_ = sx * inv_n, my_ = sy * inv_n, mz_ = sz * inv_n, mw_ = sw * inv_n;
-            float qx = 0.f, qy = 0.f, qz = 0.f, qw = 0.f;
-#pragma unroll
-            for (int k = 0; k < KMAX; ++k) {
-                const float dx = z[k].x - mx_, dy = z[k].y - my_, dz = z[k].z - mz_, dw = z[k].w - mw_;
-                qx = fmaf(dx, dx, qx); qy = fmaf(dy, dy, qy); qz = fmaf(dz, dz, qz); qw = fmaf(dw, dw, qw);
-            }
-            // a missing row read as 0 and contributed mean^2: take that back
-            mo[0].mean = mx_; mo[0].m2 = fmaf(-fmissing * mx_, mx_, qx);
-            mo[1].mean = my_; mo[1].m2 = fmaf(-fmissing * my_, my_, qy);
-            mo[2].mean = mz_; mo[2].m2 = fmaf(-fmissing * mz_, mz_, qz);
-            mo[3].mean = mw_; mo[3].m2 = fmaf(-fmissing * mw_, mw_, qw);
-            mo[0].n = mo[1].n = mo[2].n = mo[3].n = fn;
-        }
-        int fih;
-        const Moments mr = reduce_frames16(mo[0], mo[1], mo[2], mo[3], lane, merge_moments, fih);
-        if (lane < 8) { const float v3[3] = {mr.n, mr.mean, mr.m2}; red_store<3>(red, 4 * h + fih, w, v3); }
-        bar_compute();
-        if (w < kLnTT) {
-            Moments a;
-            const float *src = red + (w * 16 + (lane & 15)) * 4;
-            a.n = src[0]; a.mean = src[1]; a.m2 = src[2];
-            if ((lane & 15) >= kLnWarps) { a.n = 0.f; a.mean = 0.f; a.m2 = 0.f; }
-#pragma unroll
-            for (int o = 1; o < 16; o <<= 1) a = merge_moments(a, Moments::shfl_xor(a, o));
-            if (lane == 0) {
-                const float var = fmaxf(a.m2, 0.f) / a.n;                      // sum(diff^2) / size, no epsilon (:44)
-                const float rstd = 1.f / sqrtf(var);
-                tot[w * 8 + 0] = a.mean;
-                tot[w * 8 + 1] = rstd;
-                const int t = m.t0 + w;
-                if (t < Tb) { mu_out[(size_t)m.b * p.Tq + t] = a.mean; rstd_out[(size_t)m.b * p.Tq + t] = rstd; }
-            }
-        }
+        int fih = ln_frame_moments<KMAX>(z, fn, inv_n, fmissing, lane, h, w, red, [&](const Moments &a) {
+            const float var = fmaxf(a.m2, 0.f) / a.n;                      // sum(diff^2) / size, no epsilon (:44)
+            const float rstd = 1.f / sqrtf(var);
+            tot[w * 8 + 0] = a.mean;
+            tot[w * 8 + 1] = rstd;
+            const int t = m.t0 + w;
+            if (t < Tb) { mu_out[(size_t)m.b * p.Tq + t] = a.mean; rstd_out[(size_t)m.b * p.Tq + t] = rstd; }
+        });
         bar_compute();
 
         // ---- round 2: a = gamma * (z - mean) * rstd + beta (asr/nn/nn.py:265), in place; softmax statistics ----
@@ -698,7 +721,7 @@ __global__ void __launch_bounds__(kLnThreads, 1) ln_gradient_kernel(const __grid
     const int w = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
     const int lane = threadIdx.x & 31;
     if (w == kLnWarps) {
-        if (lane == 0) ln_producer<true>(&tmap, &tmap_dz, p, smem, sm);
+        if (lane == 0) ln_producer<kLnBackward>(&tmap, &tmap_dz, p, smem, sm);
         else if (lane == 1) ln_storer(&tmap_dz, p, smem, sm);
         return;
     }
@@ -931,6 +954,156 @@ __global__ void ln_reduce_params_kernel(const float *part, int nparts, int Vp, i
     if (dbeta) dbeta[v] = b;
 }
 
+// ---------------------------------------------------------------------------------------------
+// greedy argmax (the development loop, run/ctc/cnn/train.py:224-234: xp.argmax(y.data, axis=2) on the normalised output)
+// ---------------------------------------------------------------------------------------------
+constexpr int kLnNoRow = 0x7fffffff;      // "no candidate": loses to every real row, whatever its value
+struct ArgMax {                           // best normalised value of a frame so far and its vocabulary row
+    float v;
+    int i;
+    static __device__ __forceinline__ ArgMax shfl_xor(const ArgMax &a, int o) {
+        ArgMax r;
+        r.v = __shfl_xor_sync(0xffffffffu, a.v, o);
+        r.i = __shfl_xor_sync(0xffffffffu, a.i, o);
+        return r;
+    }
+};
+// numpy.argmax order: a NaN above everything, then the larger value, then (equal values, or two NaNs) the smaller row.
+// The merges run in an order that depends on which lane owns which rows, so ties are broken by the row, never by order.
+__device__ __forceinline__ ArgMax merge_argmax(const ArgMax &a, const ArgMax &b) {
+    const bool an = a.v != a.v, bn = b.v != b.v;
+    const bool take_b = an != bn ? bn : (b.v > a.v || (!(b.v < a.v) && b.i < a.i));
+    return take_b ? b : a;
+}
+
+// One read of z, no workspace: round 1 as in the forward kernel, then every thread keeps the best (value, row) of its four
+// frames over its rows and the CTA merges them like the softmax statistics.  Rows v >= V are excluded by index: the
+// value of a row is no protection in a frame whose values are all NaN.  A frame with a NaN or an infinity anywhere gives
+// 0 (the reference's every normalised value is NaN then), and so does a frame of zeros (0/0).
+template <int KMAX>
+__global__ void __launch_bounds__(kLnThreads, 1) ln_argmax_kernel(const __grid_constant__ CUtensorMap tmap, LnParams p, LnSmem sm,
+                                                                  int64_t *out) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    uint64_t *full = reinterpret_cast<uint64_t *>(smem + sm.off_full);
+    uint64_t *empty = reinterpret_cast<uint64_t *>(smem + sm.off_empty);
+    LnTileMeta *metas = reinterpret_cast<LnTileMeta *>(smem + sm.off_meta);
+    float *red = reinterpret_cast<float *>(smem + sm.off_red);
+    float *tot = reinterpret_cast<float *>(smem + sm.off_tot);
+    float *gb = reinterpret_cast<float *>(smem + sm.off_gb);
+    const uint32_t ring = smem_u32(smem + sm.off_ring);
+    const ProblemDesc &d = p.d;
+    const unsigned R = (unsigned)p.R;
+    const int K = p.K;
+    constexpr int Vt = KMAX * kLnBoxRows;
+    if (threadIdx.x == 0) {
+        for (unsigned i = 0; i < R; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], kLnWarps); }
+        mbar_init_fence();
+    }
+    for (int i = threadIdx.x; i < Vt; i += blockDim.x) {
+        gb[i] = i < d.V ? __ldg(p.gamma + i) : 0.f;
+        gb[Vt + i] = i < d.V ? __ldg(p.beta + i) : 0.f;
+    }
+    __syncthreads();
+    const int w = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
+    const int lane = threadIdx.x & 31;
+    if (w == kLnWarps) {
+        if (lane == 0) ln_producer<kLnArgmax>(&tmap, nullptr, p, smem, sm);
+        return;
+    }
+    const int r = lane >> 1, h = lane & 1;
+    const int vrow = 16 * w + r;
+    int nrows = 0;                                        // this thread's rows that exist: k < nrows
+#pragma unroll
+    for (int k = 0; k < KMAX; ++k) nrows += (k < K && kLnBoxRows * k + vrow < d.V) ? 1 : 0;
+    const float fn = (float)nrows, inv_n = nrows > 0 ? 1.f / (float)nrows : 0.f, fmissing = (float)(KMAX - nrows);
+    const uint32_t lane_off = (uint32_t)(w * 512 + lane * 16);
+
+    SlotIter it = {0u, 0u};
+    unsigned seq = 0;
+    for (;;) {
+        mbar_spin(&full[it.slot], it.phase);
+        const LnTileMeta m = metas[seq % kLnMetaRing];
+        ++seq;
+        if (m.kind < 0) break;
+        float4 z[KMAX];
+        {
+            SlotIter s = it;
+#pragma unroll
+            for (int k = 0; k < KMAX; ++k) {
+                z[k] = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (k < K) {
+                    if (k > 0) mbar_spin(&full[s.slot], s.phase);
+                    z[k] = lds128(ring + s.slot * kLnBoxBytes + lane_off);
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(&empty[s.slot]);
+                    s.next(R);
+                }
+            }
+            it = s;
+        }
+
+        // ---- round 1 ----
+        int fih = ln_frame_moments<KMAX>(z, fn, inv_n, fmissing, lane, h, w, red, [&](const Moments &a) {
+            const float rstd = 1.f / sqrtf(fmaxf(a.m2, 0.f) / a.n);
+            // a NaN or an infinity in the frame leaves a NaN mean or a NaN second moment (inf - inf); make the mean NaN
+            // so that every value of the frame is NaN, as in the reference -- fmaxf above would have hidden a NaN m2
+            tot[w * 8 + 0] = (a.mean != a.mean || a.m2 != a.m2) ? __int_as_float(0x7fc00000) : a.mean;
+            tot[w * 8 + 1] = rstd;
+        });
+        bar_compute();
+
+        // ---- round 2: a = gamma * (z - mean) * rstd + beta (asr/nn/nn.py:265); best (value, row) of each frame ----
+        ArgMax am[4];
+        {
+            float rs[4], mur[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) { rs[j] = tot[(4 * h + j) * 8 + 1]; mur[j] = -tot[(4 * h + j) * 8 + 0] * rs[j]; }
+            float bv[4];
+            int bi[4];
+            {                                             // row k = 0 (it exists unless V <= 16w + lane/2)
+                const float g0 = gb[vrow], b0 = gb[Vt + vrow];
+                const bool has = nrows > 0;
+                bv[0] = has ? fmaf(fmaf(z[0].x, rs[0], mur[0]), g0, b0) : -INFINITY;
+                bv[1] = has ? fmaf(fmaf(z[0].y, rs[1], mur[1]), g0, b0) : -INFINITY;
+                bv[2] = has ? fmaf(fmaf(z[0].z, rs[2], mur[2]), g0, b0) : -INFINITY;
+                bv[3] = has ? fmaf(fmaf(z[0].w, rs[3], mur[3]), g0, b0) : -INFINITY;
+                bi[0] = bi[1] = bi[2] = bi[3] = has ? vrow : kLnNoRow;
+            }
+#pragma unroll
+            for (int k = 1; k < KMAX; ++k) {
+                if (k < nrows) {                          // rows ascend with k: a strict win keeps the first of equal values
+                    const int row = kLnBoxRows * k + vrow;
+                    const float gk = gb[row], bk = gb[Vt + row];
+                    const float v[4] = {fmaf(fmaf(z[k].x, rs[0], mur[0]), gk, bk), fmaf(fmaf(z[k].y, rs[1], mur[1]), gk, bk),
+                                        fmaf(fmaf(z[k].z, rs[2], mur[2]), gk, bk), fmaf(fmaf(z[k].w, rs[3], mur[3]), gk, bk)};
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {
+                        const bool take = v[j] > bv[j] || (v[j] != v[j] && bv[j] == bv[j]);
+                        bv[j] = take ? v[j] : bv[j];
+                        bi[j] = take ? row : bi[j];
+                    }
+                }
+            }
+#pragma unroll
+            for (int j = 0; j < 4; ++j) { am[j].v = bv[j]; am[j].i = bi[j]; }
+        }
+        const ArgMax ar = reduce_frames16(am[0], am[1], am[2], am[3], lane, merge_argmax, fih);
+        if (lane < 8) { const float v2[2] = {ar.v, __int_as_float(ar.i)}; red_store<2>(red, 4 * h + fih, w, v2); }
+        bar_compute();
+        if (w < kLnTT) {
+            ArgMax b;
+            const float *src = red + (w * 16 + (lane & 15)) * 4;
+            b.v = src[0]; b.i = __float_as_int(src[1]);
+            if ((lane & 15) >= kLnWarps) { b.v = -INFINITY; b.i = kLnNoRow; }
+#pragma unroll
+            for (int o = 1; o < 16; o <<= 1) b = merge_argmax(b, ArgMax::shfl_xor(b, o));
+            const int t = m.t0 + w;
+            if (lane == 0 && t < d.T) out[(size_t)m.b * d.T + t] = b.i;
+        }
+        bar_compute();            // protects red against the next tile
+    }
+}
+
 static int ln_kmax(int K) { return K <= 5 ? 5 : (K <= 9 ? 9 : (K <= 15 ? 15 : 17)); }
 
 // The backward kernel's shared-memory plan -- the one place that decides whether a shape's backward pass can run:
@@ -945,6 +1118,20 @@ LnSmem plan_ln_backward(const WsLayout &w) {
     return plan_ln_smem(K, (size_t)2 * kLnTT * w.Np * 8, (size_t)kLnTT * ((w.Umax + 3) & ~3),
                         (size_t)kLnTT * w.Np + (size_t)kLnTT * kLnBlankChunks, (size_t)2 * w.Nmax + 2, (size_t)2 * Vt,
                         (size_t)2 * (Vt / 32 + 1), kLnBoxBytes);
+}
+
+// Shared memory of the kernels that only stream tiles through the ring (forward, argmax): the gamma/beta table, the
+// reductions' scratch and the ring.  smem_reserve: room to leave to a lattice CTA on the same SM, given up when the ring
+// would then hold fewer than K + 2 boxes.
+LnSmem plan_ln_stream(int K, size_t smem_reserve) {
+    const size_t gbf = (size_t)2 * ln_kmax(K) * kLnBoxRows;
+    LnSmem sm = plan_ln_smem(K, 0, 0, 0, 0, gbf, 0, 0, smem_reserve);
+    if (sm.R < K + 2) sm = plan_ln_smem(K, 0, 0, 0, 0, gbf, 0, 0, 0);     // no room to share the SM
+    if (sm.R > 2 * K + 4) {                       // more than two tiles' worth buys nothing; leave the rest to the L1
+        sm.total -= (size_t)(sm.R - (2 * K + 4)) * kLnBoxBytes;
+        sm.R = 2 * K + 4;
+    }
+    return sm;
 }
 
 // ---- host side ----
@@ -984,12 +1171,12 @@ bool make_z_map(CUtensorMap *map, const float *z, int B, int T, int V, int64_t z
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <typename Kern, typename... Maps>
-cudaError_t launch_ln(Kern kern, int grid, const LnParams &p, const LnSmem &sm, cudaStream_t stream, const Maps &...maps) {
+template <typename Kern, typename... Args>
+cudaError_t launch_ln(Kern kern, int grid, const LnSmem &sm, cudaStream_t stream, const Args &...args) {
     (void)cudaGetLastError();
     cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void *>(kern), sm.total);
     if (e != cudaSuccess) { note_failure_site("shared-memory opt-in"); return e; }
-    kern<<<grid, kLnThreads, sm.total, stream>>>(maps..., p, sm);
+    kern<<<grid, kLnThreads, sm.total, stream>>>(args...);
     e = cudaGetLastError();
     if (e != cudaSuccess) note_failure_site("tile kernel launch");
     return e;
@@ -1034,14 +1221,8 @@ cudaError_t launch_ln_forward(const ProblemDesc &d, const LnLayout &ll, void *ws
     p.Tq = (d.T + 3) & ~3;
     p.K = (d.V + kLnBoxRows - 1) / kLnBoxRows;
     p.nTB = (d.T + kLnTT - 1) / kLnTT;
-    const size_t gbf = (size_t)2 * ln_kmax(p.K) * kLnBoxRows;
-    LnSmem sm = plan_ln_smem(p.K, 0, 0, 0, 0, gbf, 0, 0, smem_reserve);
-    if (sm.R < p.K + 2) sm = plan_ln_smem(p.K, 0, 0, 0, 0, gbf, 0, 0, 0);     // no room to share the SM
+    const LnSmem sm = plan_ln_stream(p.K, smem_reserve);
     if (sm.R < p.K + 2) return cudaErrorInvalidConfiguration;
-    if (sm.R > 2 * p.K + 4) {                     // more than two tiles' worth buys nothing; leave the rest to the L1
-        sm.total -= (size_t)(sm.R - (2 * p.K + 4)) * kLnBoxBytes;
-        sm.R = 2 * p.K + 4;
-    }
     p.R = sm.R;
     CUtensorMap map;
     if (!make_z_map(&map, z, d.B, d.T, d.V, zs_b, zs_v)) return cudaErrorInvalidValue;
@@ -1049,10 +1230,10 @@ cudaError_t launch_ln_forward(const ProblemDesc &d, const LnLayout &ll, void *ws
     int grid = (int)(tiles < sm_count() ? tiles : sm_count());
     if (grid < 1) grid = 1;
     switch (ln_kmax(p.K)) {
-        case 5: return launch_ln(ln_softmax_gather_kernel<5>, grid, p, sm, stream, map);
-        case 9: return launch_ln(ln_softmax_gather_kernel<9>, grid, p, sm, stream, map);
-        case 15: return launch_ln(ln_softmax_gather_kernel<15>, grid, p, sm, stream, map);
-        default: return launch_ln(ln_softmax_gather_kernel<17>, grid, p, sm, stream, map);
+        case 5: return launch_ln(ln_softmax_gather_kernel<5>, grid, sm, stream, map, p, sm);
+        case 9: return launch_ln(ln_softmax_gather_kernel<9>, grid, sm, stream, map, p, sm);
+        case 15: return launch_ln(ln_softmax_gather_kernel<15>, grid, sm, stream, map, p, sm);
+        default: return launch_ln(ln_softmax_gather_kernel<17>, grid, sm, stream, map, p, sm);
     }
 }
 
@@ -1084,10 +1265,10 @@ cudaError_t launch_ln_backward(const GradParams &g, const LnLayout &ll, const vo
     if (grid < 1) grid = 1;
     cudaError_t e;
     switch (ln_kmax(p.K)) {
-        case 5: e = launch_ln(ln_gradient_kernel<5>, grid, p, sm, stream, map, map_dz); break;
-        case 9: e = launch_ln(ln_gradient_kernel<9>, grid, p, sm, stream, map, map_dz); break;
-        case 15: e = launch_ln(ln_gradient_kernel<15>, grid, p, sm, stream, map, map_dz); break;
-        default: e = launch_ln(ln_gradient_kernel<17>, grid, p, sm, stream, map, map_dz); break;
+        case 5: e = launch_ln(ln_gradient_kernel<5>, grid, sm, stream, map, map_dz, p, sm); break;
+        case 9: e = launch_ln(ln_gradient_kernel<9>, grid, sm, stream, map, map_dz, p, sm); break;
+        case 15: e = launch_ln(ln_gradient_kernel<15>, grid, sm, stream, map, map_dz, p, sm); break;
+        default: e = launch_ln(ln_gradient_kernel<17>, grid, sm, stream, map, map_dz, p, sm); break;
     }
     if (e != cudaSuccess) return e;
     if (dgamma || dbeta) {
@@ -1097,6 +1278,30 @@ cudaError_t launch_ln_backward(const GradParams &g, const LnLayout &ll, const vo
         if (e != cudaSuccess) note_failure_site("dgamma/dbeta reduction launch");
     }
     return e;
+}
+
+cudaError_t launch_ln_argmax(const float *z, int64_t zs_b, int64_t zs_v, const float *gamma, const float *beta, int B, int T, int V,
+                             int64_t *argmax_out, cudaStream_t stream) {
+    if ((long long)B * T == 0) return cudaSuccess;
+    LnParams p;
+    memset(&p, 0, sizeof(p));
+    p.d.B = B; p.d.T = T; p.d.V = V;
+    p.z = z; p.zs_b = zs_b; p.zs_v = zs_v; p.gamma = gamma; p.beta = beta;
+    p.K = (V + kLnBoxRows - 1) / kLnBoxRows;
+    p.nTB = (T + kLnTT - 1) / kLnTT;
+    const LnSmem sm = plan_ln_stream(p.K, 0);
+    if (sm.R < p.K + 2) { note_failure_site("shared-memory plan"); return cudaErrorInvalidConfiguration; }
+    p.R = sm.R;
+    CUtensorMap map;
+    if (!make_z_map(&map, z, B, T, V, zs_b, zs_v)) { note_failure_site("tensor map of z"); return cudaErrorNotSupported; }
+    const long long tiles = (long long)B * p.nTB;
+    const int grid = (int)(tiles < sm_count() ? tiles : sm_count());
+    switch (ln_kmax(p.K)) {
+        case 5: return launch_ln(ln_argmax_kernel<5>, grid, sm, stream, map, p, sm, argmax_out);
+        case 9: return launch_ln(ln_argmax_kernel<9>, grid, sm, stream, map, p, sm, argmax_out);
+        case 15: return launch_ln(ln_argmax_kernel<15>, grid, sm, stream, map, p, sm, argmax_out);
+        default: return launch_ln(ln_argmax_kernel<17>, grid, sm, stream, map, p, sm, argmax_out);
+    }
 }
 
 }  // namespace b200ctc

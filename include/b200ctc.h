@@ -42,7 +42,7 @@
 extern "C" {
 #endif
 
-#define B200CTC_VERSION 201
+#define B200CTC_VERSION 202
 
 enum {
     B200CTC_OK = 0,
@@ -154,6 +154,22 @@ int b200ctc_ln_backward(int kind,
 /* Greedy path alone (run/ctc/cnn/train.py:232 and its 9 sibling call sites): out (B,T) int64. */
 int b200ctc_greedy_argmax(const float *acts, int64_t stride_t, int64_t stride_b,
                           int B, int T, int V, int64_t *argmax_out, void *stream);
+
+/*
+ * Greedy path with LayerNormalization fused in: the development loop of a model built without its final
+ * LayerNormalization (run/ctc/cnn/train.py:224-234, `xp.argmax(model(x, split_into_variables=False).data, axis=2)`).
+ *   z, gamma, beta  as for b200ctc_ln_forward (same layout and alignment rules)
+ *   argmax_out      (B,T) int64, out: argmax_v of gamma * (z - mean_v z) / std_v z + beta for EVERY frame (the reference
+ *                   decodes the padded frames too, asr/error.py:40); numpy.argmax rules: the first of equal maxima wins,
+ *                   NaN counts as maximal and the first NaN wins, the result is always in [0, V).  A frame with a NaN or
+ *                   an infinity in z, or whose V values are all 0, normalises to NaN everywhere and gives 0.
+ * z is read once; nothing else is read or written, and no workspace is needed.  Returns B200CTC_UNSUPPORTED for
+ * V > 4080 or unaligned rows (checked before the driver is touched), and when the driver cannot describe z as a TMA
+ * tensor.
+ */
+int b200ctc_ln_greedy_argmax(const float *z, int64_t zstride_b, int64_t zstride_v,
+                             const float *gamma, const float *beta,
+                             int B, int T, int V, int64_t *argmax_out, void *stream);
 
 /*
  * Evaluation path after the greedy argmax (SURVEY.md 8f rank 1): replaces compute_minibatch_error

@@ -19,6 +19,16 @@ configs[2] with V cut to the fused limit (B=32, T=600, V=4000, L<=60, variable l
   reference_style  the reference's model tail op by op, then b200ctc.gram_ctc(joint_ctc=True) on the transposed copy
 
     python tools/ln_bench.py --kind joint > profiles/r3_layernorm_joint.txt
+
+--kind argmax: the development loop's greedy ids (run/ctc/cnn/train.py:224-234) at the bench shape (B=64, T=800, V=3500),
+z (B,V,1,T) as the model's last convolution leaves it.  Arms:
+
+  fused            b200ctc.layernorm_greedy_argmax(z, gamma, beta): one read of z
+  torch_native     torch.nn.functional.layer_norm over a (B,T,V) view (one transposing copy + one fused LN kernel), then
+                   b200ctc.greedy_argmax
+  reference_style  the reference's model tail op by op, then b200ctc.greedy_argmax on the transposed copy
+
+    python tools/ln_bench.py --kind argmax > profiles/r3_layernorm_argmax.txt
 """
 import argparse, importlib, json, os, subprocess, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -170,10 +180,79 @@ def measure_joint(B=32, T=600, V=4000, L=60, steps=20, warmup=3, rounds=3):
     return out
 
 
+COPY_PEAK_GBS = 6549.8            # measured device-to-device copy peak of the B200 (DESIGN.md §3 "Roofline")
+
+
+def measure_argmax(B=64, T=800, V=3500, steps=50, warmup=5, rounds=3):
+    dev = torch.device("cuda:0")
+    g = torch.Generator(device=dev); g.manual_seed(0)
+    z = torch.randn((B, V, 1, T), device=dev, generator=g) * 1.7 + 0.3
+    gamma = 1 + 0.2 * torch.randn(V, device=dev, generator=g)
+    beta = 0.1 * torch.randn(V, device=dev, generator=g)
+
+    def fused():
+        return b200ctc.layernorm_greedy_argmax(z, gamma, beta)
+
+    def torch_native():
+        y = torch.nn.functional.layer_norm(z.squeeze(2).transpose(1, 2), (V,), gamma, beta, eps=0.0)   # (B,T,V)
+        return b200ctc.greedy_argmax(y)
+
+    def reference_style():
+        mean = z.mean(dim=(1, 2), keepdim=True)
+        diff = z - mean
+        std = torch.sqrt((diff * diff).sum(dim=(1, 2), keepdim=True) / V)
+        y = diff / std * gamma[None, :, None, None] + beta[None, :, None, None]
+        return b200ctc.greedy_argmax(y.swapaxes(1, 3).reshape(B, -1).view(B, T, V))   # the transposed copy
+
+    arms = (("fused", fused), ("torch_native", torch_native), ("reference_style", reference_style))
+    out = {name: {"ms_per_call_rounds": []} for name, _ in arms}
+    with torch.no_grad():
+        for name, fn in arms:
+            for _ in range(warmup):
+                fn()
+        torch.cuda.synchronize()
+        for _ in range(rounds):                   # the arms alternate: drift on a shared host hits all of them alike
+            for name, fn in arms:
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record()
+                for _ in range(steps):
+                    fn()
+                e1.record()
+                torch.cuda.synchronize()
+                out[name]["ms_per_call_rounds"].append(e0.elapsed_time(e1) / steps)
+        ids = {name: fn() for name, fn in arms}
+    for name, _ in arms:
+        out[name]["ms_per_call"] = float(np.median(out[name]["ms_per_call_rounds"]))
+        # the arms normalise with different float32 arithmetic: a frame whose two best values are within rounding may differ
+        out[name]["frames_agreeing_with_fused"] = float((ids[name] == ids["fused"]).double().mean())
+    nbytes = 4 * B * V * T + 8 * B * T           # read z once, write the (B,T) int64 ids
+    f = out["fused"]
+    f["algorithmic_bytes"] = nbytes
+    f["achieved_GBps"] = nbytes / (f["ms_per_call"] * 1e-3) / 1e9
+    f["share_of_copy_peak"] = f["achieved_GBps"] / COPY_PEAK_GBS
+    out["shape"] = {"B": B, "T": T, "V": V, "frames": B * T}
+    out["timing"] = "CUDA events; median of %d rounds of %d calls after %d warm-up calls per arm; z (%.0f MB) in HBM" % (
+        rounds, steps, warmup, 4.0 * B * V * T / 1e6)
+    out.update(gpu_identity())
+    return out
+
+
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("--kind", choices=("ctc", "joint"), default="ctc")
-    if ap.parse_args().kind == "joint":
+    ap.add_argument("--kind", choices=("ctc", "joint", "argmax"), default="ctc")
+    kind = ap.parse_args().kind
+    if kind == "argmax":
+        r = measure_argmax()
+        print(json.dumps(r))
+        print("# %s, power limit %s" % (r["gpu"], r["nvidia_smi_name_power_limit"]))
+        f = r["fused"]["ms_per_call"]
+        for k in ("fused", "torch_native", "reference_style"):
+            print("# %-16s %8.3f ms per call   %6.2fx the fused call   ids equal to fused on %.4f%% of frames" % (
+                k, r[k]["ms_per_call"], r[k]["ms_per_call"] / f, 100 * r[k]["frames_agreeing_with_fused"]))
+        print("# fused: %.0f algorithmic bytes (4BVT + 8BT) in %.3f ms = %.0f GB/s, %.1f%% of the %.1f GB/s copy peak" % (
+            r["fused"]["algorithmic_bytes"], f, r["fused"]["achieved_GBps"], 100 * r["fused"]["share_of_copy_peak"], COPY_PEAK_GBS))
+        sys.exit(0)
+    if kind == "joint":
         r = measure_joint()
         print(json.dumps(r))
         print("# %s, power limit %s" % (r["gpu"], r["nvidia_smi_name_power_limit"]))
