@@ -17,6 +17,14 @@ constexpr float SENT = -1.0e30f;              // exponent of probability zero ("
 constexpr float SENT_TEST = -1.0e29f;         // anything below this is treated as log 0
 constexpr float LOG2E_HI = 1.44269502162933349609375f;      // float(log2 e)
 constexpr float LOG2E_LO = 1.92596299112661746e-8f;         // log2 e - LOG2E_HI
+// Per-frame softmax normaliser of the gradient kernels, (la, s): softmax(x) = 2^(x*LOG2E_HI - la) * s.  la + lb is the
+// log2 normaliser as the lattice gets it, an unevaluated float pair; rounding la + lb to one float costs up to half an
+// ulp of la in log2 p (6e-5 relative at |logits| ~ 1000), so lb goes into the per-frame scale s instead.  s also leaves
+// out m*LOG2E_LO (m = the row maximum), as the row loop leaves out x*LOG2E_LO: what remains is (x - m)*LOG2E_LO,
+// below 1e-6 wherever the softmax is not negligible.
+__device__ __forceinline__ float2 grad_normaliser(float m, float la, float lb) {
+    return make_float2(la, exp2f(fmaf(m, LOG2E_LO, -lb)));
+}
 constexpr double LN2_D = 0.693147180559945309417232121458;
 constexpr int kProgBlock = 16;                // frames per progress counter = frames per lattice pipeline chunk
 constexpr float RINT_MAGIC = 12582912.0f;     // 1.5 * 2^23: (x + M) - M == rint(x) for |x| < 2^22
@@ -91,7 +99,7 @@ __host__ inline WsLayout make_layout(int kind, int B, int T, int V, int Lmax) {
     const size_t BT = (size_t)B * (size_t)T;
     w.off_hdr = o;   o = align_up(o + sizeof(WsHeader), 256);
     w.off_utt = o;   o = align_up(o + sizeof(UttInfo) * (size_t)B, 256);
-    w.off_lse = o;   o = align_up(o + sizeof(float) * BT, 256);
+    w.off_lse = o;   o = align_up(o + sizeof(float2) * BT, 256);     // grad_normaliser() per frame
     w.off_lp = o;    o = align_up(o + sizeof(float2) * BT * w.W, 256);
     w.off_av = o;    o = align_up(o + sizeof(float2) * BT * w.Np, 256);      // alpha_t[j] as (m, e)
     w.off_bv = o;    o = align_up(o + sizeof(float2) * BT * w.Np, 256);      // beta_t[j] (excludes emission at t), at [j + boff]

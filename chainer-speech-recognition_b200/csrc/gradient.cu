@@ -77,7 +77,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) gradient_kernel(GradParams 
     const float2 *bv2_all = reinterpret_cast<const float2 *>(ws + w.off_bv2);
     WsHeader *hdr = reinterpret_cast<WsHeader *>(ws + w.off_hdr);
     const UttInfo *utt = reinterpret_cast<const UttInfo *>(ws + w.off_utt);
-    const float *lse_all = reinterpret_cast<const float *>(ws + w.off_lse);
+    const float2 *lse_all = reinterpret_cast<const float2 *>(ws + w.off_lse);
     const float2 *av_all = reinterpret_cast<const float2 *>(ws + w.off_av);
     const float2 *bv_all = reinterpret_cast<const float2 *>(ws + w.off_bv);
     const int *uoff_all = reinterpret_cast<const int *>(ws + w.off_uoff);
@@ -100,10 +100,10 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) gradient_kernel(GradParams 
         if (t >= ui.Tb) { zero_row(grow, d.V, lane); continue; }             // :296
 
         const float *row = d.acts + (int64_t)t * d.stride_t + (int64_t)b * d.stride_b;
-        const float lse2 = lse_all[(size_t)b * d.T + t];
+        const float2 nrm = lse_all[(size_t)b * d.T + t];                     // grad_normaliser (common.cuh)
         const float gy = gp.per_utterance ? gp.grad_loss[b] : gp.grad_loss[0];
         const float sc = gy * gp.scale;                                      // :291-294
-        const float c = -lse2;
+        const float c = -nrm.x;
 
         // ---- posteriors of this frame: e[j] = alpha*beta/P[t][j], merged per emitted id (:180-217) ----
         const float2 *arow = av_all + ((size_t)b * d.T + t) * w.Np;
@@ -141,7 +141,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) gradient_kernel(GradParams 
             post_sm[u] = post * sc;
         }
         __syncwarp();
-        const float sc_soft = w.joint ? 2.f * sc : sc;                       // two losses, two softmax terms
+        const float sc_soft = (w.joint ? 2.f * sc : sc) * nrm.y;             // two losses, two softmax terms
 
         // ---- stream the row: grad = (softmax - posterior) * sc, one read and one write ----
         const unsigned *bm = bm_all + (size_t)b * w.nwords;
@@ -318,7 +318,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) gradient_ring_kernel(GradPara
     }
 
     // ===== consumers =====
-    const float *lse_all = reinterpret_cast<const float *>(ws + w.off_lse);
+    const float2 *lse_all = reinterpret_cast<const float2 *>(ws + w.off_lse);
     const int *unode_all = reinterpret_cast<const int *>(ws + w.off_unode);
     const int4 *urec_all = reinterpret_cast<const int4 *>(ws + w.off_urec);
     constexpr int kRecBatch = 4;                          // id records per lane requested in one go
@@ -345,7 +345,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) gradient_ring_kernel(GradPara
         float *e2_sm = reinterpret_cast<float *>(const_cast<float2 *>(a2_sm));
         const UttInfo ui = utt_cached ? utt_sm[b] : utt[b];
         // requested now, needed after the posteriors: their round trip hides behind the node loop
-        const float lse2 = __ldg(lse_all + (size_t)b * d.T + t);
+        const float2 nrm = __ldg(lse_all + (size_t)b * d.T + t);             // grad_normaliser (common.cuh)
         const float sc = (gp.per_utterance ? __ldg(gp.grad_loss + b) : __ldg(gp.grad_loss)) * gp.scale;      // :291-294
         const int4 *urec = urec_all + (size_t)b * w.Nmax;
         int4 rec[kRecBatch];
@@ -379,8 +379,8 @@ __global__ void __launch_bounds__(kRingThreads, 1) gradient_ring_kernel(GradPara
             }
         }
         blank_part = warp_sum(blank_part);
-        const float sc_soft = w.joint ? 2.f * sc : sc;                       // two losses, two softmax terms
-        const float c = -lse2;
+        const float sc_soft = (w.joint ? 2.f * sc : sc) * nrm.y;             // two losses, two softmax terms
+        const float c = -nrm.x;
         // softmax * sc in place, over the whole aligned span (what lies outside the row is never stored)
         float4 *row4 = reinterpret_cast<float4 *>(slotf);
 #pragma unroll 4

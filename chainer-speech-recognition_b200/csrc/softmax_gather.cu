@@ -185,7 +185,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) softmax_gather_kernel(Probl
                                                                           unsigned char *ws, int64_t *argmax_out) {
     const int lane = threadIdx.x & 31;
     WsHeader *hdr = reinterpret_cast<WsHeader *>(ws + w.off_hdr);
-    float *lse_out = reinterpret_cast<float *>(ws + w.off_lse);
+    float2 *lse_out = reinterpret_cast<float2 *>(ws + w.off_lse);
     float2 *lp_out = reinterpret_cast<float2 *>(ws + w.off_lp);
     const unsigned frames = (unsigned)d.B * (unsigned)d.T;
     // The "row written" signal of a frame is a release at GPU scope, i.e. it waits for the warp's outstanding stores.
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) softmax_gather_kernel(Probl
         float la, lb;
         split_lse2(row_max, lse2, la, lb);
         if (lane == 0 && pend_b >= 0 && d.concurrent) signal_frame_done(ws, w, pend_b, pend_t);
-        if (lane == 0) lse_out[(size_t)b * d.T + t] = la + lb;
+        if (lane == 0) lse_out[(size_t)b * d.T + t] = grad_normaliser(row_max, la, lb);
         // gather: column 0 = blank, 1..Lmax = labels, Lmax+1.. = bigrams (gram_ctc.py:24-32, :155)
         int Lb = d.label_lengths ? d.label_lengths[b] : d.Lmax;
         Lb = max(0, min(Lb, d.Lmax));
@@ -329,14 +329,18 @@ __device__ __forceinline__ bool fast_row_scan(const float4 *__restrict__ row4, i
     const bool lane_ok = sl >= 0.f && sl < 1e30f && (ref == -INFINITY || fabsf(ref) < 4194304.f);
     return __all_sync(0xffffffffu, lane_ok) && __any_sync(0xffffffffu, sl > 0.f);
 }
-__device__ __forceinline__ void fast_row_finish(float ref, float sl, float &la, float &lb) {
+// The sums above are of 2^(x*LOG2E_HI); emission_pair adds x*LOG2E_LO to every symbol, so the normaliser gets the
+// row maximum's share of it, m*LOG2E_LO with m ~ R/LOG2E_HI, as split_lse2 gives it (2e-5 in log2 p at |logits| ~ 1000).
+// m is returned for grad_normaliser.
+__device__ __forceinline__ void fast_row_finish(float ref, float sl, float &la, float &lb, float &m) {
     const float R = warp_max(ref);
     const float S = warp_sum(sl * ex2_approx(ref - R));                  // ref - R: integer <= 0 (or -inf for an empty lane)
     const float lg = log2f(S);
     const float a = R + lg;                                              // TwoSum(R, lg)
     const float bb = a - R;
+    m = R * (1.f / LOG2E_HI);
     la = a;
-    lb = (R - (a - bb)) + (lg - bb);
+    lb = fmaf(m, LOG2E_LO, (R - (a - bb)) + (lg - bb));
 }
 
 template <bool ARGMAX>
@@ -438,7 +442,7 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
     }
 
     // ===== consumers =====
-    float *lse_out = reinterpret_cast<float *>(ws + w.off_lse);
+    float2 *lse_out = reinterpret_cast<float2 *>(ws + w.off_lse);
     float2 *lp_out = reinterpret_cast<float2 *>(ws + w.off_lp);
     if (warp - 1 >= ring.nc) return;                      // short ring: fewer active consumers (row_ring.cuh)
     unsigned pushed = 0;
@@ -483,7 +487,7 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
                 for (int k = 0; k < kGatherRegs; ++k) syms[k] = (lane + 32 * k < ncol) ? symbol_of(lane + 32 * k) : -1;
             }
         }
-        float la = 0.f, lb = 0.f;
+        float la = 0.f, lb = 0.f, mx = 0.f;
         float ref = 0.f, sl = 0.f;
         bool fast = false;
         if (!ARGMAX && m.kind == 0) fast = fast_row_scan(row4, n4, lane, ref, sl);
@@ -522,7 +526,7 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
                 if (lane == 0) argmax_out[(size_t)m.b * d.T + m.t] = bi < 0 ? 0 : bi;
             }
             if (m.kind == 0) {
-                const float mx = warp_max(st.m);
+                mx = warp_max(st.m);
                 float sum = st.m == -INFINITY ? 0.f : st.s * ex2_approx((st.m - mx) * LOG2E_HI);
                 sum = warp_sum(sum);
                 split_lse2(mx, sum, la, lb);
@@ -544,16 +548,16 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&ring.empty[s]);
                 released = true;
-                if (fast) fast_row_finish(ref, sl, la, lb);
-                if (lane == 0) lse_out[(size_t)m.b * d.T + m.t] = la + lb;
+                if (fast) fast_row_finish(ref, sl, la, lb, mx);
+                if (lane == 0) lse_out[(size_t)m.b * d.T + m.t] = grad_normaliser(mx, la, lb);
 #pragma unroll
                 for (int k = 0; k < kGatherRegs; ++k) {
                     const int cidx = lane + 32 * k;
                     if (cidx < ncol) lprow[cidx] = ok[k] ? emission_pair(xv[k], la, lb) : make_float2(0.f, SENT);
                 }
             } else {
-                if (fast) fast_row_finish(ref, sl, la, lb);
-                if (lane == 0) lse_out[(size_t)m.b * d.T + m.t] = la + lb;
+                if (fast) fast_row_finish(ref, sl, la, lb, mx);
+                if (lane == 0) lse_out[(size_t)m.b * d.T + m.t] = grad_normaliser(mx, la, lb);
                 for (int cidx = lane; cidx < ncol; cidx += 32) {
                     const int sym = symbol_of(cidx);
                     float2 v = make_float2(0.f, SENT);

@@ -161,7 +161,10 @@ def utterance(logp_tv, lat, dtype=np.float64):
     T, V = logp_tv.shape
     alpha, beta = alpha_beta(logp_tv, lat, dtype)
     finals = lat.final_nodes
-    logP = _lse(alpha[T - 1, finals]) if T > 0 and finals else np.array(NEG_INF)
+    if T > 0:
+        logP = _lse(alpha[T - 1, finals]) if finals else np.array(NEG_INF)
+    else:                                               # no frames: P = 1 iff there is nothing to emit (DESIGN.md quirks)
+        logP = np.array(0.0 if lat.N == 1 else NEG_INF)
     logP = float(logP)
     post = np.zeros((T, V), dtype)
     if np.isfinite(logP):
