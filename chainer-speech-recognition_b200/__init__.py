@@ -8,6 +8,7 @@ The directory name is not a Python identifier; import it with
     asr/loss/ctc.py        connectionist_temporal_classification(...)   (reference: Chainer's, via run/ctc/*)
     asr/loss/layernorm_loss.py  layernorm_ctc(...), layernorm_gram_ctc(...), layernorm_greedy_argmax(...)   (reference: asr/nn/layernorm.py + asr/model/cnn.py:41-44 + the loss)
     asr/data/processing.py labels_to_minibatch(...)   (reference: asr/data/processing.py, label half of features_to_minibatch)
+    asr/align.py           ctc_forced_align(...), gram_ctc_forced_align(...)   (Viterbi path of the same lattices; no reference counterpart)
     asr/error.py           compute_minibatch_error(...), compute_character_error_rate(...)   (reference: asr/error.py)
     csrc/                  sm_100a kernels + the C ABI (include/b200ctc.h)
 """
@@ -17,10 +18,11 @@ from .asr.loss import (gram_ctc, joint_gram_ctc, GramCTC, connectionist_temporal
                        ConnectionistTemporalClassification, greedy_argmax, ctc_host, gram_ctc_host,
                        layernorm_ctc, layernorm_gram_ctc, layernorm_greedy_argmax, GraphedStep)
 
+from .asr.align import Alignment, ctc_forced_align, gram_ctc_forced_align
 from .asr.data import labels_to_minibatch
 from .asr.error import (compute_minibatch_error, compute_character_error_rate, build_expansion_table,
                         minibatch_error_details)
 
-__all__ = ["GraphedStep", "layernorm_ctc", "layernorm_gram_ctc", "layernorm_greedy_argmax", "labels_to_minibatch", "joint_gram_ctc", "compute_minibatch_error", "compute_character_error_rate", "build_expansion_table", "minibatch_error_details",
+__all__ = ["Alignment", "ctc_forced_align", "gram_ctc_forced_align", "GraphedStep", "layernorm_ctc", "layernorm_gram_ctc", "layernorm_greedy_argmax", "labels_to_minibatch", "joint_gram_ctc", "compute_minibatch_error", "compute_character_error_rate", "build_expansion_table", "minibatch_error_details",
            "gram_ctc", "GramCTC", "connectionist_temporal_classification", "ctc",
            "ConnectionistTemporalClassification", "greedy_argmax", "ctc_host", "gram_ctc_host", "build", "distributed", "synth"]

@@ -15,7 +15,8 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "_lib")
 SO_PATH = os.path.join(LIBDIR, "libb200ctc.so")
 STAMP = os.path.join(LIBDIR, "libb200ctc.stamp")
-SOURCES = ["api.cu", "host_cache.cu", "softmax_gather.cu", "lattice.cu", "gradient.cu", "greedy_error.cu", "layernorm_loss.cu"]
+SOURCES = ["api.cu", "host_cache.cu", "softmax_gather.cu", "lattice.cu", "gradient.cu", "greedy_error.cu", "layernorm_loss.cu",
+           "viterbi.cu"]
 HEADERS = ["common.cuh", "kernels.h", "row_ring.cuh", "prep.cuh", os.path.join("..", "..", "include", "b200ctc.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-cudart", "shared"]

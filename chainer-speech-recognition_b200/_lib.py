@@ -47,6 +47,11 @@ def _bind(lib):
         c.c_int, c.c_void_p, c.c_int64, c.c_int64, c.c_void_p, c.c_void_p, c.c_void_p, c.c_void_p,
         c.c_int, c.c_int, c.c_int, c.c_int, c.c_int, c.c_void_p, c.c_int, c.c_float,
         c.c_void_p, c.c_int64, c.c_int64, c.c_void_p, c.c_void_p, c.c_void_p, c.c_size_t, c.c_void_p]
+    lib.b200ctc_align.restype = c.c_int
+    lib.b200ctc_align.argtypes = [
+        c.c_int, c.c_void_p, c.c_int64, c.c_int64, c.c_void_p, c.c_void_p, c.c_void_p, c.c_void_p,
+        c.c_int, c.c_int, c.c_int, c.c_int, c.c_int, c.c_void_p, c.c_void_p, c.c_void_p, c.c_void_p, c.c_void_p,
+        c.c_void_p, c.c_size_t, c.c_void_p]
     lib.b200ctc_greedy_argmax.restype = c.c_int
     lib.b200ctc_greedy_argmax.argtypes = [c.c_void_p, c.c_int64, c.c_int64, c.c_int, c.c_int, c.c_int,
                                           c.c_void_p, c.c_void_p]

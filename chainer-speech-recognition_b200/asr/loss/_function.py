@@ -192,11 +192,9 @@ class LatticeLossFunction(torch.autograd.Function):
         return (grad,) + (None,) * 10
 
 
-def lattice_loss(kind, xs, labels, bigrams, blank_symbol, input_length, label_length, reduce,
-                 batch_first=False, batch_global=None, group=None, return_argmax=False):
-    """Shared front end of ``ctc`` and ``gram_ctc``: reference-style argument checks, then the kernels."""
-    if reduce not in ("mean", "no"):                             # gram_ctc.py:224-227
-        raise ValueError("only 'mean' and 'no' are valid for 'reduce', but '%s' is given" % reduce)
+def lattice_inputs(kind, xs, labels, bigrams, blank_symbol, input_length, label_length, batch_first=False):
+    """Reference-style argument checks and normalisation shared by the losses and the forced alignment: returns the
+    (T,B,V) activation view and the int32 device tensors (acts, labels, bigrams, input_length, label_length, blank)."""
     if isinstance(blank_symbol, bool) or not isinstance(blank_symbol, (int, np.integer)):   # :303-304
         raise TypeError("blank_symbol must be non-negative integer.")
     blank_symbol = int(blank_symbol)
@@ -245,6 +243,18 @@ def lattice_loss(kind, xs, labels, bigrams, blank_symbol, input_length, label_le
     for name, v in (("input_length", input_length), ("label_length", label_length)):
         if v is not None and v.shape != (B,):
             raise ValueError("%s must have shape (B,)" % name)
+    return acts, labels, bigrams, input_length, label_length, blank_symbol
+
+
+def lattice_loss(kind, xs, labels, bigrams, blank_symbol, input_length, label_length, reduce,
+                 batch_first=False, batch_global=None, group=None, return_argmax=False):
+    """Shared front end of ``ctc`` and ``gram_ctc``: reference-style argument checks, then the kernels."""
+    if reduce not in ("mean", "no"):                             # gram_ctc.py:224-227
+        raise ValueError("only 'mean' and 'no' are valid for 'reduce', but '%s' is given" % reduce)
+    acts, labels, bigrams, input_length, label_length, blank_symbol = lattice_inputs(
+        kind, xs, labels, bigrams, blank_symbol, input_length, label_length, batch_first)
+    B = acts.shape[1]
+    dev = acts.device
     if batch_global is None:
         batch_global = B
         if group is not None and reduce == "mean":

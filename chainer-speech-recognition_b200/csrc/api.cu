@@ -296,6 +296,51 @@ int b200ctc_ln_backward(int kind, const float *z, int64_t zstride_b, int64_t zst
                       "layernorm gradient kernel");
 }
 
+int b200ctc_align(int kind, const float *acts, int64_t stride_t, int64_t stride_b, const int32_t *labels,
+                  const int32_t *bigrams, const int32_t *input_lengths, const int32_t *label_lengths, int blank, int B, int T,
+                  int V, int Lmax, float *score, int32_t *path, int64_t *ids, float *frame_logp, int32_t *spans,
+                  void *workspace, size_t workspace_bytes, void *stream_) {
+    if (kind != B200CTC_KIND_CTC && kind != B200CTC_KIND_GRAM)
+        return fail(B200CTC_INVALID_ARGUMENT, "alignment needs kind 0 (CTC) or 1 (Gram-CTC): the best path of a sum of two "
+                                              "losses is not an alignment%s");
+    int rc = validate(kind, B, T, V, Lmax, blank, true);
+    if (rc) return rc;
+    if (B == 0) return B200CTC_OK;
+    const bool frames = (size_t)B * T > 0;
+    if (!acts && frames) return fail(B200CTC_INVALID_ARGUMENT, "acts is NULL%s");
+    if (!labels && Lmax > 0) return fail(B200CTC_INVALID_ARGUMENT, "labels is NULL%s");
+    if (kind == B200CTC_KIND_GRAM && !bigrams && Lmax > 0) return fail(B200CTC_INVALID_ARGUMENT, "bigrams is NULL for Gram-CTC%s");
+    if (!score || ((!path || !ids) && frames) || !workspace)
+        return fail(B200CTC_INVALID_ARGUMENT, "output or workspace pointer is NULL%s");
+    if ((reinterpret_cast<uintptr_t>(workspace) & 15) != 0) return fail(B200CTC_INVALID_ARGUMENT, "workspace must be 16-byte aligned%s");
+    if ((reinterpret_cast<uintptr_t>(acts) & 3) != 0) return fail(B200CTC_INVALID_ARGUMENT, "acts must be 4-byte aligned%s");
+    const WsLayout w = make_layout(kind, B, T, V, Lmax);
+    if (workspace_bytes < w.total)
+        return fail(B200CTC_WORKSPACE_TOO_SMALL, "workspace too small%s: %lld < %lld bytes", "", (long long)workspace_bytes,
+                    (long long)w.total);
+    if (align_smem_bytes(w, nullptr) > 227 * 1024)
+        return fail(B200CTC_UNSUPPORTED, "lattice of %s%lld nodes does not fit the alignment kernel's shared memory", "", w.Nmax);
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+
+    ProblemDesc d;
+    d.kind = kind; d.B = B; d.T = T; d.V = V; d.Lmax = Lmax; d.blank = blank;
+    d.acts = acts; d.stride_t = stride_t; d.stride_b = stride_b;
+    d.labels = labels; d.bigrams = kind == B200CTC_KIND_GRAM ? bigrams : nullptr;
+    d.input_lengths = input_lengths; d.label_lengths = label_lengths;
+    d.concurrent = 0;
+    unsigned char *ws = static_cast<unsigned char *>(workspace);
+    const int nprog = B * w.nblk;
+    zero_header_kernel<<<(nprog + 255) / 256 > 0 ? (nprog + 255) / 256 : 1, 256, 0, stream>>>(
+        reinterpret_cast<WsHeader *>(ws + w.off_hdr), reinterpret_cast<unsigned *>(ws + w.off_prog), nprog);
+    if ((rc = check_cuda(cudaGetLastError(), "workspace header reset"))) return rc;
+    if ((rc = check_cuda(launch_softmax_gather(d, w, ws, nullptr, 0, stream), "softmax/gather kernel"))) return rc;
+    AlignParams a;
+    a.d = d; a.w = w; a.ws = ws;
+    a.score = score; a.path = path; a.ids = ids; a.frame_logp = frame_logp; a.spans = spans;
+    a.buf_stride = 0; a.chunk = 0;
+    return check_cuda(launch_align(a, stream), "alignment kernel");
+}
+
 int b200ctc_greedy_argmax(const float *acts, int64_t stride_t, int64_t stride_b, int B, int T, int V,
                           int64_t *argmax_out, void *stream_) {
     if (B < 0 || T < 0 || V <= 0) return fail(B200CTC_INVALID_ARGUMENT, "bad dimensions%s");

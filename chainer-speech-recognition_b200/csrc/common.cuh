@@ -78,6 +78,9 @@ struct WsLayout {
 
 __host__ __device__ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// An utterance's input or label length as every kernel reads it: clamped into [0, hi] (T or Lmax)
+__host__ __device__ inline int clamp_length(int v, int hi) { return v < 0 ? 0 : (v > hi ? hi : v); }
+
 // kind: 0 = CTC, 1 = Gram-CTC, 2 = joint Gram-CTC + CTC (laid out as Gram-CTC plus a second lattice)
 __host__ inline WsLayout make_layout(int kind, int B, int T, int V, int Lmax) {
     WsLayout w;

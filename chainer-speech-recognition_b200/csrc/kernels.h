@@ -88,6 +88,28 @@ cudaError_t launch_ln_backward(const GradParams &g, const LnLayout &ll, const vo
 cudaError_t launch_ln_argmax(const float *z, int64_t zs_b, int64_t zs_v, const float *gamma, const float *beta, int B, int T, int V,
                              int64_t *argmax_out, cudaStream_t stream);
 
+// forced alignment (viterbi.cu): best path through the lattice on the emission rows of kernel 1, backpointers in the
+// workspace's alpha region
+struct AlignParams {
+    ProblemDesc d;
+    WsLayout w;
+    unsigned char *ws;
+    float *score;            // (B)
+    int32_t *path;           // (B,T)
+    int64_t *ids;            // (B,T)
+    float *frame_logp;       // (B,T) or NULL
+    int32_t *spans;          // (B,Lmax,2) or NULL
+    int buf_stride, chunk;   // set by launch_align
+};
+struct AlignGeometry {
+    int threads, npt;        // block size, consecutive lattice nodes per thread
+    int stride;              // pitch of a score row in shared memory (float2)
+    int chunk;               // frames per emission stage
+};
+// dynamic shared memory of the alignment kernel for this layout, and its geometry (g may be NULL)
+size_t align_smem_bytes(const WsLayout &w, AlignGeometry *g);
+cudaError_t launch_align(AlignParams p, cudaStream_t stream);
+
 // evaluation path: greedy collapse + gram expansion + edit distance + error rate (greedy_error.cu)
 cudaError_t launch_greedy_error(const int64_t *argmax, const int32_t *input_lengths, int B, int T, const int32_t *labels,
                                 int Lmax, int blank, const int32_t *expansion, int V, int E, int wrap8, int32_t *hyp,

@@ -42,7 +42,7 @@
 extern "C" {
 #endif
 
-#define B200CTC_VERSION 202
+#define B200CTC_VERSION 203
 
 enum {
     B200CTC_OK = 0,
@@ -150,6 +150,34 @@ int b200ctc_ln_backward(int kind,
                         const float *grad_loss, int per_utterance, float scale,
                         float *dz, int64_t dzstride_b, int64_t dzstride_v, float *dgamma, float *dbeta,
                         const void *workspace, size_t workspace_bytes, void *stream);
+
+/*
+ * Forced alignment: the best path through the same lattice as b200ctc_forward, under the (max, x) semiring.
+ * kind is B200CTC_KIND_CTC or B200CTC_KIND_GRAM (JOINT -> B200CTC_INVALID_ARGUMENT: the best path of a sum of two losses
+ * is not an alignment).  Activations, labels, lengths (clamped into [0, T] / [0, Lmax] as the loss clamps them), the
+ * lattice size limits and the workspace (b200ctc_workspace_bytes of the same kind) are those of b200ctc_forward.
+ *   score       (B) float32, out: -ln of the best path's probability (so score >= the loss); exactly 1e10 when no
+ *               alignment exists, 0 for input length = label length = 0, NaN when a valid frame holds a NaN.
+ *   path        (B,T) int32, out: lattice node per frame (CTC: 2i+1 = label i, even = blank; Gram-CTC: 3i = blank,
+ *               3i+1 = unigram i, 3i+2 = bigram i covering labels i-1 and i); -1 beyond the input length and for an
+ *               utterance without an alignment (infeasible or NaN).
+ *   ids         (B,T) int64, out: vocabulary id of that node; the blank id where path is -1.  The greedy-id layout of
+ *               b200ctc_greedy_error.
+ *   frame_logp  (B,T) float32 or NULL, out: ln softmax(x_t)[ids[t]] on the path, 0 where path is -1.
+ *   spans       (B,Lmax,2) int32 or NULL, out: [first frame, last frame + 1) of the node that emits label position i
+ *               (a bigram node gives both its positions its span); (-1, -1) for i >= the label length and for an
+ *               utterance without an alignment.
+ * Ties between exactly equal scores: among a node's predecessors the smallest back-offset wins (self-loop, j-1, j-2,
+ * j-3, j-5, j-6, j-7); among the end nodes the final blank, then N-2, then N-3.  Results are bit-identical from run to
+ * run and between a batched call and calls on single utterances.  Work is enqueued on `stream` only.
+ */
+int b200ctc_align(int kind, const float *acts, int64_t stride_t, int64_t stride_b,
+                  const int32_t *labels, const int32_t *bigrams,
+                  const int32_t *input_lengths, const int32_t *label_lengths,
+                  int blank, int B, int T, int V, int Lmax,
+                  float *score, int32_t *path, int64_t *ids,
+                  float *frame_logp, int32_t *spans,
+                  void *workspace, size_t workspace_bytes, void *stream);
 
 /* Greedy path alone (run/ctc/cnn/train.py:232 and its 9 sibling call sites): out (B,T) int64. */
 int b200ctc_greedy_argmax(const float *acts, int64_t stride_t, int64_t stride_b,
