@@ -192,12 +192,65 @@ class LatticeLossFunction(torch.autograd.Function):
         return (grad,) + (None,) * 10
 
 
-def lattice_inputs(kind, xs, labels, bigrams, blank_symbol, input_length, label_length, batch_first=False):
-    """Reference-style argument checks and normalisation shared by the losses and the forced alignment: returns the
-    (T,B,V) activation view and the int32 device tensors (acts, labels, bigrams, input_length, label_length, blank)."""
-    if isinstance(blank_symbol, bool) or not isinstance(blank_symbol, (int, np.integer)):   # :303-304
+def check_reduce(reduce):
+    if reduce not in ("mean", "no"):                             # gram_ctc.py:224-227
+        raise ValueError("only 'mean' and 'no' are valid for 'reduce', but '%s' is given" % reduce)
+
+
+def check_blank(blank_symbol):
+    if isinstance(blank_symbol, bool) or not isinstance(blank_symbol, (int, np.integer)):   # gram_ctc.py:303-304
         raise TypeError("blank_symbol must be non-negative integer.")
-    blank_symbol = int(blank_symbol)
+    return int(blank_symbol)
+
+
+def label_inputs(kind, B, V, dev, labels, bigrams, blank_symbol, input_length, label_length):
+    """Reference-style checks and normalisation of everything but the activations, shared by every loss path and the
+    forced alignment: returns the int32 device tensors (labels, bigrams, input_length, label_length) and the blank id."""
+    blank_symbol = check_blank(blank_symbol)
+    assert blank_symbol >= 0                                     # gram_ctc.py:305
+    assert blank_symbol < V                                      # :306
+    labels = _as_int32(labels, dev, "labels")                    # :234
+    if labels.dim() != 2 or labels.shape[0] != B:
+        raise ValueError("labels must have shape (B, Lmax)")
+    if kind != _lib.KIND_CTC:
+        bigrams = _as_int32(bigrams, dev, "label_bigram")        # :235
+        assert labels.shape[1] == bigrams.shape[1]               # :308
+        if bigrams.shape != labels.shape:
+            raise ValueError("label_bigram must have the shape of label_unigram")
+    else:
+        bigrams = None
+    if input_length is None:
+        # gram_ctc.py:310-313 (and Chainer's CTC, which it derives from): when input_length is omitted BOTH lengths
+        # default to the full padded widths -- a label_length passed without an input_length is ignored there, so it
+        # is ignored here
+        label_length = None
+    input_length = _as_int32(input_length, dev, "input_length")
+    label_length = _as_int32(label_length, dev, "label_length")
+    for name, v in (("input_length", input_length), ("label_length", label_length)):
+        if v is not None and v.shape != (B,):
+            raise ValueError("%s must have shape (B,)" % name)
+    return labels, bigrams, input_length, label_length, blank_symbol
+
+
+def resolve_batch_global(B, batch_global, group, reduce, dev):
+    """The denominator of the 'mean' loss: the local batch size, or the sum over `group` of the local batch sizes."""
+    if batch_global is None:
+        batch_global = B
+        if group is not None and reduce == "mean":
+            # shards may differ in size (distributed.shard_range): the mean's denominator is the sum of the local
+            # batch sizes, agreed on with one small all-reduce (a host sync -- pass batch_global to avoid it)
+            import torch.distributed as dist
+            n = torch.tensor([B], dtype=torch.int64, device=dev)
+            dist.all_reduce(n, op=dist.ReduceOp.SUM, group=group)
+            batch_global = int(n.item())
+    return batch_global
+
+
+def lattice_inputs(kind, xs, labels, bigrams, blank_symbol, input_length, label_length, batch_first=False):
+    """Reference-style argument checks and normalisation of the losses on activations and of the forced alignment:
+    returns the (T,B,V) activation view and the int32 device tensors (acts, labels, bigrams, input_length, label_length,
+    blank)."""
+    check_blank(blank_symbol)
     if not isinstance(xs, (torch.Tensor, collections.abc.Sequence)):
         xs = as_device_tensor(xs, "xs")                          # CuPy array / Chainer Variable / DLPack capsule owner
     elif not isinstance(xs, torch.Tensor) and len(xs) > 0 and not isinstance(xs[0], torch.Tensor):
@@ -220,50 +273,16 @@ def lattice_inputs(kind, xs, labels, bigrams, blank_symbol, input_length, label_
     if acts.stride(2) != 1 and acts.shape[2] > 1:
         acts = acts.contiguous()
     T, B, V = acts.shape
-    assert blank_symbol >= 0                                     # :305
-    assert blank_symbol < V                                      # :306
-    dev = acts.device
-    labels = _as_int32(labels, dev, "labels")                    # :234
-    if labels.dim() != 2 or labels.shape[0] != B:
-        raise ValueError("labels must have shape (B, Lmax)")
-    if kind != _lib.KIND_CTC:
-        bigrams = _as_int32(bigrams, dev, "label_bigram")        # :235
-        assert labels.shape[1] == bigrams.shape[1]               # :308
-        if bigrams.shape != labels.shape:
-            raise ValueError("label_bigram must have the shape of label_unigram")
-    else:
-        bigrams = None
-    if input_length is None:
-        # gram_ctc.py:310-313 (and Chainer's CTC, which it derives from): when input_length is omitted BOTH lengths
-        # default to the full padded widths -- a label_length passed without an input_length is ignored there, so it
-        # is ignored here
-        label_length = None
-    input_length = _as_int32(input_length, dev, "input_length")
-    label_length = _as_int32(label_length, dev, "label_length")
-    for name, v in (("input_length", input_length), ("label_length", label_length)):
-        if v is not None and v.shape != (B,):
-            raise ValueError("%s must have shape (B,)" % name)
-    return acts, labels, bigrams, input_length, label_length, blank_symbol
+    return (acts,) + label_inputs(kind, B, V, acts.device, labels, bigrams, blank_symbol, input_length, label_length)
 
 
 def lattice_loss(kind, xs, labels, bigrams, blank_symbol, input_length, label_length, reduce,
                  batch_first=False, batch_global=None, group=None, return_argmax=False):
     """Shared front end of ``ctc`` and ``gram_ctc``: reference-style argument checks, then the kernels."""
-    if reduce not in ("mean", "no"):                             # gram_ctc.py:224-227
-        raise ValueError("only 'mean' and 'no' are valid for 'reduce', but '%s' is given" % reduce)
+    check_reduce(reduce)
     acts, labels, bigrams, input_length, label_length, blank_symbol = lattice_inputs(
         kind, xs, labels, bigrams, blank_symbol, input_length, label_length, batch_first)
-    B = acts.shape[1]
-    dev = acts.device
-    if batch_global is None:
-        batch_global = B
-        if group is not None and reduce == "mean":
-            # shards may differ in size (distributed.shard_range): the mean's denominator is the sum of the local
-            # batch sizes, agreed on with one small all-reduce (a host sync -- pass batch_global to avoid it)
-            import torch.distributed as dist
-            n = torch.tensor([B], dtype=torch.int64, device=dev)
-            dist.all_reduce(n, op=dist.ReduceOp.SUM, group=group)
-            batch_global = int(n.item())
+    batch_global = resolve_batch_global(acts.shape[1], batch_global, group, reduce, acts.device)
     return LatticeLossFunction.apply(acts, kind, labels, bigrams, input_length, label_length, blank_symbol,
                                      reduce, batch_global, group, return_argmax)
 

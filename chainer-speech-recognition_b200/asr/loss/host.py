@@ -22,7 +22,7 @@ import numpy as np
 import torch
 
 from ... import _lib
-from ._function import _as_int32
+from ._function import check_blank, check_reduce, label_inputs
 
 _streams = {}
 _pool = None
@@ -81,10 +81,8 @@ def lattice_loss_host(kind, x_host, labels, bigrams, blank_symbol, input_length,
                       grad_out=None, groups=16, device=None, gy=1.0):
     """x_host: (B,T,V) float32 host tensor / ndarray.  Returns (loss, grad_host): loss a Python float ('mean') or a
     (B,) ndarray ('no'); grad_host a (B,T,V) host tensor = d loss / d x (times gy)."""
-    if reduce not in ("mean", "no"):
-        raise ValueError("only 'mean' and 'no' are valid for 'reduce', but '%s' is given" % reduce)
-    if isinstance(blank_symbol, bool) or not isinstance(blank_symbol, (int, np.integer)):
-        raise TypeError("blank_symbol must be non-negative integer.")
+    check_reduce(reduce)
+    check_blank(blank_symbol)
     if not torch.cuda.is_available():
         raise RuntimeError("b200ctc has no CPU path: a CUDA device is required")
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
@@ -93,20 +91,17 @@ def lattice_loss_host(kind, x_host, labels, bigrams, blank_symbol, input_length,
         raise TypeError("activations must be a float32 (B,T,V) array")
     x_host = x_host.contiguous()
     B, T, V = x_host.shape
-    assert 0 <= int(blank_symbol) < V
     if grad_out is None:
         grad_out = torch.empty((B, T, V), dtype=torch.float32, pin_memory=True)
     elif not (isinstance(grad_out, torch.Tensor) and grad_out.dtype == torch.float32 and not grad_out.is_cuda and
               tuple(grad_out.shape) == (B, T, V) and grad_out.is_contiguous()):
         raise ValueError("grad_out must be a contiguous float32 host tensor of shape (B,T,V)")
-    labels = _as_int32(labels, dev, "labels")
-    bigrams = _as_int32(bigrams, dev, "label_bigram") if kind == _lib.KIND_GRAM else None
     il_host = None
     if input_length is not None:
         il_host = (input_length.detach().cpu().numpy() if isinstance(input_length, torch.Tensor)
                    else np.asarray(input_length)).astype(np.int64)
-    input_length = _as_int32(input_length, dev, "input_length")
-    label_length = _as_int32(label_length, dev, "label_length")
+    labels, bigrams, input_length, label_length, blank_symbol = label_inputs(
+        kind, B, V, dev, labels, bigrams, blank_symbol, input_length, label_length)
     s_in, s_run, s_out = _get_streams(dev)
     cur = torch.cuda.current_stream(dev)
     for s in (s_in, s_run, s_out):
@@ -148,7 +143,7 @@ def lattice_loss_host(kind, x_host, labels, bigrams, blank_symbol, input_length,
             loss_b, loss_red = _raw_forward_backward(
                 kind, x_dev[b0:b1].transpose(0, 1), labels[b0:b1], None if bigrams is None else bigrams[b0:b1],
                 None if input_length is None else input_length[b0:b1],
-                None if label_length is None else label_length[b0:b1], int(blank_symbol), loss_scale,
+                None if label_length is None else label_length[b0:b1], blank_symbol, loss_scale,
                 loss_scale, g_dev[b0:b1].transpose(0, 1), gy_one, s_run)
             parts.append((loss_b, loss_red))
             e_run = torch.cuda.Event(); e_run.record(s_run)

@@ -19,11 +19,10 @@ normalised tensor, its transpose and their gradients are never materialised (csr
     y = layernorm_greedy_argmax(z, ln.gamma, ln.beta)              # the development loop's greedy ids, (B, T)
     # instead of:  y = xp.argmax(model(x, split_into_variables=False).data, axis=2)
 """
-import numpy as np
 import torch
 
 from ... import _lib
-from ._function import _as_int32, _flags, _stream_ptr, as_device_tensor
+from ._function import _flags, _stream_ptr, as_device_tensor, check_blank, check_reduce, label_inputs, resolve_batch_global
 
 
 class LayerNormLossFunction(torch.autograd.Function):
@@ -108,35 +107,13 @@ def _layernorm_inputs(z, gamma, beta):
 
 def _layernorm_loss(kind, z, gamma, beta, labels, bigrams, blank_symbol, input_length, label_length, reduce,
                     batch_global=None, group=None):
-    if reduce not in ("mean", "no"):                             # gram_ctc.py:224-227
-        raise ValueError("only 'mean' and 'no' are valid for 'reduce', but '%s' is given" % reduce)
-    if isinstance(blank_symbol, bool) or not isinstance(blank_symbol, (int, np.integer)):   # :303-304
-        raise TypeError("blank_symbol must be non-negative integer.")
+    check_reduce(reduce)
+    check_blank(blank_symbol)
     z3, gamma, beta = _layernorm_inputs(z, gamma, beta)
     B, V, T = z3.shape
-    dev = z3.device
-    blank_symbol = int(blank_symbol)
-    assert 0 <= blank_symbol < V                                 # :305-306
-    labels = _as_int32(labels, dev, "labels")
-    if labels.dim() != 2 or labels.shape[0] != B:
-        raise ValueError("labels must have shape (B, Lmax)")
-    if kind != _lib.KIND_CTC:
-        bigrams = _as_int32(bigrams, dev, "label_bigram")
-        if bigrams.shape != labels.shape:
-            raise ValueError("label_bigram must have the shape of label_unigram")
-    else:
-        bigrams = None
-    if input_length is None:
-        label_length = None                                      # :310-313: both default together
-    input_length = _as_int32(input_length, dev, "input_length")
-    label_length = _as_int32(label_length, dev, "label_length")
-    if batch_global is None:
-        batch_global = B
-        if group is not None and reduce == "mean":
-            import torch.distributed as dist
-            n = torch.tensor([B], dtype=torch.int64, device=dev)
-            dist.all_reduce(n, op=dist.ReduceOp.SUM, group=group)
-            batch_global = int(n.item())
+    labels, bigrams, input_length, label_length, blank_symbol = label_inputs(
+        kind, B, V, z3.device, labels, bigrams, blank_symbol, input_length, label_length)
+    batch_global = resolve_batch_global(B, batch_global, group, reduce, z3.device)
     out = LayerNormLossFunction.apply(z3, gamma, beta, kind, labels, bigrams, input_length, label_length, blank_symbol,
                                       reduce, batch_global, group)
     return out

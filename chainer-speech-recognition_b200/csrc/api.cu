@@ -93,6 +93,44 @@ int validate(int kind, int B, int T, int V, int Lmax, int blank, bool need_blank
     return B200CTC_OK;
 }
 
+// The problem as the kernels see it: kind 0 (CTC) or 1 (Gram-CTC; a joint call adds its CTC lattice itself), bigrams for
+// Gram-CTC only
+ProblemDesc make_desc(int kind, const float *acts, int64_t stride_t, int64_t stride_b, const int32_t *labels,
+                      const int32_t *bigrams, const int32_t *input_lengths, const int32_t *label_lengths, int blank, int B, int T,
+                      int V, int Lmax) {
+    ProblemDesc d;
+    d.kind = kind == B200CTC_KIND_CTC ? 0 : 1; d.B = B; d.T = T; d.V = V; d.Lmax = Lmax; d.blank = blank;
+    d.acts = acts; d.stride_t = stride_t; d.stride_b = stride_b;
+    d.labels = labels; d.bigrams = kind != B200CTC_KIND_CTC ? bigrams : nullptr;
+    d.input_lengths = input_lengths; d.label_lengths = label_lengths;
+    d.concurrent = 0;
+    return d;
+}
+
+// The pointer, alignment and size checks the loss and the alignment share (outputs_ok: the caller's output pointers are
+// there); `need` is the workspace the call uses
+int check_buffers(int kind, int Lmax, const float *acts, bool need_acts, const int32_t *labels, const int32_t *bigrams,
+                  bool outputs_ok, const void *workspace, size_t workspace_bytes, size_t need) {
+    if (need_acts && !acts) return fail(B200CTC_INVALID_ARGUMENT, "acts is NULL%s");
+    if (!labels && Lmax > 0) return fail(B200CTC_INVALID_ARGUMENT, "labels is NULL%s");
+    if (kind != B200CTC_KIND_CTC && !bigrams && Lmax > 0) return fail(B200CTC_INVALID_ARGUMENT, "bigrams is NULL for Gram-CTC%s");
+    if (!outputs_ok || !workspace) return fail(B200CTC_INVALID_ARGUMENT, "output or workspace pointer is NULL%s");
+    if ((reinterpret_cast<uintptr_t>(workspace) & 15) != 0) return fail(B200CTC_INVALID_ARGUMENT, "workspace must be 16-byte aligned%s");
+    if ((reinterpret_cast<uintptr_t>(acts) & 3) != 0) return fail(B200CTC_INVALID_ARGUMENT, "acts must be 4-byte aligned%s");
+    if (workspace_bytes < need)
+        return fail(B200CTC_WORKSPACE_TOO_SMALL, "workspace too small%s: %lld < %lld bytes", "", (long long)workspace_bytes,
+                    (long long)need);
+    return B200CTC_OK;
+}
+
+// zeroes the workspace header and the frame-progress counters in stream order, ahead of a softmax/gather launch
+int reset_workspace_header(const WsLayout &w, unsigned char *ws, cudaStream_t stream) {
+    const int nprog = w.B * w.nblk;
+    zero_header_kernel<<<(nprog + 255) / 256 > 0 ? (nprog + 255) / 256 : 1, 256, 0, stream>>>(
+        reinterpret_cast<WsHeader *>(ws + w.off_hdr), reinterpret_cast<unsigned *>(ws + w.off_prog), nprog);
+    return check_cuda(cudaGetLastError(), "workspace header reset");
+}
+
 // LayerNormalization fused in front of the loss (layernorm_loss.cu): z (B, V, T) + gamma/beta instead of activations
 struct LnInput {
     const float *z;
@@ -106,7 +144,6 @@ int forward_impl(const LnInput *ln, int kind, const float *acts, int64_t stride_
                  void *workspace, size_t workspace_bytes, unsigned flags, void *stream_) {
     int rc = validate(kind, B, T, V, Lmax, blank, true);
     if (rc) return rc;
-    if (!ln && !acts && (size_t)B * T > 0) return fail(B200CTC_INVALID_ARGUMENT, "acts is NULL%s");
     if (ln) {
         if ((!ln->z && (size_t)B * T > 0) || !ln->gamma || !ln->beta) return fail(B200CTC_INVALID_ARGUMENT, "z, gamma or beta is NULL%s");
         if (argmax_out) return fail(B200CTC_UNSUPPORTED, "the fused LayerNormalization path has no greedy output%s");
@@ -115,31 +152,17 @@ int forward_impl(const LnInput *ln, int kind, const float *acts, int64_t stride_
                                              "backward tile fits shared memory at this V, and 16-byte aligned rows of z "
                                              "(pitch %% 4 == 0)%s");
     }
-    if (!labels && Lmax > 0) return fail(B200CTC_INVALID_ARGUMENT, "labels is NULL%s");
-    if (kind != B200CTC_KIND_CTC && !bigrams && Lmax > 0) return fail(B200CTC_INVALID_ARGUMENT, "bigrams is NULL for Gram-CTC%s");
-    if (!loss_per_utt || !loss_reduced || !workspace) return fail(B200CTC_INVALID_ARGUMENT, "output or workspace pointer is NULL%s");
-    if ((reinterpret_cast<uintptr_t>(workspace) & 15) != 0) return fail(B200CTC_INVALID_ARGUMENT, "workspace must be 16-byte aligned%s");
-    if ((reinterpret_cast<uintptr_t>(acts) & 3) != 0) return fail(B200CTC_INVALID_ARGUMENT, "acts must be 4-byte aligned%s");
     const LnLayout ll = ln ? make_ln_layout(kind, B, T, V, Lmax) : LnLayout();
     const WsLayout w = ln ? ll.w : make_layout(kind, B, T, V, Lmax);
-    const size_t need = ln ? ll.total : w.total;
-    if (workspace_bytes < need)
-        return fail(B200CTC_WORKSPACE_TOO_SMALL, "workspace too small%s: %lld < %lld bytes", "", (long long)workspace_bytes,
-                    (long long)need);
+    if ((rc = check_buffers(kind, Lmax, acts, !ln && (size_t)B * T > 0, labels, bigrams, loss_per_utt && loss_reduced, workspace,
+                            workspace_bytes, ln ? ll.total : w.total)))
+        return rc;
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     if (B == 0) return check_cuda(cudaMemsetAsync(loss_reduced, 0, sizeof(float), stream), "memset");
 
-    ProblemDesc d;
-    d.kind = kind == B200CTC_KIND_CTC ? 0 : 1; d.B = B; d.T = T; d.V = V; d.Lmax = Lmax; d.blank = blank;
-    d.acts = acts; d.stride_t = stride_t; d.stride_b = stride_b;
-    d.labels = labels; d.bigrams = kind != B200CTC_KIND_CTC ? bigrams : nullptr;
-    d.input_lengths = input_lengths; d.label_lengths = label_lengths;
-    d.concurrent = 0;
+    ProblemDesc d = make_desc(kind, acts, stride_t, stride_b, labels, bigrams, input_lengths, label_lengths, blank, B, T, V, Lmax);
     unsigned char *ws = static_cast<unsigned char *>(workspace);
-    const int nprog = B * w.nblk;
-    zero_header_kernel<<<(nprog + 255) / 256 > 0 ? (nprog + 255) / 256 : 1, 256, 0, stream>>>(
-        reinterpret_cast<WsHeader *>(ws + w.off_hdr), reinterpret_cast<unsigned *>(ws + w.off_prog), nprog);
-    if ((rc = check_cuda(cudaGetLastError(), "workspace header reset"))) return rc;
+    if ((rc = reset_workspace_header(w, ws, stream))) return rc;
 
     LatticeParams lp;
     lp.d = d; lp.w = w; lp.ws = ws;
@@ -237,10 +260,7 @@ int b200ctc_backward(int kind, const float *acts, int64_t stride_t, int64_t stri
     const WsLayout w = make_layout(kind, B, T, V, Lmax);
     if (workspace_bytes < w.total) return fail(B200CTC_WORKSPACE_TOO_SMALL, "workspace too small%s");
     GradParams g;
-    g.d.kind = kind == B200CTC_KIND_CTC ? 0 : 1; g.d.B = B; g.d.T = T; g.d.V = V; g.d.Lmax = Lmax; g.d.blank = blank;
-    g.d.acts = acts; g.d.stride_t = stride_t; g.d.stride_b = stride_b;
-    g.d.labels = labels; g.d.bigrams = bigrams; g.d.input_lengths = nullptr; g.d.label_lengths = nullptr;
-    g.d.concurrent = 0;
+    g.d = make_desc(kind, acts, stride_t, stride_b, labels, bigrams, nullptr, nullptr, blank, B, T, V, Lmax);
     g.grad_loss = grad_loss; g.per_utterance = per_utterance; g.scale = scale;
     g.grad_out = grad_out; g.gstride_t = gstride_t; g.gstride_b = gstride_b;
     return check_cuda(launch_gradient(g, w, workspace, static_cast<cudaStream_t>(stream_)), "gradient kernel");
@@ -285,10 +305,7 @@ int b200ctc_ln_backward(int kind, const float *z, int64_t zstride_b, int64_t zst
     const LnLayout ll = make_ln_layout(kind, B, T, V, Lmax);
     if (workspace_bytes < ll.total) return fail(B200CTC_WORKSPACE_TOO_SMALL, "workspace too small%s");
     GradParams g;
-    g.d.kind = kind == B200CTC_KIND_CTC ? 0 : 1; g.d.B = B; g.d.T = T; g.d.V = V; g.d.Lmax = Lmax; g.d.blank = blank;
-    g.d.acts = nullptr; g.d.stride_t = 0; g.d.stride_b = 0;
-    g.d.labels = labels; g.d.bigrams = bigrams; g.d.input_lengths = nullptr; g.d.label_lengths = nullptr;
-    g.d.concurrent = 0;
+    g.d = make_desc(kind, nullptr, 0, 0, labels, bigrams, nullptr, nullptr, blank, B, T, V, Lmax);
     g.grad_loss = grad_loss; g.per_utterance = per_utterance; g.scale = scale;
     g.grad_out = nullptr; g.gstride_t = 0; g.gstride_b = 0;
     return check_cuda(launch_ln_backward(g, ll, workspace, z, zstride_b, zstride_v, gamma, beta, dz, dzstride_b, dzstride_v, dgamma,
@@ -307,32 +324,17 @@ int b200ctc_align(int kind, const float *acts, int64_t stride_t, int64_t stride_
     if (rc) return rc;
     if (B == 0) return B200CTC_OK;
     const bool frames = (size_t)B * T > 0;
-    if (!acts && frames) return fail(B200CTC_INVALID_ARGUMENT, "acts is NULL%s");
-    if (!labels && Lmax > 0) return fail(B200CTC_INVALID_ARGUMENT, "labels is NULL%s");
-    if (kind == B200CTC_KIND_GRAM && !bigrams && Lmax > 0) return fail(B200CTC_INVALID_ARGUMENT, "bigrams is NULL for Gram-CTC%s");
-    if (!score || ((!path || !ids) && frames) || !workspace)
-        return fail(B200CTC_INVALID_ARGUMENT, "output or workspace pointer is NULL%s");
-    if ((reinterpret_cast<uintptr_t>(workspace) & 15) != 0) return fail(B200CTC_INVALID_ARGUMENT, "workspace must be 16-byte aligned%s");
-    if ((reinterpret_cast<uintptr_t>(acts) & 3) != 0) return fail(B200CTC_INVALID_ARGUMENT, "acts must be 4-byte aligned%s");
     const WsLayout w = make_layout(kind, B, T, V, Lmax);
-    if (workspace_bytes < w.total)
-        return fail(B200CTC_WORKSPACE_TOO_SMALL, "workspace too small%s: %lld < %lld bytes", "", (long long)workspace_bytes,
-                    (long long)w.total);
+    if ((rc = check_buffers(kind, Lmax, acts, frames, labels, bigrams, score && ((path && ids) || !frames), workspace, workspace_bytes,
+                            w.total)))
+        return rc;
     if (align_smem_bytes(w, nullptr) > 227 * 1024)
         return fail(B200CTC_UNSUPPORTED, "lattice of %s%lld nodes does not fit the alignment kernel's shared memory", "", w.Nmax);
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
 
-    ProblemDesc d;
-    d.kind = kind; d.B = B; d.T = T; d.V = V; d.Lmax = Lmax; d.blank = blank;
-    d.acts = acts; d.stride_t = stride_t; d.stride_b = stride_b;
-    d.labels = labels; d.bigrams = kind == B200CTC_KIND_GRAM ? bigrams : nullptr;
-    d.input_lengths = input_lengths; d.label_lengths = label_lengths;
-    d.concurrent = 0;
+    const ProblemDesc d = make_desc(kind, acts, stride_t, stride_b, labels, bigrams, input_lengths, label_lengths, blank, B, T, V, Lmax);
     unsigned char *ws = static_cast<unsigned char *>(workspace);
-    const int nprog = B * w.nblk;
-    zero_header_kernel<<<(nprog + 255) / 256 > 0 ? (nprog + 255) / 256 : 1, 256, 0, stream>>>(
-        reinterpret_cast<WsHeader *>(ws + w.off_hdr), reinterpret_cast<unsigned *>(ws + w.off_prog), nprog);
-    if ((rc = check_cuda(cudaGetLastError(), "workspace header reset"))) return rc;
+    if ((rc = reset_workspace_header(w, ws, stream))) return rc;
     if ((rc = check_cuda(launch_softmax_gather(d, w, ws, nullptr, 0, stream), "softmax/gather kernel"))) return rc;
     AlignParams a;
     a.d = d; a.w = w; a.ws = ws;

@@ -58,7 +58,10 @@ struct WsHeader {
 // Workspace carve-up (all offsets in bytes from a 16-byte aligned base).
 struct WsLayout {
     int kind, B, T, V, Lmax;
-    int W;         // emission row width: [blank, label_0..label_{Lmax-1} (, bigram_0..)] padded to even
+    int W;         // emission row width: [blank, label_0..label_{Lmax-1} (, bigram_0..)] padded to even.  An utterance with
+                   // Lb labels fills EmissionColumns::count(Lb) of them (the bigram columns past Lb are not written): column c
+                   // is the (m, e) pair emission_pair() gives for the id EmissionColumns::symbol(c, Lb), or (0, SENT) for a
+                   // padded label column (id -1) and an id outside [0, V)
     int Nmax;      // lattice nodes for Lmax
     int Np;        // Nmax (+ boff) padded to a multiple of 4
     int boff;      // beta_t[j] is stored at bv[t][j + boff]: 1 for CTC (aligns the reversed direction's node pairs), else 0
@@ -76,10 +79,20 @@ struct WsLayout {
     size_t off_hdr, off_utt, off_lse, off_lp, off_av, off_bv, off_usym, off_uoff, off_unode, off_urec, off_bm, off_pc, total;
 };
 
+// The problem as the kernels see it (built by api.cu from the entry point's arguments)
+struct ProblemDesc {
+    int kind, B, T, V, Lmax, blank;   // kind: 0 = CTC, 1 = Gram-CTC (a joint call is 1 here plus a second, CTC lattice)
+    const float *acts;
+    int64_t stride_t, stride_b;
+    const int32_t *labels, *bigrams, *input_lengths, *label_lengths;
+    int concurrent; // the lattice kernel runs next to the softmax/gather kernel: the latter signals every finished
+                    // frame (progress counters), the former waits on them, and tickets walk the frames from both ends
+};
+
 __host__ __device__ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // An utterance's input or label length as every kernel reads it: clamped into [0, hi] (T or Lmax)
-__host__ __device__ inline int clamp_length(int v, int hi) { return v < 0 ? 0 : (v > hi ? hi : v); }
+__host__ __device__ inline int clamp_length(int v, int hi) { return max(0, min(v, hi)); }
 
 // kind: 0 = CTC, 1 = Gram-CTC, 2 = joint Gram-CTC + CTC (laid out as Gram-CTC plus a second lattice)
 __host__ inline WsLayout make_layout(int kind, int B, int T, int V, int Lmax) {
@@ -162,6 +175,59 @@ __device__ __forceinline__ void renorm_pair(float &m, float &e) {
 // tools/ubench_step_linear.cu) and flushes to 0 below -126.
 __device__ __forceinline__ float node_posterior(float2 a, float2 b, float Ph, float Pinv) {
     return (a.x * b.x) * ex2_approx((a.y + b.y) - Ph) * Pinv;
+}
+
+// ---- an utterance's lengths and its emission row (format: WsLayout::W) ----
+// A missing length array means the full width (T or Lmax).
+__device__ __forceinline__ int utt_input_length(const ProblemDesc &d, int b) {
+    return clamp_length(d.input_lengths ? __ldg(d.input_lengths + b) : d.T, d.T);
+}
+__device__ __forceinline__ int utt_label_length(const ProblemDesc &d, int b) {
+    return clamp_length(d.label_lengths ? __ldg(d.label_lengths + b) : d.Lmax, d.Lmax);
+}
+// The columns of utterance b's emission row: how many an utterance with Lb (clamped) labels fills, and the vocabulary id
+// of column c (gram_ctc.py:24-32, :155), -1 for a padded label column
+struct EmissionColumns {
+    const int32_t *lab, *big;
+    int Lmax, blank, gram;
+    __device__ __forceinline__ EmissionColumns(const ProblemDesc &d, int b)
+        : lab(d.labels + (size_t)b * d.Lmax), big(d.kind == 1 ? d.bigrams + (size_t)b * d.Lmax : nullptr), Lmax(d.Lmax),
+          blank(d.blank), gram(d.kind == 1) {}
+    __device__ __forceinline__ int count(int Lb) const { return 1 + (gram ? Lmax + Lb : Lb); }
+    __device__ __forceinline__ int symbol(int c, int Lb) const {
+        if (c == 0) return blank;
+        if (c <= Lmax) return (c - 1 < Lb) ? __ldg(lab + c - 1) : -1;
+        return __ldg(big + c - 1 - Lmax);
+    }
+};
+
+// log2 normaliser of a row, max*log2(e) + log2(sum), as an unevaluated float pair
+__device__ __forceinline__ void split_lse2(float m, float s, float &la, float &lb) {
+    const float mh = m * LOG2E_HI;
+    float ml = fmaf(m, LOG2E_HI, -mh);
+    ml = fmaf(m, LOG2E_LO, ml);
+    const float lg = log2f(s);
+    const float a = mh + lg;                                  // TwoSum(mh, lg)
+    const float bb = a - mh;
+    const float err = (mh - (a - bb)) + (lg - bb);
+    la = a;
+    lb = err + ml;
+}
+// Emission probability p = 2^(x*log2(e) - lse2) in the lattice's (mantissa, integer exponent) format.  log2 p is first
+// formed as integer hi + small lo, exact to ~1e-7 between symbols (lse2 comes as an unevaluated sum la + lb so that its
+// own rounding does not enter); the mantissa is then 2^lo in [0.70, 1.42].
+__device__ __forceinline__ float2 emission_pair(float x, float la, float lb) {
+    const float ph = x * LOG2E_HI;
+    float pl = fmaf(x, LOG2E_HI, -ph);
+    pl = fmaf(x, LOG2E_LO, pl);
+    const float dd = ph - la;                                 // TwoSum(ph, -la)
+    const float bb = dd - ph;
+    const float err = (ph - (dd - bb)) + (-la - bb);
+    const float lo_full = (err + pl) - lb;
+    const float hi = rintf(dd);
+    const float lo = (dd - hi) + lo_full;
+    if (dd < SENT_TEST) return make_float2(0.f, SENT);        // -inf activation: probability 0 (a NaN still propagates)
+    return make_float2(exp2f(lo), hi);
 }
 
 // ---- frame progress between the softmax/gather kernel and a concurrently running lattice kernel ----

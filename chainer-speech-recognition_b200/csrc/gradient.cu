@@ -449,8 +449,7 @@ cudaError_t launch_gradient(const GradParams &g, const WsLayout &w, const void *
     const int b_major = g.gstride_b > g.gstride_t ? 1 : 0;
     const size_t extra = sizeof(float) * (size_t)((g.d.V + 4 + 3) & ~3) + (g.d.B <= kUttCache ? sizeof(UttInfo) * (size_t)g.d.B : 0);
     const RingLayout rl = make_ring(ring_row_bytes(g.d.V) + sizeof(float) * (4 * (size_t)w.Np + (w.joint ? 4 * (size_t)w.Np2 : 0)), extra);
-    if (ring_usable(g.d.acts, g.d.stride_t, g.d.stride_b, g.d.V, rl) &&
-        ring_usable(g.grad_out, g.gstride_t, g.gstride_b, g.d.V, rl)) {
+    if (ring_usable(g.d.acts, rl) && ring_usable(g.grad_out, rl)) {
         long long ctas = (frames + kTicketBatch - 1) / kTicketBatch;
         if (ctas > sm_count()) ctas = sm_count();
         if (ctas < 1) ctas = 1;

@@ -88,7 +88,7 @@ __global__ void __launch_bounds__(kErrThreads) greedy_error_kernel(
 
     if (warp == 0) {
         // ---- collapse + expansion (asr/error.py:38-53) ----
-        int Tb = input_lengths ? max(0, min(input_lengths[b], T)) : T;
+        int Tb = input_lengths ? clamp_length(input_lengths[b], T) : T;
         int base = 0, prev_last = blank;
         for (int t0 = 0; t0 < Tb; t0 += 32) {
             const int t = t0 + lane;
@@ -139,7 +139,7 @@ __global__ void __launch_bounds__(kErrThreads) edit_distance_kernel(
     const int b = blockIdx.x;
     int *r = sm;
     int *diag = sm + Rmax;
-    const int R = max(0, min(ref_len_in[b], Rmax)), H = max(0, min(hyp_len_in[b], Hmax));
+    const int R = clamp_length(ref_len_in[b], Rmax), H = clamp_length(hyp_len_in[b], Hmax);
     for (int i = threadIdx.x; i < R; i += blockDim.x) r[i] = ref[(size_t)b * Rmax + i];
     __syncthreads();
     const int dist = edit_distance_cta(r, R, hyp + (size_t)b * Hmax, H, diag, wrap8);

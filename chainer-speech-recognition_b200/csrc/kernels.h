@@ -6,15 +6,6 @@
 
 namespace b200ctc {
 
-struct ProblemDesc {
-    int kind, B, T, V, Lmax, blank;
-    const float *acts;
-    int64_t stride_t, stride_b;
-    const int32_t *labels, *bigrams, *input_lengths, *label_lengths;
-    int concurrent; // the lattice kernel runs next to the softmax/gather kernel: the latter signals every finished
-                    // frame (progress counters), the former waits on them, and tickets walk the frames from both ends
-};
-
 // kernel 1: fused log-softmax statistics + label gather (+ optional greedy argmax)
 // smem_reserve: shared memory to leave free per SM for a lattice CTA running next to this kernel (0 = none)
 cudaError_t launch_softmax_gather(const ProblemDesc &d, const WsLayout &w, void *ws, int64_t *argmax_out,
@@ -24,7 +15,7 @@ cudaError_t launch_argmax(const float *acts, int64_t stride_t, int64_t stride_b,
 
 // shared by the two row-streaming kernels (defined in softmax_gather.cu)
 struct RingLayout;
-bool ring_usable(const void *base, int64_t stride_t, int64_t stride_b, int V, const RingLayout &rl);
+bool ring_usable(const void *base, const RingLayout &rl);
 
 // ---- host-side caches (host_cache.cu): nothing below costs a driver call after its first use ----
 // a launcher that fails names the step that failed; api.cu appends it to the error message

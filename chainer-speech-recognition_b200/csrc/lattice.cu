@@ -516,10 +516,8 @@ __global__ void __launch_bounds__(32 * (MAXW + 1)) lattice_kernel(LatticeParams 
     UttInfo *ui = reinterpret_cast<UttInfo *>(p.ws + p.w.off_utt) + b;
     WsHeader *hdr = reinterpret_cast<WsHeader *>(p.ws + p.w.off_hdr);
 
-    int Tb = d.input_lengths ? d.input_lengths[b] : d.T;
-    int Lb = d.label_lengths ? d.label_lengths[b] : d.Lmax;
-    Tb = __shfl_sync(0xffffffffu, max(0, min(Tb, d.T)), 0);
-    Lb = __shfl_sync(0xffffffffu, max(0, min(Lb, d.Lmax)), 0);
+    const int Tb = __shfl_sync(0xffffffffu, utt_input_length(d, b), 0);
+    const int Lb = __shfl_sync(0xffffffffu, utt_label_length(d, b), 0);
     const int Nb = (GRAM ? 3 : 2) * Lb + 1;
 
     const SmemPlan sp = plan_smem(p.w.W, W, S, PAD, CH);

@@ -83,7 +83,7 @@ struct LnSmem {
 };
 
 // ring of R boxes + everything else a kernel needs (the backward-only parts are 0 in the forward kernel)
-LnSmem plan_ln_smem(int K, size_t ab_bytes, size_t post_floats, size_t ebuf_floats, size_t csr_ints, size_t gb_floats,
+LnSmem plan_ln_smem(size_t ab_bytes, size_t post_floats, size_t ebuf_floats, size_t csr_ints, size_t gb_floats,
                     size_t bm_words, size_t zero_bytes, size_t smem_reserve = 0) {
     LnSmem s;
     size_t o = 0;
@@ -109,7 +109,6 @@ LnSmem plan_ln_smem(int K, size_t ab_bytes, size_t post_floats, size_t ebuf_floa
     if (R > 64) R = 64;
     s.R = R;
     s.total = o + (size_t)(R > 0 ? R : 0) * kLnBoxBytes;
-    (void)K;
     return s;
 }
 
@@ -225,33 +224,6 @@ struct Pair2 {                        // two plain sums
 };
 __device__ __forceinline__ Pair2 merge_pair2(const Pair2 &x, const Pair2 &y) { return Pair2{x.a + y.a, x.b + y.b}; }
 
-// log2 normaliser as an unevaluated pair, emission probability as (mantissa, exponent): same arithmetic as the row
-// kernels (softmax_gather.cu), restated here because those helpers are file-local there
-__device__ __forceinline__ void ln_split_lse2(float m, float s, float &la, float &lb) {
-    const float mh = m * LOG2E_HI;
-    float ml = fmaf(m, LOG2E_HI, -mh);
-    ml = fmaf(m, LOG2E_LO, ml);
-    const float lg = log2f(s);
-    const float a = mh + lg;
-    const float bb = a - mh;
-    const float err = (mh - (a - bb)) + (lg - bb);
-    la = a;
-    lb = err + ml;
-}
-__device__ __forceinline__ float2 ln_emission_pair(float x, float la, float lb) {
-    const float ph = x * LOG2E_HI;
-    float pl = fmaf(x, LOG2E_HI, -ph);
-    pl = fmaf(x, LOG2E_LO, pl);
-    const float dd = ph - la;
-    const float bb = dd - ph;
-    const float err = (ph - (dd - bb)) + (-la - bb);
-    const float lo_full = (err + pl) - lb;
-    const float hi = rintf(dd);
-    const float lo = (dd - hi) + lo_full;
-    if (dd < SENT_TEST) return make_float2(0.f, SENT);
-    return make_float2(exp2f(lo), hi);
-}
-
 struct LnParams {
     ProblemDesc d;                  // d.acts unused; kind/B/T/V/Lmax/blank/labels/bigrams/lengths/concurrent as usual
     WsLayout w;
@@ -320,10 +292,8 @@ __device__ __forceinline__ void ln_producer(const CUtensorMap *tmap, const CUten
         } else if (PASS == kLnArgmax) {
             mm.Tb = p.d.T; mm.Lb = 0;
         } else {
-            int Tb = p.d.input_lengths ? __ldg(p.d.input_lengths + b) : p.d.T;
-            int Lb = p.d.label_lengths ? __ldg(p.d.label_lengths + b) : p.d.Lmax;
-            mm.Tb = max(0, min(Tb, p.d.T));
-            mm.Lb = max(0, min(Lb, p.d.Lmax));
+            mm.Tb = utt_input_length(p.d, b);
+            mm.Lb = utt_label_length(p.d, b);
         }
         if (t0 >= mm.Tb) {                            // nothing but padding
             if (BACKWARD) {
@@ -549,15 +519,12 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
         ++seq;
         if (m.kind < 0) break;
         const int Tb = m.Tb, Lb = m.Lb;
-        const int ncol = 1 + (d.kind == 1 ? d.Lmax + Lb : Lb);
-        // the id of this thread's emission column, requested now (its round trip hides behind the tile load and the
-        // moments): thread c takes column c -- 0 = blank, 1..Lmax = labels, Lmax+1.. = bigrams (gram_ctc.py:24-32, :155)
+        const EmissionColumns cols(d, m.b);
+        const int ncol = cols.count(Lb);
+        // the id of this thread's emission column (thread c takes column c of WsLayout::W), requested now: its round trip
+        // hides behind the tile load and the moments
         int sym = -1;
-        if (tid < ncol) {
-            if (tid == 0) sym = d.blank;
-            else if (tid <= d.Lmax) sym = (tid - 1 < Lb) ? __ldg(d.labels + (size_t)m.b * d.Lmax + tid - 1) : -1;
-            else sym = __ldg(d.bigrams + (size_t)m.b * d.Lmax + tid - 1 - d.Lmax);
-        }
+        if (tid < ncol) sym = cols.symbol(tid, Lb);
         // ---- the tile into registers: rows 240k + 16w + r, frames 4h .. 4h+3; the threads that own an emission column
         //      pick up their symbol's row on the way.  Every box goes back to the loader as soon as this warp has read it:
         //      the ring is a sliding window of boxes in flight ----
@@ -634,7 +601,7 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
             for (int o = 1; o < 16; o <<= 1) a = merge_maxsum(a, MaxSum::shfl_xor(a, o));
             if (lane == 0) {
                 float la, lb;
-                ln_split_lse2(a.m, a.s, la, lb);
+                split_lse2(a.m, a.s, la, lb);
                 tot[w * 8 + 2] = la;
                 tot[w * 8 + 3] = lb;
                 const int t = m.t0 + w;
@@ -654,7 +621,7 @@ __global__ void __maxnreg__(104) ln_softmax_gather_kernel(const __grid_constant_
                     float2 v = make_float2(0.f, SENT);
                     if (sym >= 0) {
                         const float a = fmaf((zz[f] - tot[f * 8 + 0]) * tot[f * 8 + 1], gs, bs);
-                        v = ln_emission_pair(a, tot[f * 8 + 2], tot[f * 8 + 3]);
+                        v = emission_pair(a, tot[f * 8 + 2], tot[f * 8 + 3]);
                     }
                     lp_out[((size_t)m.b * d.T + t) * p.w.W + tid] = v;
                 }
@@ -1115,7 +1082,7 @@ static int ln_kmax(int K) { return K <= 5 ? 5 : (K <= 9 ? 9 : (K <= 15 ? 15 : 17
 LnSmem plan_ln_backward(const WsLayout &w) {
     const int K = (w.V + kLnBoxRows - 1) / kLnBoxRows;
     const int Vt = ln_kmax(K) * kLnBoxRows;
-    return plan_ln_smem(K, (size_t)2 * kLnTT * w.Np * 8, (size_t)kLnTT * ((w.Umax + 3) & ~3),
+    return plan_ln_smem((size_t)2 * kLnTT * w.Np * 8, (size_t)kLnTT * ((w.Umax + 3) & ~3),
                         (size_t)kLnTT * w.Np + (size_t)kLnTT * kLnBlankChunks, (size_t)2 * w.Nmax + 2, (size_t)2 * Vt,
                         (size_t)2 * (Vt / 32 + 1), kLnBoxBytes);
 }
@@ -1125,8 +1092,8 @@ LnSmem plan_ln_backward(const WsLayout &w) {
 // would then hold fewer than K + 2 boxes.
 LnSmem plan_ln_stream(int K, size_t smem_reserve) {
     const size_t gbf = (size_t)2 * ln_kmax(K) * kLnBoxRows;
-    LnSmem sm = plan_ln_smem(K, 0, 0, 0, 0, gbf, 0, 0, smem_reserve);
-    if (sm.R < K + 2) sm = plan_ln_smem(K, 0, 0, 0, 0, gbf, 0, 0, 0);     // no room to share the SM
+    LnSmem sm = plan_ln_smem(0, 0, 0, 0, gbf, 0, 0, smem_reserve);
+    if (sm.R < K + 2) sm = plan_ln_smem(0, 0, 0, 0, gbf, 0, 0, 0);     // no room to share the SM
     if (sm.R > 2 * K + 4) {                       // more than two tiles' worth buys nothing; leave the rest to the L1
         sm.total -= (size_t)(sm.R - (2 * K + 4)) * kLnBoxBytes;
         sm.R = 2 * K + 4;
@@ -1171,6 +1138,20 @@ bool make_z_map(CUtensorMap *map, const float *z, int B, int T, int V, int64_t z
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+// The fields every tile kernel reads (the backward-only ones zero; the argmax passes no workspace)
+LnParams ln_params(const ProblemDesc &d, const LnLayout &ll, const void *ws, const float *z, int64_t zs_b, int64_t zs_v,
+                   const float *gamma, const float *beta) {
+    LnParams p;
+    memset(&p, 0, sizeof(p));
+    p.d = d; p.w = ll.w; p.ws = const_cast<unsigned char *>(static_cast<const unsigned char *>(ws));
+    p.z = z; p.zs_b = zs_b; p.zs_v = zs_v; p.gamma = gamma; p.beta = beta;
+    p.off_mu = ll.off_mu; p.off_rstd = ll.off_rstd; p.off_lse = ll.off_lse; p.off_part = ll.off_part;
+    p.Tq = (d.T + 3) & ~3;
+    p.K = (d.V + kLnBoxRows - 1) / kLnBoxRows;
+    p.nTB = (d.T + kLnTT - 1) / kLnTT;
+    return p;
+}
+
 template <typename Kern, typename... Args>
 cudaError_t launch_ln(Kern kern, int grid, const LnSmem &sm, cudaStream_t stream, const Args &...args) {
     (void)cudaGetLastError();
@@ -1213,14 +1194,7 @@ int ln_supported(int kind, int B, int T, int V, int Lmax, int64_t zs_v, int64_t 
 cudaError_t launch_ln_forward(const ProblemDesc &d, const LnLayout &ll, void *ws, const float *z, int64_t zs_b, int64_t zs_v,
                               const float *gamma, const float *beta, size_t smem_reserve, cudaStream_t stream) {
     if ((long long)d.B * d.T == 0) return cudaSuccess;
-    LnParams p;
-    memset(&p, 0, sizeof(p));
-    p.d = d; p.w = ll.w; p.ws = static_cast<unsigned char *>(ws);
-    p.z = z; p.zs_b = zs_b; p.zs_v = zs_v; p.gamma = gamma; p.beta = beta;
-    p.off_mu = ll.off_mu; p.off_rstd = ll.off_rstd; p.off_lse = ll.off_lse; p.off_part = ll.off_part;
-    p.Tq = (d.T + 3) & ~3;
-    p.K = (d.V + kLnBoxRows - 1) / kLnBoxRows;
-    p.nTB = (d.T + kLnTT - 1) / kLnTT;
+    LnParams p = ln_params(d, ll, ws, z, zs_b, zs_v, gamma, beta);
     const LnSmem sm = plan_ln_stream(p.K, smem_reserve);
     if (sm.R < p.K + 2) return cudaErrorInvalidConfiguration;
     p.R = sm.R;
@@ -1242,14 +1216,7 @@ cudaError_t launch_ln_backward(const GradParams &g, const LnLayout &ll, const vo
                                float *dbeta, cudaStream_t stream) {
     const ProblemDesc &d = g.d;
     if ((long long)d.B * d.T == 0) return cudaSuccess;
-    LnParams p;
-    memset(&p, 0, sizeof(p));
-    p.d = d; p.w = ll.w; p.ws = const_cast<unsigned char *>(static_cast<const unsigned char *>(ws));
-    p.z = z; p.zs_b = zs_b; p.zs_v = zs_v; p.gamma = gamma; p.beta = beta;
-    p.off_mu = ll.off_mu; p.off_rstd = ll.off_rstd; p.off_lse = ll.off_lse; p.off_part = ll.off_part;
-    p.Tq = (d.T + 3) & ~3;
-    p.K = (d.V + kLnBoxRows - 1) / kLnBoxRows;
-    p.nTB = (d.T + kLnTT - 1) / kLnTT;
+    LnParams p = ln_params(d, ll, ws, z, zs_b, zs_v, gamma, beta);
     p.grad_loss = g.grad_loss; p.per_utterance = g.per_utterance; p.scale = g.scale;
     p.dz = dz; p.dzs_b = dzs_b; p.dzs_v = dzs_v; p.dgamma = dgamma; p.dbeta = dbeta;
     const int Vp = p.K * kLnBoxRows;
@@ -1283,12 +1250,10 @@ cudaError_t launch_ln_backward(const GradParams &g, const LnLayout &ll, const vo
 cudaError_t launch_ln_argmax(const float *z, int64_t zs_b, int64_t zs_v, const float *gamma, const float *beta, int B, int T, int V,
                              int64_t *argmax_out, cudaStream_t stream) {
     if ((long long)B * T == 0) return cudaSuccess;
-    LnParams p;
-    memset(&p, 0, sizeof(p));
-    p.d.B = B; p.d.T = T; p.d.V = V;
-    p.z = z; p.zs_b = zs_b; p.zs_v = zs_v; p.gamma = gamma; p.beta = beta;
-    p.K = (V + kLnBoxRows - 1) / kLnBoxRows;
-    p.nTB = (T + kLnTT - 1) / kLnTT;
+    ProblemDesc d;
+    memset(&d, 0, sizeof(d));
+    d.B = B; d.T = T; d.V = V;
+    LnParams p = ln_params(d, LnLayout(), nullptr, z, zs_b, zs_v, gamma, beta);
     const LnSmem sm = plan_ln_stream(p.K, 0);
     if (sm.R < p.K + 2) { note_failure_site("shared-memory plan"); return cudaErrorInvalidConfiguration; }
     p.R = sm.R;

@@ -78,6 +78,22 @@ __device__ __forceinline__ void fold1(RowStat &st, float x, int idx) {
     fold<ARGMAX>(st, x, idx);
 }
 
+// numpy.argmax over the warp from each lane's (best value, its index): lane order is not index order, so reduce on
+// (value, index) with "NaN beats all, then larger value, then smaller index".  Returns the index, warp-uniform.
+__device__ __forceinline__ int warp_argmax(float bv, int bi) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        const bool onan = (ov != ov), mnan = (bv != bv);
+        bool take;
+        if (onan || mnan) take = onan && (!mnan || oi < bi);
+        else take = (ov > bv) || (ov == bv && oi < bi);
+        if (take) { bv = ov; bi = oi; }
+    }
+    return bi;
+}
+
 // Scan one row with the whole warp.  Returns warp-uniform (max, log2 normaliser, argmax).
 template <bool ARGMAX, bool SOFTMAX>
 __device__ __forceinline__ void scan_row(const float *__restrict__ row, int V, int lane, float &row_max,
@@ -132,52 +148,7 @@ __device__ __forceinline__ void scan_row(const float *__restrict__ row, int V, i
         row_max = m;
         lse2 = s;                                                // caller finishes with split_lse2(row_max, lse2)
     }
-    if (ARGMAX) {
-        // lane order is not index order: reduce on (value, index) with "NaN beats all, then larger value,
-        // then smaller index"
-        float bv = st.bv; int bi = st.bi;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
-            const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-            const bool onan = (ov != ov), mnan = (bv != bv);
-            bool take;
-            if (onan || mnan) take = onan && (!mnan || oi < bi);
-            else take = (ov > bv) || (ov == bv && oi < bi);
-            if (take) { bv = ov; bi = oi; }
-        }
-        amax = bi;
-    }
-}
-
-// Emission probability p = 2^(x*log2(e) - lse2) in the lattice's (mantissa, integer exponent) format
-// (common.cuh).  log2 p is first formed as integer hi + small lo, exact to ~1e-7 between symbols (lse2 comes as
-// an unevaluated sum la + lb so that its own rounding does not enter); the mantissa is then 2^lo in [0.70, 1.42].
-__device__ __forceinline__ float2 emission_pair(float x, float la, float lb) {
-    const float ph = x * LOG2E_HI;
-    float pl = fmaf(x, LOG2E_HI, -ph);
-    pl = fmaf(x, LOG2E_LO, pl);
-    const float dd = ph - la;                                 // TwoSum(ph, -la)
-    const float bb = dd - ph;
-    const float err = (ph - (dd - bb)) + (-la - bb);
-    const float lo_full = (err + pl) - lb;
-    const float hi = rintf(dd);
-    const float lo = (dd - hi) + lo_full;
-    if (dd < SENT_TEST) return make_float2(0.f, SENT);        // -inf activation: probability 0 (a NaN still propagates)
-    return make_float2(exp2f(lo), hi);
-}
-
-// log2 normaliser of a row, max*log2(e) + log2(sum), as an unevaluated float pair
-__device__ __forceinline__ void split_lse2(float m, float s, float &la, float &lb) {
-    const float mh = m * LOG2E_HI;
-    float ml = fmaf(m, LOG2E_HI, -mh);
-    ml = fmaf(m, LOG2E_LO, ml);
-    const float lg = log2f(s);
-    const float a = mh + lg;                                  // TwoSum(mh, lg)
-    const float bb = a - mh;
-    const float err = (mh - (a - bb)) + (lg - bb);
-    la = a;
-    lb = err + ml;
+    if (ARGMAX) amax = warp_argmax(st.bv, st.bi);
 }
 
 template <bool ARGMAX>
@@ -201,9 +172,10 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) softmax_gather_kernel(Probl
         if (f >= frames) break;
         int b, t;
         frame_of_ticket(f, d.B, d.T, d.concurrent != 0, b, t);
-        int Tb = d.input_lengths ? d.input_lengths[b] : d.T;
-        Tb = max(0, min(Tb, d.T));
-        const bool valid = t < Tb;
+        // Lengths and label ids are read with plain (coherent) loads here, not through the read-only path of
+        // utt_input_length() / EmissionColumns: with those ptxas issues only two of the four row loads of scan_row's
+        // unrolled step up front, and this kernel took 8 % longer (V = 20000, B200).
+        const bool valid = t < clamp_length(d.input_lengths ? d.input_lengths[b] : d.T, d.T);
         if (!valid && !ARGMAX) continue;
         const float *row = d.acts + (int64_t)t * d.stride_t + (int64_t)b * d.stride_b;
         float row_max = 0.f, lse2 = 0.f;
@@ -216,9 +188,8 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) softmax_gather_kernel(Probl
         split_lse2(row_max, lse2, la, lb);
         if (lane == 0 && pend_b >= 0 && d.concurrent) signal_frame_done(ws, w, pend_b, pend_t);
         if (lane == 0) lse_out[(size_t)b * d.T + t] = grad_normaliser(row_max, la, lb);
-        // gather: column 0 = blank, 1..Lmax = labels, Lmax+1.. = bigrams (gram_ctc.py:24-32, :155)
-        int Lb = d.label_lengths ? d.label_lengths[b] : d.Lmax;
-        Lb = max(0, min(Lb, d.Lmax));
+        // gather the emission row (WsLayout::W, as EmissionColumns maps it)
+        const int Lb = clamp_length(d.label_lengths ? d.label_lengths[b] : d.Lmax, d.Lmax);
         float2 *lprow = lp_out + ((size_t)b * d.T + t) * w.W;
         const int32_t *lab = d.labels + (size_t)b * d.Lmax;
         const int32_t *big = d.kind == 1 ? d.bigrams + (size_t)b * d.Lmax : nullptr;
@@ -363,10 +334,8 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
     const bool len_cached = d.B <= kLenCache;
     if (len_cached) {
         for (int i = threadIdx.x; i < d.B; i += blockDim.x) {
-            const int Tb = d.input_lengths ? __ldg(d.input_lengths + i) : d.T;
-            const int Lb = d.label_lengths ? __ldg(d.label_lengths + i) : d.Lmax;
-            len_sm[i] = max(0, min(Tb, d.T));
-            len_sm[d.B + i] = max(0, min(Lb, d.Lmax));
+            len_sm[i] = utt_input_length(d, i);
+            len_sm[d.B + i] = utt_label_length(d, i);
         }
     }
     __syncthreads();
@@ -388,12 +357,7 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
                 frame_of_ticket(f, d.B, d.T, d.concurrent != 0, b, t);
                 int Tb;
                 if (len_cached) { Tb = len_sm[b]; Lb = len_sm[d.B + b]; }
-                else {
-                    Tb = d.input_lengths ? __ldg(d.input_lengths + b) : d.T;
-                    Lb = d.label_lengths ? __ldg(d.label_lengths + b) : d.Lmax;
-                    Tb = max(0, min(Tb, d.T));
-                    Lb = max(0, min(Lb, d.Lmax));
-                }
+                else { Tb = utt_input_length(d, b); Lb = utt_label_length(d, b); }
                 valid = t < Tb;
                 need = valid || ARGMAX;
             }
@@ -466,25 +430,19 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
             __syncwarp();
         }
         bool released = false;                  // the slot has already been handed back (early, see the gather)
-        // Emitted ids of this lane's columns, requested now so that their latency hides behind the row scan:
-        // column 0 = blank, 1..Lmax = labels, Lmax+1.. = bigrams (gram_ctc.py:24-32, :155)
+        // Emitted ids of this lane's columns of the emission row (WsLayout::W), requested now so that their latency
+        // hides behind the row scan
         int Lb = 0, ncol = 0;
-        const int32_t *lab = d.labels + (size_t)m.b * d.Lmax;
-        const int32_t *big = d.kind == 1 ? d.bigrams + (size_t)m.b * d.Lmax : nullptr;
-        auto symbol_of = [&](int cidx) {
-            if (cidx == 0) return d.blank;
-            if (cidx <= d.Lmax) return (cidx - 1 < Lb) ? __ldg(lab + cidx - 1) : -1;
-            return __ldg(big + cidx - 1 - d.Lmax);
-        };
+        const EmissionColumns cols(d, m.b);
         int syms[kGatherRegs];
         bool early = false;
         if (m.kind == 0) {
             Lb = m.Lb;
-            ncol = 1 + (d.kind == 1 ? d.Lmax + Lb : Lb);
+            ncol = cols.count(Lb);
             early = ncol <= 32 * kGatherRegs;
             if (early) {
 #pragma unroll
-                for (int k = 0; k < kGatherRegs; ++k) syms[k] = (lane + 32 * k < ncol) ? symbol_of(lane + 32 * k) : -1;
+                for (int k = 0; k < kGatherRegs; ++k) syms[k] = (lane + 32 * k < ncol) ? cols.symbol(lane + 32 * k, Lb) : -1;
             }
         }
         float la = 0.f, lb = 0.f, mx = 0.f;
@@ -510,17 +468,7 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
                 }
             }
             if (ARGMAX) {
-                float bv = st.bv; int bi = st.bi;
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {
-                    const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
-                    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-                    const bool onan = (ov != ov), mnan = (bv != bv);
-                    bool take;
-                    if (onan || mnan) take = onan && (!mnan || oi < bi);
-                    else take = (ov > bv) || (ov == bv && oi < bi);
-                    if (take) { bv = ov; bi = oi; }
-                }
+                const int bi = warp_argmax(st.bv, st.bi);
                 // an element of the span in front of the row (index < 0, value -inf) can only "win" when every
                 // element of the row is -inf, and numpy.argmax of such a row is 0
                 if (lane == 0) argmax_out[(size_t)m.b * d.T + m.t] = bi < 0 ? 0 : bi;
@@ -559,7 +507,7 @@ __global__ void __launch_bounds__(kK1Threads, 1) softmax_gather_ring_kernel(Prob
                 if (fast) fast_row_finish(ref, sl, la, lb, mx);
                 if (lane == 0) lse_out[(size_t)m.b * d.T + m.t] = grad_normaliser(mx, la, lb);
                 for (int cidx = lane; cidx < ncol; cidx += 32) {
-                    const int sym = symbol_of(cidx);
+                    const int sym = cols.symbol(cidx, Lb);
                     float2 v = make_float2(0.f, SENT);
                     if (sym >= 0 && sym < d.V) v = emission_pair(row[sym], la, lb);
                     lprow[cidx] = v;
@@ -605,8 +553,7 @@ int grid_for_frames(long long frames) {
 
 // Rows qualify for the TMA ring when at least kMinSlots of them (each with room for the 16-byte aligned span around a
 // row that is only 4-byte aligned) fit in shared memory; base pointer and strides are in floats, so any of them do.
-bool ring_usable(const void *base, int64_t stride_t, int64_t stride_b, int V, const RingLayout &rl) {
-    (void)stride_t; (void)stride_b; (void)V;
+bool ring_usable(const void *base, const RingLayout &rl) {
     return (reinterpret_cast<uintptr_t>(base) & 3) == 0 && rl.slots >= kMinSlots;
 }
 
@@ -616,7 +563,7 @@ cudaError_t launch_softmax_gather(const ProblemDesc &d, const WsLayout &w, void 
     if (frames == 0) return cudaSuccess;
     unsigned char *wsb = static_cast<unsigned char *>(ws);
     const RingLayout rl = make_ring(ring_row_bytes(d.V), kFifoBytes + (d.B <= kLenCache ? 8 * (size_t)d.B : 0), smem_reserve, kK1Consumers);
-    if (ring_usable(d.acts, d.stride_t, d.stride_b, d.V, rl)) {
+    if (ring_usable(d.acts, rl)) {
         long long ctas = (frames + kTicketBatch - 1) / kTicketBatch;
         if (ctas > sm_count()) ctas = sm_count();
         if (ctas < 1) ctas = 1;
